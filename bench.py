@@ -9,6 +9,7 @@ all-reduce of the 4 KB sweep header (the metric counters) at the end of the time
     python bench.py [--gpus N] [--steps K] [--warmup W]            # this repo's CUDA path
     python bench.py --workload c2                                  # BASELINE config 2: decode+NMS+mask assembly, masks out
     python bench.py --impl reference ...                           # the reference's ops on the host cores (torch port)
+    python bench.py ... --dump-outputs DIR                         # also write the last timed step's outputs as DIR/*.npy
 
 Prints ONE JSON line (rank 0).  See DESIGN.md "Measurement" for the definition of every key.
 """
@@ -33,6 +34,39 @@ UNIT = "images/s"
 SEED = 20262
 KERNELS = ["gt_pack_kernel", "decode_filter_l2_kernel", "nms_kernel", "plan_kernel", "coeff_gather_kernel", "match_kernel",
            "contract_kernel", "cells_kernel", "finalize_kernel"]
+DUMP_BYTES = 64 * 10**6    # --dump-outputs: all files of one dump together
+
+
+def dump_outputs(out, path, budget=DUMP_BYTES):
+    """Writes one step's outputs (`out`: name -> tensor) as <path>/<name>.npy, so that two builds can be compared output
+    for output.  Integer and float64 outputs are stored as float64, the others as float32: every value is kept exactly.
+    When the whole set would exceed `budget` bytes, each output larger than a common element count is cut to that many
+    of its flattened elements at most: distinct flat indices drawn from a generator seeded with SEED and the output's name,
+    in ascending order, so that the same arguments select the same elements.  Returns the names of the cut outputs."""
+    import zlib
+
+    import torch
+    path = Path(path)
+    path.mkdir(parents=True, exist_ok=True)
+    wide = {k: t.dtype == torch.float64 or (not t.is_floating_point() and t.element_size() >= 4) for k, t in out.items()}
+    sizes = {k: t.numel() for k, t in out.items()}
+
+    def nbytes(cap):                                    # 256 bytes per file for the .npy header
+        return sum((8 if wide[k] else 4) * min(n, cap) + 256 for k, n in sizes.items())
+
+    lo, hi = 0, max(sizes.values(), default=0)          # the largest common cap that fits the budget
+    while lo < hi:
+        mid = (lo + hi + 1) // 2
+        lo, hi = (mid, hi) if nbytes(mid) <= budget else (lo, mid - 1)
+    cut = []
+    for k in sorted(out):
+        t = out[k]
+        if sizes[k] > lo:
+            rng = np.random.default_rng([SEED, zlib.crc32(k.encode())])
+            t = t.reshape(-1)[torch.from_numpy(np.unique(rng.integers(0, sizes[k], lo))).to(t.device)]
+            cut.append(k)
+        np.save(path / f"{k}.npy", t.to(torch.float64 if wide[k] else torch.float32).cpu().numpy())
+    return cut
 
 
 def algorithmic_bytes_per_image(S, nc=3, nm=32):
@@ -213,7 +247,14 @@ def main():
                     help="batches in flight = slots with their own input set (0 = auto: 6, 5 or 4, whichever divides --steps; 2 for c2; 1 = strictly serial steps)")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--clock-period-ms", type=int, default=100, help="nvidia-smi sampling period during the timed region (0 = off)")
+    ap.add_argument("--dump-outputs", dest="dump_outputs", metavar="DIR",
+                    help="after the timed steps, write the outputs the last of them returned (rank 0's) as DIR/<name>.npy, "
+                         f"float32 / float64, at most {DUMP_BYTES // 10**6} MB in all (larger outputs: a fixed, seeded sample)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of --impl b200")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     if args.pipeline <= 0:
         # a slot runs its steps one after the other, so a ragged last round (steps not a multiple of the depth) leaves
@@ -296,7 +337,7 @@ def main():
     ev0.record()
     pipe.fork()
     for _ in range(args.steps):
-        pipe.replay()      # step i on slot i % depth: consecutive batches overlap, every step does all of its work
+        last = pipe.replay()      # step i on slot i % depth: consecutive batches overlap, every step does all of its work
     pipe.join()
     if world > 1:
         dist.all_reduce(hdr)  # the only collective: the sweep header = all metric counters (NCCL over NVLink)
@@ -310,6 +351,12 @@ def main():
     ms = float(t.item())
     value = B * world * args.steps / (ms / 1e3)
     det_mean = float(sum(p.out["det_count"].sum() for p in pipe.procs)) / (depth * B)
+    if args.dump_outputs and rank == 0:
+        # the slot's outputs as a caller of the last step receives them; cm / seg_cnt4 / uni_cnt4 are the counters all
+        # slots share, summed over the timed steps
+        cut = dump_outputs(last.out, args.dump_outputs)
+        print(f"bench: wrote {len(last.out)} outputs of the last timed step to {args.dump_outputs}"
+              + (f" (sampled: {', '.join(cut)})" if cut else ""), file=sys.stderr, flush=True)
 
     # ---------------- strictly serial steps (one stream, one batch in flight): the latency of a step
     torch.cuda.synchronize()
