@@ -2,7 +2,6 @@
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
-#include <stdlib.h>
 
 #include "../../include/btpost.h"
 
@@ -29,14 +28,6 @@
 #endif
 
 namespace bt {
-
-// Developer switches (tile buffers, CTAs per SM, ...) exist in the debug build only (`make dbg`: -DBT_DEBUG_HOOKS);
-// the product library reads no environment variables.
-#ifdef BT_DEBUG_HOOKS
-static inline int dbg_env_int(const char *name, int dflt) { const char *e = getenv(name); return e ? atoi(e) : dflt; }
-#else
-static inline int dbg_env_int(const char *, int dflt) { return dflt; }
-#endif
 
 // sigmoid(x) > 0.5 in fp32 (src/running_main_v2.py:702-703, src/test_model.py:85) holds exactly
 // for x > 1.5 * 2^-24 (pinned against torch in tests/golden/make_golden.py).

@@ -49,11 +49,10 @@ typedef unsigned long long u64;
 
 struct K3Params {
     int B, S_h, S_w, PH, PW, K, gt_f32, proto_bf16, NBY, NBX, ntx, nty, m1_items, nq;
-    int pref;               // contract_kernel: tiles prefetched into the L2 ahead of the tile being loaded
-    int interleave;         // contract_kernel: tiles dealt round-robin to the CTAs instead of in contiguous ranges
-    float bias, inv_K, inv_m1;
+    float bias, inv_K;
     const int2 *items;      // plan of the cells kernel: (image * K + detection, chunk)
     const int32_t *n_items;
+    float inv_m1;
     int item_cap;
     const void *protos;     // [B, NM, PH, PW] fp32 or bfloat16 (proto_bf16)
     const float *proj_weight, *det_coeff;
@@ -98,13 +97,6 @@ __device__ __forceinline__ void tma_tile_g2s(void *dst, const CUtensorMap *tm, i
             smem_u32(dst)),
         "l"(reinterpret_cast<uint64_t>(tm)), "r"(col), "r"(row), "r"(chan0), "r"(smem_u32(bar)), "l"(policy)
         : "memory");
-}
-// The same box, DRAM -> L2 only: issued a tile (or two) ahead of the load, it costs no shared memory or registers and
-// turns the load's DRAM latency into an L2 hit.
-__device__ __forceinline__ void tma_tile_prefetch_l2(const CUtensorMap *tm, int col, int row, int chan0) {
-    asm volatile("cp.async.bulk.prefetch.tensor.3d.L2.global.tile [%0, {%1, %2, %3}];" ::"l"(reinterpret_cast<uint64_t>(tm)), "r"(col),
-                 "r"(row), "r"(chan0)
-                 : "memory");
 }
 __device__ __forceinline__ void cp_async16(void *dst, const void *src) {
     asm volatile("cp.async.ca.shared.global [%0], [%1], 16;" ::"r"(smem_u32(dst)), "l"(src) : "memory");
@@ -411,15 +403,15 @@ __global__ void __launch_bounds__(G_THREADS) gt_pack_kernel(const __grid_constan
 // =================================================================================================
 // BF16: the prototypes arrive as bfloat16 (the reference validates under bf16-mixed autocast and upcasts with
 // .float()): a 16 KB tile with the 64-byte swizzle, widened exactly to fp32 on the way into the registers.
-template <int NBUF, int MINB, bool BF16 = false>
-__global__ void __launch_bounds__(A_THREADS, MINB)
+template <bool BF16>
+__global__ void __launch_bounds__(A_THREADS, 4)
 contract_kernel(const __grid_constant__ K3Params P, const __grid_constant__ CUtensorMap tmap) {
     extern __shared__ __align__(1024) unsigned char smem_dyn[];
     // the swizzled TMA destination must be 1024-byte aligned: align by hand (1024 spare bytes are allocated)
     unsigned char *smem = smem_dyn + ((1024u - (smem_u32(smem_dyn) & 1023u)) & 1023u);
     constexpr int TILE_FLOATS = NM * TA_H * TA_W / (BF16 ? 2 : 1);                     // tile size in 4-byte words
-    float *s_tiles = reinterpret_cast<float *>(smem);                                  // [NBUF][NM][TA_H][TA_W], 16-byte chunks XOR row
-    __shared__ __align__(8) uint64_t s_bar[NBUF];
+    float *s_tile = reinterpret_cast<float *>(smem);                                   // [NM][TA_H][TA_W], 16-byte chunks XOR row
+    __shared__ __align__(8) uint64_t s_bar;
     // per-tile tables of the listed detections (coefficients, crop regions, pool offsets of the box origins), two sets:
     // the next tile's set is filled by cp.async while this tile is computed, so a tile costs ONE block barrier
     __shared__ __align__(16) float s_cf2[2][A_LCAP][NM];
@@ -430,17 +422,16 @@ contract_kernel(const __grid_constant__ K3Params P, const __grid_constant__ CUte
     const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
     const int tiles = P.ntx * P.nty, total = tiles * P.B;
     const int PH = P.PH, PW = P.PW, K = P.K;
-    // this CTA's contiguous range of tiles
-    // Tiles of a CTA.  Interleaved (P.interleave): CTA i takes tiles i, i + grid, i + 2 grid, ...: at any moment the CTAs of
-    // the grid read a window of neighbouring tiles, i.e. whole rows of every channel plane (DRAM pages are consumed while
-    // they are open).  Contiguous: a range of total / grid tiles per CTA.
-    const int ts = P.interleave ? (int)gridDim.x : 1;
-    const int t_begin = P.interleave ? (int)blockIdx.x : (int)(((long long)blockIdx.x * total) / gridDim.x);
-    const int t_end = P.interleave ? total : (int)(((long long)(blockIdx.x + 1) * total) / gridDim.x);
+    // this CTA's contiguous range of tiles (measured and not kept: tiles dealt round-robin to the CTAs, so that the grid
+    // reads neighbouring tiles at the same time, 103.4 vs 100.5 us per pipelined step)
+    const int t_begin = (int)(((long long)blockIdx.x * total) / gridDim.x);
+    const int t_end = (int)(((long long)(blockIdx.x + 1) * total) / gridDim.x);
     if (t_begin >= t_end) return;
 
     // The tile buffer is dead as soon as every thread holds its pixels in registers: the next tile's TMA is issued
-    // right then and lands under this tile's arithmetic (one buffer, four CTAs per SM).
+    // right then and lands under this tile's arithmetic (one buffer, four CTAs per SM).  Measured and not kept: two or
+    // three buffers with three or two CTAs per SM (53.6 / 59.5 us: the kernel wants warps, not bytes in flight), and the
+    // next 1 / 2 / 4 tiles prefetched into the L2 (101.5 / 102.6 / 106.6 vs 99.6 us per pipelined step).
     const bool keep_protos = __ldg(P.n_items + 1) != 0;
     // tile coordinates are stepped, not divided out, per tile (the divisions were a fifth of the kernel's instructions)
     struct TileAt { int b, ty, tx; };
@@ -451,29 +442,21 @@ contract_kernel(const __grid_constant__ K3Params P, const __grid_constant__ CUte
         a.ty = t / P.ntx; a.tx = t - a.ty * P.ntx;
         return a;
     };
-    // one step of `ts` tiles, decomposed once into (images, tile rows, tiles)
-    const int ts_b = ts / tiles, ts_y = (ts - ts_b * tiles) / P.ntx, ts_x = ts - ts_b * tiles - ts_y * P.ntx;
-    auto step = [&](TileAt &a) {
-        a.tx += ts_x;
-        if (a.tx >= P.ntx) { a.tx -= P.ntx; ++a.ty; }
-        a.ty += ts_y;
-        if (a.ty >= P.nty) { a.ty -= P.nty; ++a.b; }
-        a.b += ts_b;
+    auto step = [&](TileAt &a) {   // to the next tile
+        if (++a.tx == P.ntx) {
+            a.tx = 0;
+            if (++a.ty == P.nty) { a.ty = 0; ++a.b; }
+        }
     };
-    auto issue = [&](const TileAt &a, int buf) {   // thread 0
-        mbar_expect_tx(&s_bar[buf], (uint32_t)(TILE_FLOATS * sizeof(float)));
-        tma_tile_g2s(s_tiles + buf * TILE_FLOATS, &tmap, a.tx * TA_W, a.ty * TA_H, a.b * NM, &s_bar[buf], keep_protos);
+    auto issue = [&](const TileAt &a) {   // thread 0
+        mbar_expect_tx(&s_bar, (uint32_t)(TILE_FLOATS * sizeof(float)));
+        tma_tile_g2s(s_tile, &tmap, a.tx * TA_W, a.ty * TA_H, a.b * NM, &s_bar, keep_protos);
     };
-    TileAt at = tile_at(t_begin), at_issue = at, at_pref = at;   // current tile; next tile to load / to prefetch (thread 0)
-    const int pref = P.pref;
+    TileAt at = tile_at(t_begin);   // current tile
     if (tid == 0) {
-        for (int i = 0; i < NBUF; ++i) mbar_init(&s_bar[i], 1);
+        mbar_init(&s_bar, 1);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-        for (int i = 0; i < NBUF; ++i)
-            if (t_begin + i * ts < t_end) { issue(at_issue, i); step(at_issue); }
-        at_pref = at_issue;
-        for (int i = 0; i < pref; ++i)
-            if (t_begin + (NBUF + i) * ts < t_end) { tma_tile_prefetch_l2(&tmap, at_pref.tx * TA_W, at_pref.ty * TA_H, at_pref.b * NM); step(at_pref); }
+        issue(at);
     }
     if (tid < NM) s_w[tid] = __ldg(P.proj_weight + tid);
     __syncthreads();
@@ -513,13 +496,12 @@ contract_kernel(const __grid_constant__ K3Params P, const __grid_constant__ CUte
     };
     Meta cur = fetch_meta(t_begin), nxt = cur;
     stage_async(cur, at.b, 0);
-    TileAt at_n = at;   // the tile after the current one
-    step(at_n);
-    if (t_begin + ts < t_end) nxt = fetch_meta(t_begin + ts);
+    if (t_begin + 1 < t_end) nxt = fetch_meta(t_begin + 1);
 
-    for (int tile = t_begin, it = 0; tile < t_end; tile += ts, ++it, step(at), step(at_n)) {
+    for (int tile = t_begin, it = 0; tile < t_end; ++tile, ++it) {
         const int b = at.b;
         const int R0 = at.ty * TA_H, C0 = at.tx * TA_W;
+        step(at);   // from here on `at` is the next tile
         const int r = R0 + row, c = C0 + colp;
         const int nlist = cur.nlist, set = it & 1;
         const unsigned short *list = P.tile_list + (size_t)tile * K;
@@ -528,11 +510,10 @@ contract_kernel(const __grid_constant__ K3Params P, const __grid_constant__ CUte
         int *s_off = s_off2[set];
 
         // ---- the tile: shared memory -> registers, then the buffer is free for the next tile
-        const int buf = it % NBUF;
-        mbar_wait(&s_bar[buf], (uint32_t)((it / NBUF) & 1));
+        mbar_wait(&s_bar, (uint32_t)(it & 1));
         u64 p[NM];
         {
-            const float *src = s_tiles + buf * TILE_FLOATS + soff;
+            const float *src = s_tile + soff;
             if (BF16) {
 #pragma unroll
                 for (int k = 0; k < NM; ++k) {
@@ -546,14 +527,11 @@ contract_kernel(const __grid_constant__ K3Params P, const __grid_constant__ CUte
         }
         cp_async_wait_all();   // this thread's copies into the tile's table set (issued a tile ago)
         __syncthreads();       // the tile buffer is free, the table set is complete, the other set is no longer read
-        if (tid == 0 && tile + NBUF * ts < t_end) {
-            issue(at_issue, buf); step(at_issue);
-            if (pref > 0 && tile + (NBUF + pref) * ts < t_end) { tma_tile_prefetch_l2(&tmap, at_pref.tx * TA_W, at_pref.ty * TA_H, at_pref.b * NM); step(at_pref); }
-        }
-        if (tile + ts < t_end) {
+        if (tile + 1 < t_end) {
+            if (tid == 0) issue(at);
             cur = nxt;
-            stage_async(cur, at_n.b, set ^ 1);
-            if (tile + 2 * ts < t_end) nxt = fetch_meta(tile + 2 * ts);
+            stage_async(cur, at.b, set ^ 1);
+            if (tile + 2 < t_end) nxt = fetch_meta(tile + 2);
         }
 
         // ---- M1 projection: bias + sum_k w_k p_k, sequential fma (== torch conv2d, pinned)
@@ -953,16 +931,17 @@ __device__ __forceinline__ void det_phase(const K3Params &P, int q, int ndet, in
     }
 }
 
-template <int MINB, int GS>
-__global__ void __launch_bounds__(C_WARPS * 32, MINB) cells_kernel(const __grid_constant__ K3Params P) {
+__global__ void __launch_bounds__(C_WARPS * 32, 8) cells_kernel(const __grid_constant__ K3Params P) {
     const int lane = threadIdx.x & 31;
     const int ndet = min(__ldg(P.n_items), P.item_cap);
     const int q = (blockIdx.x * C_WARPS + (threadIdx.x >> 5)) & (P.nq - 1);
-    // Some detection found no room in the logit pool (huge crop boxes / crop off): its items contract their corners from
-    // the prototypes, 32 channels x 9 loads per block; that path runs best with whole-warp items (measured: L1 layout with
-    // random DFL boxes, mask stage 519 us with whole warps, 685 us with groups of 16).
-    if (GS != 32 && __ldg(P.n_items + 1) != 0) det_phase<32>(P, q, ndet, lane);
-    else det_phase<GS>(P, q, ndet, lane);
+    // Detection items are taken by groups of 16 lanes (measured and not kept, pipelined step: groups of 32 / 8 / 4 lanes
+    // = 99.4 / 101.1 / 108.4 us against 97.4 us for 16).  Some detection found no room in the logit pool (huge crop
+    // boxes / crop off): its items contract their corners from the prototypes, 32 channels x 9 loads per block; that path
+    // runs best with whole-warp items (measured: L1 layout with random DFL boxes, mask stage 519 us with whole warps,
+    // 685 us with groups of 16).
+    if (__ldg(P.n_items + 1) != 0) det_phase<32>(P, q, ndet, lane);
+    else det_phase<16>(P, q, ndet, lane);
     {
         const int total = P.B * P.m1_items;
         int *ctr = P.work + q * C_QSTRIDE + 1;
@@ -1048,12 +1027,10 @@ static int make_proto_tmap(CUtensorMap *tm, const void *protos, int bf16, int B,
     const cuuint64_t gstride[2] = {(cuuint64_t)PW * esz, (cuuint64_t)PW * PH * esz};
     const cuuint32_t box[3] = {(cuuint32_t)TA_W, (cuuint32_t)TA_H, (cuuint32_t)NM};
     const cuuint32_t estr[3] = {1u, 1u, 1u};
-    const int pv = dbg_env_int("BTPOST_A_PROMO", 0);   // debug build: L2 promotion (measured: none 47.7 us, 128 B 48.0, 256 B 50.5)
-    const CUtensorMapL2promotion promo = pv == 0 ? CU_TENSOR_MAP_L2_PROMOTION_NONE
-                                       : pv == 1 ? CU_TENSOR_MAP_L2_PROMOTION_L2_128B : CU_TENSOR_MAP_L2_PROMOTION_L2_256B;
+    // no L2 promotion (measured and not kept: 128 B / 256 B promotion, 48.0 / 50.5 us against 47.7 us without)
     const CUresult r = fn(tm, bf16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, const_cast<void *>(protos),
                           gdim, gstride, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                          bf16 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_128B, promo,
+                          bf16 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_NONE,
                           CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     return r == CUDA_SUCCESS ? BT_OK : BT_ERR_CUDA;
 }
@@ -1078,8 +1055,6 @@ int launch_masks(const BtParams &p, const BtIO &io, const Workspace &w, cudaStre
     P.NBY = mask_blocks(p.proto_h); P.NBX = mask_blocks(p.proto_w);
     P.ntx = (p.proto_w + TA_W - 1) / TA_W; P.nty = (p.proto_h + TA_H - 1) / TA_H;
     P.m1_items = (P.NBY * P.NBX + 31) / 32;
-    P.interleave = dbg_env_int("BTPOST_A_ILV", 0);
-    P.pref = dbg_env_int("BTPOST_A_PREF", 0);   // measured: 0 / 1 / 2 / 4 tiles ahead = 99.6 / 101.5 / 102.6 / 106.6 us per pipelined step
     P.inv_K = 1.0f / (float)p.max_det; P.inv_m1 = 1.0f / (float)P.m1_items; P.inv_NBX = 1.0f / (float)P.NBX;
     {
         const int rows[3] = {0, P.NBY > 2 ? 1 : 0, P.NBY - 1}, cols[3] = {0, P.NBX > 2 ? 1 : 0, P.NBX - 1};
@@ -1094,21 +1069,15 @@ int launch_masks(const BtParams &p, const BtIO &io, const Workspace &w, cudaStre
         gt_pack_kernel<<<dim3((P.NBY + G_ROWS - 1) / G_ROWS, p.batch), G_THREADS, smem_g, s>>>(P);
     }
 
-    const int nbuf = P.proto_bf16 ? 1 : dbg_env_int("BTPOST_A_NBUF", 1);   // debug build: tile buffers per CTA
-    const size_t smem_a = (size_t)nbuf * NM * TA_H * TA_W * (P.proto_bf16 ? 2 : 4) + 1024;
+    const size_t smem_a = (size_t)NM * TA_H * TA_W * (P.proto_bf16 ? 2 : 4) + 1024;
     // function attributes are per device: one flag per device ordinal
     static bool attr_done[64] = {};
     int attr_dev = 0;
     if (cudaGetDevice(&attr_dev) != cudaSuccess || attr_dev < 0 || attr_dev >= 64) return BT_ERR_CUDA;
     if (!attr_done[attr_dev]) {
-        if (cudaFuncSetAttribute(contract_kernel<1, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024) != cudaSuccess ||
-            cudaFuncSetAttribute(contract_kernel<1, 4, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024) != cudaSuccess ||
-            cudaFuncSetAttribute(contract_kernel<2, 3>, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024) != cudaSuccess ||
-            cudaFuncSetAttribute(contract_kernel<3, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, 110 * 1024) != cudaSuccess)
+        if (cudaFuncSetAttribute(contract_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024) != cudaSuccess ||
+            cudaFuncSetAttribute(contract_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024) != cudaSuccess)
             return BT_ERR_CUDA;
-#ifdef BT_DEBUG_HOOKS
-        if (cudaFuncSetAttribute(contract_kernel<2, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024) != cudaSuccess) return BT_ERR_CUDA;
-#endif
         attr_done[attr_dev] = true;
     }
     {
@@ -1122,35 +1091,22 @@ int launch_masks(const BtParams &p, const BtIO &io, const Workspace &w, cudaStre
         // SM instead of 4 / 8, which fill the register file) let the other batches' CTAs become resident beside them:
         // 93.1 -> 91.7 us per pipelined step (profiles/r02c_ctas.txt); alone, the kernels are fastest with the full grids.
         const bool shared_gpu = p.in_flight >= 2;
-        const int ntiles = p.batch * P.ntx * P.nty, cta_a = sm_count * dbg_env_int("BTPOST_A_CTAS", nbuf == 1 ? (shared_gpu ? 3 : 4) : nbuf == 2 ? 3 : 2);
+        const int ctas_per_sm_a = shared_gpu ? 3 : 4, ctas_per_sm_c = shared_gpu ? 6 : 8;   // contract_kernel, cells_kernel
+        const int ntiles = p.batch * P.ntx * P.nty, cta_a = sm_count * ctas_per_sm_a;
         const int grid_a = ntiles < cta_a ? ntiles : cta_a;
         if (parts & BT_MASKS_CONTRACT) {
-            if (P.proto_bf16) contract_kernel<1, 4, true><<<grid_a, A_THREADS, smem_a, s>>>(P, tm);
-#ifdef BT_DEBUG_HOOKS
-            else if (nbuf == 2 && dbg_env_int("BTPOST_A_MINB", 3) == 4) contract_kernel<2, 4><<<grid_a, A_THREADS, smem_a, s>>>(P, tm);
-#endif
-            else if (nbuf == 2) contract_kernel<2, 3><<<grid_a, A_THREADS, smem_a, s>>>(P, tm);
-            else if (nbuf == 3) contract_kernel<3, 2><<<grid_a, A_THREADS, smem_a, s>>>(P, tm);
-            else contract_kernel<1, 4><<<grid_a, A_THREADS, smem_a, s>>>(P, tm);
+            if (P.proto_bf16) contract_kernel<true><<<grid_a, A_THREADS, smem_a, s>>>(P, tm);
+            else contract_kernel<false><<<grid_a, A_THREADS, smem_a, s>>>(P, tm);
         }
         const long long items = (long long)p.batch * (p.max_det + P.m1_items);   // grid sizing only: the kernel reads the real count
-        const long long want = (items + C_WARPS - 1) / C_WARPS, cap = (long long)sm_count * dbg_env_int("BTPOST_C_CTAS", shared_gpu ? 6 : 8);
+        const long long want = (items + C_WARPS - 1) / C_WARPS, cap = (long long)sm_count * ctas_per_sm_c;
         if (parts & BT_MASKS_CELLS) {
             const long long ctas = want < cap ? want : cap;
             P.nq = 1;   // queues: a power of two <= warps in the grid (every queue needs a home warp), at most C_NQ
             while (P.nq * 2 <= C_NQ && P.nq * 2 <= ctas * C_WARPS) P.nq *= 2;
             const size_t inst_words = (size_t)p.batch * p.max_det * p.img_h * (p.img_w / 32);
             if (io.inst_bits && cudaMemsetAsync(io.inst_bits, 0, inst_words * 4, s) != cudaSuccess) return BT_ERR_CUDA;
-#ifdef BT_DEBUG_HOOKS
-            const int gs = dbg_env_int("BTPOST_C_GS", 16), mb = dbg_env_int("BTPOST_C_MINB", 8);
-            if (gs == 32 && mb == 7) cells_kernel<7, 32><<<(unsigned)ctas, C_WARPS * 32, 0, s>>>(P);
-            else if (gs == 32) cells_kernel<8, 32><<<(unsigned)ctas, C_WARPS * 32, 0, s>>>(P);
-            else if (gs == 16 && mb == 7) cells_kernel<7, 16><<<(unsigned)ctas, C_WARPS * 32, 0, s>>>(P);
-            else if (gs == 8 && mb == 7) cells_kernel<7, 8><<<(unsigned)ctas, C_WARPS * 32, 0, s>>>(P);
-            else if (gs == 8) cells_kernel<8, 8><<<(unsigned)ctas, C_WARPS * 32, 0, s>>>(P);
-            else
-#endif
-            cells_kernel<8, 16><<<(unsigned)ctas, C_WARPS * 32, 0, s>>>(P);   // measured (pipelined step): groups of 32 / 16 / 8 / 4 lanes = 99.4 / 97.4 / 101.1 / 108.4 us
+            cells_kernel<<<(unsigned)ctas, C_WARPS * 32, 0, s>>>(P);
             if (io.inst_bits && io.inst_masks) {
                 const size_t want_d = (inst_words + C_THREADS - 1) / C_THREADS, cap_d = (size_t)sm_count * 16;
                 inst_dense_kernel<<<(unsigned)(want_d < cap_d ? want_d : cap_d), C_THREADS, 0, s>>>(P.inst_bits, io.inst_masks, inst_words);

@@ -60,15 +60,9 @@ extern "C" __attribute__((visibility("default"))) int btpost_debug_phase_cycles(
 namespace bt {
 
 constexpr int NMS_CHUNK = 64;
-#ifndef NMS_MINB_512
-#define NMS_MINB_512 3   // CTAs per SM the 512-thread variant is compiled for (3: 40 registers, measured in profiles/r02c_summary.md)
-#endif
-#ifndef NMS_WIN_512
-#define NMS_WIN_512 1024  // sorted candidates staged per window by the 512-thread variant
-#endif
-#ifndef A_SUBS_WIDE
-#define A_SUBS_WIDE 8
-#endif
+constexpr int NMS_MINB_512 = 3;     // CTAs per SM the 512-thread variant is compiled for (3: 40 registers, measured in profiles/r02c_summary.md)
+constexpr int NMS_WIN_512 = 1024;   // sorted candidates staged per window by the 512-thread variant
+constexpr int A_SUBS_WIDE = 8;      // phase A threads per candidate of the 512- and 1024-thread variants
 constexpr int SORT_REG_MAX = 16384;  // keys sorted in registers (16 per thread) up to this many
 constexpr int SORT_SMALL_MAX = 4096; // same for the 512-thread variant (8 per thread): its shared memory stays below 80 KB
 constexpr int GM_THREADS = 256;      // match_kernel block
@@ -158,7 +152,6 @@ struct K2Params {
     int32_t *acc, *inst_area, *inst_inter;
     double *seg_prob_sum;
     int region0_bytes;    // shared region 0: list of candidate indices in NMS order
-    int bucket_global;    // longer lists: bucket rank sort with its pairs in the workspace (developer switch, default on)
     size_t sort_stride;   // u64 words per image of sort_keys
     int bucket_max;       // longest list the bucket rank sort takes (shared memory behind region 0 holds its pairs)
     int crop, PW, PH; float rx, ry; short4 *det_region;   // crop regions for the mask kernel
@@ -501,7 +494,7 @@ __global__ void __launch_bounds__(K2_THREADS, K2_THREADS == 512 ? NMS_MINB_512 :
         unsigned long long *gslice = P.sort_keys + (size_t)b * P.sort_stride;
         unsigned long long *sbuf = reinterpret_cast<unsigned long long *>(smem_raw + P.region0_bytes);
         if (M_all <= P.bucket_max) sorted = bucket_sort<K2_THREADS, false>(cscore, M_all, sbuf, reinterpret_cast<int *>(sbuf + Mp_all), s_sidx);
-        else if (P.bucket_global) {
+        else {
             sorted = bucket_sort<K2_THREADS, true>(cscore, M_all, gslice, reinterpret_cast<int *>(sbuf), reinterpret_cast<uint32_t *>(gslice + Mp_all));
             if (sorted) gidx = reinterpret_cast<const uint32_t *>(gslice + Mp_all);
         }
@@ -1161,8 +1154,7 @@ int launch_nms_match(const BtParams &p, const BtIO &io, const Workspace &w, cuda
     // SM for a second image and for CTAs of the other batches' kernels (btpost.Pipeline asks for it: 93.8 vs 98.7 us per
     // pipelined step, profiles/r02c_nms_threads.txt).  The 1024-thread variant (default) sorts lists of up to 16 384
     // candidates in shared memory; the small ones keep the pairs of lists above 4096 in the workspace.
-    const int nt_req = p.nms_threads ? p.nms_threads : dbg_env_int("BTPOST_NMS_NT", 1024);
-    const int nt = nt_req == 512 ? 512 : (nt_req == 256 ? 256 : 1024);
+    const int nt = p.nms_threads == 512 ? 512 : (p.nms_threads == 256 ? 256 : 1024);
     const int sort_max = nt <= 512 ? SORT_SMALL_MAX : SORT_REG_MAX;
     const int sort_slots = P.cap_pow2 < 1024 ? 1024 : (P.cap_pow2 > sort_max ? sort_max : P.cap_pow2);
     const size_t region0 = align_up((size_t)sort_slots * 4, 16);
@@ -1185,8 +1177,7 @@ int launch_nms_match(const BtParams &p, const BtIO &io, const Workspace &w, cuda
         } else {
             while (want > 0 && fixed + 8 * want > smem_a) want -= 32;
         }
-        P.bucket_max = dbg_env_int("BTPOST_NMS_BUCKET", 1) ? (int)want : 0;
-        P.bucket_global = dbg_env_int("BTPOST_NMS_BUCKET_G", 1);
+        P.bucket_max = (int)want;
         P.sort_stride = sort_stride_u64((size_t)P.cap);
     }
     // dynamic + static (~7 KB) shared memory of nms_kernel must stay below the 227 KB an SM offers one CTA: with 220 KB
@@ -1211,25 +1202,12 @@ int launch_nms_match(const BtParams &p, const BtIO &io, const Workspace &w, cuda
         attr_done[attr_dev] = true;
     }
     if (parts & BT_NMS_SORT_SWEEP) {
-        // Developer switch BTPOST_NMS_PRIO=1: launch the NMS kernel (the long pole of a step; needs whole SMs) with the
-        // highest launch priority.  Measured: one batch in flight 205.6 -> 198.5 us, four in flight 539 k -> 524 k
-        // images/s, so it is off by default.
-        int prio = 0;
-        if (dbg_env_int("BTPOST_NMS_PRIO", 0) != 0) {   // debug build only
-            int lo = 0, hi = 0;
-            if (cudaDeviceGetStreamPriorityRange(&lo, &hi) != cudaSuccess) return BT_ERR_CUDA;
-            prio = hi;   // hi = numerically lowest = highest priority
-        }
-        cudaLaunchConfig_t cfg = {};
-        cfg.gridDim = dim3(p.batch); cfg.blockDim = dim3(nt); cfg.dynamicSmemBytes = smem_a; cfg.stream = s;
-        cudaLaunchAttribute at[1];
-        at[0].id = cudaLaunchAttributePriority;
-        at[0].val.priority = prio;
-        cfg.attrs = at; cfg.numAttrs = prio != 0 ? 1 : 0;
-        if ((nt == 256   ? cudaLaunchKernelEx(&cfg, nms_kernel<256>, P)
-             : nt == 512 ? cudaLaunchKernelEx(&cfg, nms_kernel<512>, P)
-                         : cudaLaunchKernelEx(&cfg, nms_kernel<1024>, P)) != cudaSuccess)
-            return BT_ERR_CUDA;
+        // measured and not kept: the highest launch priority for this kernel (the long pole of a step; it needs whole
+        // SMs): one batch in flight 205.6 -> 198.5 us, but four in flight 539 k -> 524 k images/s
+        if (nt == 256) nms_kernel<256><<<p.batch, nt, smem_a, s>>>(P);
+        else if (nt == 512) nms_kernel<512><<<p.batch, nt, smem_a, s>>>(P);
+        else nms_kernel<1024><<<p.batch, nt, smem_a, s>>>(P);
+        if (cudaGetLastError() != cudaSuccess) return BT_ERR_CUDA;
     }
     if (parts & BT_NMS_GATHER) coeff_gather_kernel<<<dim3((p.max_det + 7) / 8, p.batch), GM_THREADS, 0, s>>>(P);
     if (parts & BT_NMS_PLAN) plan_kernel<<<p.batch, GM_THREADS, 0, s>>>(P);

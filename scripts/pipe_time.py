@@ -1,10 +1,9 @@
-"""Developer tool: pipelined step time (btpost.Pipeline, distinct inputs per slot, CUDA events) of whatever library
-BTPOST_LIB names (default: the switch build `make sw`, which reads the BTPOST_* tuning variables), plus the first
-image's detection count and Dice as a sanity check.  usage: python scripts/pipe_time.py [depth] [steps] [label]"""
+"""Developer tool: pipelined step time (btpost.Pipeline, distinct inputs per slot, CUDA events) of the library
+(BTPOST_LIB names another build), plus the first image's detection count and Dice as a sanity check.
+usage: python scripts/pipe_time.py [depth] [steps] [label]"""
 import os, sys
 from pathlib import Path
 ROOT = Path(__file__).resolve().parents[1]
-os.environ.setdefault("BTPOST_LIB", str(ROOT / "multitask-bonetumor-yolo_b200" / "btpost" / "libbtpost_sw.so"))
 sys.path[:0] = [str(ROOT), str(ROOT / "multitask-bonetumor-yolo_b200")]
 import torch
 from btpost import DeviceSweep, Pipeline, PostConfig, synth
@@ -16,12 +15,6 @@ label = sys.argv[3] if len(sys.argv) > 3 else ""
 B, S = 64, 640
 dev = torch.device("cuda:0")
 torch.zeros(1, device=dev)
-if os.environ.get("L2G"):   # cudaLimitMaxL2FetchGranularity (0x05): DRAM -> L2 fetch size hint, default 64 bytes
-    import ctypes
-    rt = ctypes.CDLL("libcudart.so.12")
-    rc = rt.cudaDeviceSetLimit(5, ctypes.c_size_t(int(os.environ["L2G"])))
-    v = ctypes.c_size_t(0); rt.cudaDeviceGetLimit(ctypes.byref(v), 5)
-    print("cudaLimitMaxL2FetchGranularity ->", rc, v.value, flush=True)
 first = synth.make_batch_device(synth.SynthConfig(batch=B, img_size=S, seed=20262), dev)
 cfg = PostConfig(batch=B, img_size=S, nms_threads=int(os.environ.get("NMS_NT", "0")))
 sweep = DeviceSweep(cfg.nc, map_iou_thresholds(), (1, 10, 100), capacity=1 << 23, max_det_per_image=300, device=dev) if os.environ.get("SWEEP") else None
@@ -46,6 +39,6 @@ run(4 * depth)
 t20 = min(run(20) for _ in range(5))
 tn = min(run(steps) for _ in range(3))
 o = pipe.procs[0].out
-sw = " ".join(f"{k}={v}" for k, v in sorted(os.environ.items()) if (k.startswith("BTPOST_") or k in ("NMS_NT", "SWEEP", "FILL", "L2G")) and k != "BTPOST_LIB")
+opts = " ".join(f"{k}={v}" for k, v in sorted(os.environ.items()) if k in ("NMS_NT", "SWEEP", "FILL"))
 print(f"{label:24s} depth {depth}: {tn:7.2f} us/step over {steps} steps, {t20:7.2f} over 20 | dets {o['det_count'][:3].tolist()} "
-      f"dice {o['seg_dice'][0].item():.6f} uni {o['uni_dice'][0].item():.6f} | {sw}", flush=True)
+      f"dice {o['seg_dice'][0].item():.6f} uni {o['uni_dice'][0].item():.6f} | {opts}", flush=True)
