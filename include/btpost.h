@@ -160,6 +160,17 @@ typedef struct BtIO {
                                    gt_ignore)                                                            */
     const int32_t *image_base;  /* [1] optional, device: added to BtParams.image_offset when the records are written, so
                                    that a step captured into a CUDA graph can be replayed for different batches  */
+    void *seg_sweep;            /* optional sweep state (same format as `sweep`, 16-byte aligned) for the v3 segmentation mAP
+                                   (a11, src/running_main_v3.py:478-498): finalize_kernel appends ONE record per image -- the
+                                   projector mask scored by its mean foreground probability against the GT mask, class 0.
+                                   Needs seg_img3 and seg_prob_sum.  Record fields:
+                                     matched / ignored  bit a * T + t: mask IoU >= min(iou_thrs[t], 1 - 1e-10); ignored = matched ?
+                                                        |G| outside area range a : |P| outside area range a (COCOeval)
+                                     score_key          desc_key(seg_prob_sum / (|P| + 1e-6)), fp32 as the reference computes it
+                                     image              BtParams.image_offset + *image_base + index in the batch
+                                     rank = class_rank = label = 0
+                                   Header: N_RECORDS, N_IMAGES, NPIG[a][0] (|G| inside area range a); the FSUM slots stay
+                                   unused.  btpost_sweep_accumulate with nc = 1, max_det_per_image = 1 gives the tables. */
 } BtIO;
 
 /* Library / build identification. */
@@ -210,7 +221,8 @@ BTPOST_API int btpost_run(const BtParams *p, const BtIO *io, void *ws, size_t ws
  * With BtIO.sweep set, btpost_run / btpost_nms_match / btpost_masks append to it on the device (no host work per
  * batch): match_kernel writes one record per kept detection and adds the batch's non-ignored GT counts and image
  * count, finalize_kernel adds the per-image Dice / IoU (2^-40 fixed point, so the sums do not depend on the order of
- * the atomics).  Every header slot is a plain sum, so shards are merged by ONE all-reduce(SUM) over the header (the
+ * the atomics).  A second state at BtIO.seg_sweep collects the v3 segmentation mAP (one record per image, nc = 1).
+ * Every header slot is a plain sum, so shards are merged by ONE all-reduce(SUM) over the header (the
  * metric-counter all-reduce of the north star) plus one all-gather of the records (AP needs the global score order).
  * The caller may point BtIO.cm / seg_cnt4 / uni_cnt4 into the header's user slots so that they travel with it. */
 #define BT_SWEEP_HEADER_I64 512

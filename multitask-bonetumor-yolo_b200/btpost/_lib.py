@@ -46,7 +46,7 @@ _IO_FIELDS = [
     "cm_pos", "seg_img3", "seg_dice", "seg_iou", "uni_img3", "uni_dice", "uni_iou", "inst_area", "inst_inter",
     "seg_mask", "seg_logits", "uni_mask", "inst_bits", "inst_masks",
     "dt_match", "dt_ignore", "gt_ignore",
-    "seg_prob_sum", "gt_rows_total", "sweep", "image_base",
+    "seg_prob_sum", "gt_rows_total", "sweep", "image_base", "seg_sweep",
 ]
 
 

@@ -218,6 +218,9 @@ class PostProcessor:
         self.sweep = sweep                # a btpost.sweep.DeviceSweep: records are appended by the library itself
         if sweep is not None and not cfg.with_coco:
             raise ValueError("a sweep needs with_coco=True (the records are written by the COCO matching)")
+        if sweep is not None and sweep.seg_ptr is not None and not cfg.with_seg_map:
+            raise ValueError("a sweep with a segmentation-mAP ring (seg_map_capacity > 0) needs with_seg_map=True "
+                             "(the records are scored with the mask kernel's seg_prob_sum)")
         self._empty_gt = torch.zeros(1, 6, dtype=torch.float32, device=dev)
         self.image_base = torch.zeros(1, dtype=torch.int32, device=dev)   # global index of image 0, read by the kernels
 
@@ -278,6 +281,7 @@ class PostProcessor:
             setattr(io, k, v.data_ptr())
         if self.sweep is not None:
             io.sweep = self.sweep.ptr
+            io.seg_sweep = self.sweep.seg_ptr
             io.image_base = self.image_base.data_ptr()
         self._keepalive = (head, protos, det_boxes_gt, masks_gt, proj_weight, maps, coeffs)
         return io

@@ -15,13 +15,14 @@ Per batch the CUDA library leaves integer counters and per-detection COCO match 
     not depend on how images were sharded.
 
 `SweepState` runs as tensor ops on whatever device the state lives on; it is the host-logic restatement used by
-the gloo tests on CPU and by the v3 segmentation mAP (one record per image, `btpost.segmap`).
+the gloo tests on CPU and by the host path of the v3 segmentation mAP (one record per image, `btpost.segmap`).
 
 `DeviceSweep` is the production path for the detection sweep (BASELINE config 5): the CUDA library itself appends the
 per-detection records, GT counts, image count and Dice / IoU sums to a caller-owned device buffer while it processes a
 batch (`BtIO.sweep`, zero host work per batch), shards are merged by ONE all-reduce of the 4 KB header and one
 `all_gather_into_tensor` of the records, and COCOeval.accumulate runs as CUDA kernels (`btpost_sweep_accumulate`:
-radix sort + scans + 101-point lookup).
+radix sort + scans + 101-point lookup).  With `seg_map_capacity` it also owns the v3 segmentation-mAP state, to which the
+mask stage appends one record per image (`BtIO.seg_sweep`); it rides in the same collectives (`merge_sweeps`).
 """
 from __future__ import annotations
 
@@ -274,31 +275,57 @@ def merge_shards(hdr: torch.Tensor, records: torch.Tensor, group=None):
     metric-counter all-reduce), `records` uint8 [capacity, 32] of which the first min(hdr[0], capacity) rows are valid
     (one `all_gather_into_tensor`, padded to the largest shard).  Returns (n_per_rank list, records of all ranks
     concatenated in rank order).  Device-agnostic (NCCL on the GPU box, gloo in the CPU tests)."""
-    n_local = int(min(int(hdr[_lib.SWEEP_N_RECORDS]), records.shape[0]))
+    ns, merged = merge_sweeps([hdr], [records], group)
+    return ns[0], merged[0]
+
+
+@torch.no_grad()
+def merge_sweeps(hdrs, rings, group=None):
+    """`merge_shards` for several sweep states at once (the detection sweep and the segmentation-mAP sweep) with the
+    same three collectives: the record counts in one all-gather, the headers, concatenated, in ONE all-reduce (each
+    `hdrs[s]` is summed in place), the valid records of every state in one `all_gather_into_tensor` (each state padded to
+    its largest shard).  Returns (ns, merged): per state, the n_per_rank list and the records of all ranks concatenated
+    in rank order."""
+    S = len(hdrs)
+    n_local = [int(min(int(h[_lib.SWEEP_N_RECORDS]), r.shape[0])) for h, r in zip(hdrs, rings)]
     if not (dist.is_available() and dist.is_initialized()) or dist.get_world_size(group) == 1:
-        return [n_local], records[:n_local]
-    W = dist.get_world_size(group)
-    counts = torch.zeros(W, dtype=torch.int64, device=hdr.device)
-    dist.all_gather_into_tensor(counts, torch.tensor([n_local], dtype=torch.int64, device=hdr.device), group=group)
-    dist.all_reduce(hdr, group=group)
-    ns = [int(v) for v in counts.tolist()]
-    cap = max(max(ns), 1)
-    if records.shape[0] >= cap:
-        send = records[:cap]
-    else:   # a smaller ring than the largest shard: pad (rows beyond n_local are never read)
-        send = torch.zeros(cap, REC_BYTES, dtype=torch.uint8, device=records.device)
-        send[:n_local] = records[:n_local]
-    allrec = torch.empty(W * cap, REC_BYTES, dtype=torch.uint8, device=records.device)
+        return [[n] for n in n_local], [r[:n] for r, n in zip(rings, n_local)]
+    W, dev = dist.get_world_size(group), hdrs[0].device
+    counts = torch.zeros(W * S, dtype=torch.int64, device=dev)
+    dist.all_gather_into_tensor(counts, torch.tensor(n_local, dtype=torch.int64, device=dev), group=group)
+    if S == 1:
+        dist.all_reduce(hdrs[0], group=group)
+    else:
+        cat = torch.cat(list(hdrs))
+        dist.all_reduce(cat, group=group)
+        for h, v in zip(hdrs, cat.split([h.numel() for h in hdrs])):
+            h.copy_(v)
+    ns = [[int(v) for v in col] for col in zip(*counts.view(W, S).tolist())]   # ns[s][rank]
+    caps = [max(max(n), 1) for n in ns]
+    rows, rdev = sum(caps), rings[0].device
+    if S == 1 and rings[0].shape[0] >= caps[0]:
+        send = rings[0][:caps[0]]
+    else:   # a ring smaller than the largest shard, or several states back to back: pad (rows beyond n_local are never read)
+        send = torch.zeros(rows, REC_BYTES, dtype=torch.uint8, device=rdev)
+        o = 0
+        for r, n, c in zip(rings, n_local, caps):
+            send[o: o + n] = r[:n]
+            o += c
+    allrec = torch.empty(W * rows, REC_BYTES, dtype=torch.uint8, device=rdev)
     dist.all_gather_into_tensor(allrec, send.contiguous(), group=group)
-    if all(n == cap for n in ns):
-        return ns, allrec                      # equal shards: the gathered buffer is the merged list
+    if S == 1 and all(n == caps[0] for n in ns[0]):
+        return ns, [allrec]                    # equal shards: the gathered buffer is the merged list
     # ragged shards: contiguous 8-byte copies (torch.cat on [n, 32] uint8 rows copies byte by byte: 13 ms for 52 MB on a B200)
-    merged = torch.empty(sum(ns), REC_BYTES, dtype=torch.uint8, device=records.device)
-    m64, a64, o = merged.view(torch.int64), allrec.view(torch.int64), 0
-    for r in range(W):
-        m64[o: o + ns[r]].copy_(a64[r * cap: r * cap + ns[r]])
-        o += ns[r]
-    return ns, merged
+    a64, out, base = allrec.view(torch.int64), [], 0
+    for s in range(S):
+        merged = torch.empty(sum(ns[s]), REC_BYTES, dtype=torch.uint8, device=rdev)
+        m64, o = merged.view(torch.int64), 0
+        for r in range(W):
+            m64[o: o + ns[s][r]].copy_(a64[r * rows + base: r * rows + base + ns[s][r]])
+            o += ns[s][r]
+        out.append(merged)
+        base += caps[s]
+    return ns, out
 
 
 def decode_records(records: torch.Tensor, T: int):
@@ -317,24 +344,29 @@ def decode_records(records: torch.Tensor, T: int):
 class DeviceSweep:
     """Sweep state on one GPU, filled by the CUDA library (`PostProcessor.sweep = DeviceSweep(...)` or
     `Pipeline(..., sweep=...)`).  `capacity` = records the ring can hold (one per kept detection of this rank's
-    shard; 32 bytes each)."""
+    shard; 32 bytes each).  `seg_map_capacity` > 0 adds a second sweep state for the v3 segmentation mAP
+    (`BtIO.seg_sweep`: one record per image, so the number of images of this rank's shard; needs
+    `PostConfig.with_seg_map`); `finish()` then also returns the `seg_`-prefixed mAP keys."""
 
     def __init__(self, nc: int, iou_thrs, max_dets=(1, 10, 100), capacity: int = 1 << 20, max_det_per_image: int = 300,
-                 device="cuda:0"):
+                 device="cuda:0", seg_map_capacity: int = 0):
         self.lib = _lib.load()
         self.nc, self.iou_thrs, self.max_dets = nc, [float(t) for t in iou_thrs], tuple(int(m) for m in max_dets)
         self.T, self.capacity, self.K = len(self.iou_thrs), int(capacity), int(max_det_per_image)
+        self.seg_map_capacity = int(seg_map_capacity)
         self.device = torch.device(device)
         if self.device.type != "cuda":
             raise RuntimeError("DeviceSweep lives on a CUDA device (the records are written by the CUDA library)")
         if not (0 < len(self.max_dets) <= 4) or nc > 16 or 4 * self.T > 64:
             raise ValueError("DeviceSweep: at most 4 maxDets, 16 classes, 16 IoU thresholds")
-        nbytes = C.c_size_t()
-        _lib.check(self.lib.btpost_sweep_bytes(C.c_int64(self.capacity), C.byref(nbytes)), "btpost_sweep_bytes")
-        self.buf = torch.zeros((nbytes.value + 7) // 8, dtype=torch.int64, device=self.device)   # torch allocations are 512-byte aligned
+        if self.seg_map_capacity < 0:
+            raise ValueError("DeviceSweep: seg_map_capacity must be >= 0")
+        self.buf, self.hdr, self.records = self._state(self.capacity)
         self.ptr = self.buf.data_ptr()
-        self.hdr = self.buf[:HDR]
-        self.records = self.buf[HDR:].view(torch.uint8)[: self.capacity * REC_BYTES].view(self.capacity, REC_BYTES)
+        self.seg_buf = self.seg_hdr = self.seg_records = self.seg_ptr = None
+        if self.seg_map_capacity:
+            self.seg_buf, self.seg_hdr, self.seg_records = self._state(self.seg_map_capacity)
+            self.seg_ptr = self.seg_buf.data_ptr()
         u = _lib.SWEEP_USER
         self.cm = self.hdr[u: u + nc * nc].view(nc, nc)
         self.seg_cnt4 = self.hdr[u + 256: u + 260]
@@ -343,18 +375,32 @@ class DeviceSweep:
         self._md = (C.c_int32 * len(self.max_dets))(*self.max_dets)
         self.reset()
 
+    def _state(self, capacity):
+        """(buffer, header view, record-ring view) of one sweep state of `capacity` records."""
+        nbytes = C.c_size_t()
+        _lib.check(self.lib.btpost_sweep_bytes(C.c_int64(capacity), C.byref(nbytes)), "btpost_sweep_bytes")
+        buf = torch.zeros((nbytes.value + 7) // 8, dtype=torch.int64, device=self.device)   # torch allocations are 512-byte aligned
+        return buf, buf[:HDR], buf[HDR:].view(torch.uint8)[: capacity * REC_BYTES].view(capacity, REC_BYTES)
+
     def reserve(self, total_records: int, world: int = 1):
         """Optional: warm torch's caching allocator for `finish()` on a sweep of `total_records` records over `world`
-        ranks (the gathered record buffer, the merged copy and the accumulate scratch), so that the end of the sweep does
-        not pay cudaMalloc calls while the GPU waits."""
-        sb = C.c_size_t()
-        _lib.check(self.lib.btpost_sweep_accumulate_bytes(C.c_int64(int(total_records)), C.byref(sb)), "btpost_sweep_accumulate_bytes")
-        per = -(-int(total_records) // max(world, 1))
-        keep = [torch.empty(sb.value, dtype=torch.uint8, device=self.device),
-                torch.empty(max(world * per, 1), REC_BYTES, dtype=torch.uint8, device=self.device),
-                torch.empty(max(int(total_records), 1), REC_BYTES, dtype=torch.uint8, device=self.device),
-                torch.empty(self.T, 101, self.nc, 4, len(self.max_dets), dtype=torch.float64, device=self.device),
-                torch.empty(self.T, self.nc, 4, len(self.max_dets), dtype=torch.float64, device=self.device)]
+        ranks (the gathered record buffer, the merged copy and the accumulate scratch, for the segmentation ring too), so
+        that the end of the sweep does not pay cudaMalloc calls while the GPU waits."""
+        def scratch(n):
+            sb = C.c_size_t()
+            _lib.check(self.lib.btpost_sweep_accumulate_bytes(C.c_int64(int(n)), C.byref(sb)), "btpost_sweep_accumulate_bytes")
+            return torch.empty(sb.value, dtype=torch.uint8, device=self.device)
+
+        def tables(nc):
+            M = len(self.max_dets)
+            return [torch.empty(self.T, 101, nc, 4, M, dtype=torch.float64, device=self.device),
+                    torch.empty(self.T, nc, 4, M, dtype=torch.float64, device=self.device)]
+        world = max(world, 1)
+        per, seg = -(-int(total_records) // world), self.seg_map_capacity
+        rows = lambda n: torch.empty(max(n, 1), REC_BYTES, dtype=torch.uint8, device=self.device)
+        keep = [scratch(total_records), rows(world * (per + seg)), rows(int(total_records))] + tables(self.nc)
+        if seg:
+            keep += [scratch(world * seg), rows(per + seg), rows(world * seg)] + tables(1)
         del keep   # back to the allocator's cache
 
     def counters(self):
@@ -365,8 +411,30 @@ class DeviceSweep:
     def reset(self, stream=None):
         st = stream if stream is not None else torch.cuda.current_stream(self.device)
         with torch.cuda.device(self.device):
-            _lib.check(self.lib.btpost_sweep_reset(C.c_void_p(self.ptr), C.c_int64(self.capacity), C.c_void_p(st.cuda_stream)),
-                       "btpost_sweep_reset")
+            for ptr, cap in ((self.ptr, self.capacity), (self.seg_ptr, self.seg_map_capacity)):
+                if ptr is not None:
+                    _lib.check(self.lib.btpost_sweep_reset(C.c_void_p(ptr), C.c_int64(cap), C.c_void_p(st.cuda_stream)),
+                               "btpost_sweep_reset")
+
+    def _accumulate(self, rec, n, hdr, nc, max_det_per_image, num_images_bound):
+        """btpost_sweep_accumulate on `n` merged records (reordered in place) -> (precision, recall) numpy tables."""
+        T, A, M = self.T, 4, len(self.max_dets)
+        precision = torch.empty(T, 101, nc, A, M, dtype=torch.float64, device=self.device)
+        recall = torch.empty(T, nc, A, M, dtype=torch.float64, device=self.device)
+        sb = C.c_size_t()
+        _lib.check(self.lib.btpost_sweep_accumulate_bytes(C.c_int64(n), C.byref(sb)), "btpost_sweep_accumulate_bytes")
+        scratch = torch.empty(sb.value, dtype=torch.uint8, device=self.device)
+        npig = hdr[_lib.SWEEP_NPIG: _lib.SWEEP_NPIG + 64]
+        bound = num_images_bound if num_images_bound is not None else (int(rec[:, 20:24].contiguous().view(torch.int32).max()) + 1 if n else 1)
+        st = torch.cuda.current_stream(self.device)
+        with torch.cuda.device(self.device):
+            rc = self.lib.btpost_sweep_accumulate(
+                C.c_void_p(rec.data_ptr() if n else 0), C.c_int64(n), C.c_void_p(npig.data_ptr()), C.c_void_p(self.rec_thrs.data_ptr()),
+                C.c_int32(101), C.c_int32(nc), C.c_int32(T), self._md, C.c_int32(M), C.c_int32(max_det_per_image), C.c_int64(bound),
+                C.c_void_p(precision.data_ptr()), C.c_void_p(recall.data_ptr()), C.c_void_p(scratch.data_ptr()), C.c_size_t(sb.value),
+                C.c_void_p(st.cuda_stream))
+        _lib.check(rc, "btpost_sweep_accumulate")
+        return precision, recall
 
     @torch.no_grad()
     def finish(self, group=None, num_images_bound: int | None = None, timings: dict | None = None) -> dict:
@@ -383,45 +451,44 @@ class DeviceSweep:
                 timings[name] = (now - _t[0]) * 1e3
                 _t[0] = now
 
-        n_here = int(self.hdr[_lib.SWEEP_N_RECORDS])
+        seg = self.seg_map_capacity > 0
+        states = [("", self.hdr, self.records, self.capacity)]
+        if seg:
+            states.append(("segmentation ", self.seg_hdr, self.seg_records, self.seg_map_capacity))
+        n_here = [int(h[_lib.SWEEP_N_RECORDS]) for _, h, _, _ in states]
         _mark("read_count")
-        if n_here > self.capacity:
-            raise RuntimeError(f"DeviceSweep ring too small: {n_here} records offered, capacity {self.capacity}")
-        hdr = self.hdr.clone()
-        ns, rec = merge_shards(hdr, self.records, group)
+        for (what, _, _, cap), n in zip(states, n_here):
+            if n > cap:
+                raise RuntimeError(f"DeviceSweep {what}ring too small: {n} records offered, capacity {cap}")
+        hdrs = [h.clone() for _, h, _, _ in states]
+        ns, recs = merge_sweeps(hdrs, [r for _, _, r, _ in states], group)
         _mark("merge_shards")
-        n = int(sum(ns))
-        if n and rec.data_ptr() == self.records.data_ptr():
-            rec = rec.clone()                              # the sort reorders in place: keep the ring as it was
-        rec = rec.contiguous()
+        for i, ((_, _, ring, _), rec) in enumerate(zip(states, recs)):
+            if sum(ns[i]) and rec.data_ptr() == ring.data_ptr():
+                rec = rec.clone()                          # the sort reorders in place: keep the ring as it was
+            recs[i] = rec.contiguous()
+        hdr, n = hdrs[0], int(sum(ns[0]))
         n_images = int(hdr[_lib.SWEEP_N_IMAGES])
-        T, A, M, nc = self.T, 4, len(self.max_dets), self.nc
-        precision = torch.empty(T, 101, nc, A, M, dtype=torch.float64, device=self.device)
-        recall = torch.empty(T, nc, A, M, dtype=torch.float64, device=self.device)
-        sb = C.c_size_t()
-        _lib.check(self.lib.btpost_sweep_accumulate_bytes(C.c_int64(n), C.byref(sb)), "btpost_sweep_accumulate_bytes")
-        scratch = torch.empty(sb.value, dtype=torch.uint8, device=self.device)
-        npig = hdr[_lib.SWEEP_NPIG: _lib.SWEEP_NPIG + 64]
-        bound = num_images_bound if num_images_bound is not None else (int(rec[:, 20:24].contiguous().view(torch.int32).max()) + 1 if n else 1)
-        st = torch.cuda.current_stream(self.device)
-        with torch.cuda.device(self.device):
-            rc = self.lib.btpost_sweep_accumulate(
-                C.c_void_p(rec.data_ptr() if n else 0), C.c_int64(n), C.c_void_p(npig.data_ptr()), C.c_void_p(self.rec_thrs.data_ptr()),
-                C.c_int32(101), C.c_int32(nc), C.c_int32(T), self._md, C.c_int32(M), C.c_int32(self.K), C.c_int64(bound),
-                C.c_void_p(precision.data_ptr()), C.c_void_p(recall.data_ptr()), C.c_void_p(scratch.data_ptr()), C.c_size_t(sb.value),
-                C.c_void_p(st.cuda_stream))
-        _lib.check(rc, "btpost_sweep_accumulate")
+        nc = self.nc
+        precision, recall = self._accumulate(recs[0], n, hdr, nc, self.K, num_images_bound)
+        if seg:
+            seg_tables = self._accumulate(recs[1], int(sum(ns[1])), hdrs[1], 1, 1, num_images_bound)
         _mark("accumulate")
         pr, rcl = precision.cpu().numpy(), recall.cpu().numpy()
         h = hdr.cpu().numpy()
         res = summarize(pr, rcl, self.iou_thrs, self.max_dets)
+        if seg:
+            spr, srcl = (t.cpu().numpy() for t in seg_tables)
+            res.update({f"seg_{k}": v for k, v in summarize(spr, srcl, self.iou_thrs, self.max_dets).items()})
+            # seg_precision is the pixel precision of the projector mask: the seg-mAP tables carry the seg_map_ prefix
+            res.update(n_seg_records=int(sum(ns[1])), seg_map_precision=spr, seg_map_recall=srcl)
         _mark("summarize")
         ni = max(n_images, 1)
         u = _lib.SWEEP_USER
         tp, fp, fn, tn = [int(v) for v in h[u + 256: u + 260]]
         fs = h[_lib.SWEEP_FSUM: _lib.SWEEP_FSUM + 4].astype(np.float64) / FSUM_SCALE
         res.update({
-            "n_images": n_images, "n_records": n, "records_per_rank": ns, "cm": torch.from_numpy(h[u: u + nc * nc].reshape(nc, nc).copy()),
+            "n_images": n_images, "n_records": n, "records_per_rank": ns[0], "cm": torch.from_numpy(h[u: u + nc * nc].reshape(nc, nc).copy()),
             "seg_f1": 2 * tp / (2 * tp + fp + fn) if (2 * tp + fp + fn) else 0.0,
             "seg_precision": tp / (tp + fp) if (tp + fp) else 0.0, "seg_recall": tp / (tp + fn) if (tp + fn) else 0.0,
             "seg_accuracy": (tp + tn) / max(tp + tn + fp + fn, 1),

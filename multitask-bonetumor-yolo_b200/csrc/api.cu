@@ -75,6 +75,8 @@ static int check_stage3(const BtParams *p, const BtIO *io) {
     if ((io->seg_mask && !aligned16(io->seg_mask)) || (io->uni_mask && !aligned16(io->uni_mask))) return BT_ERR_MISALIGNED;
     if (io->inst_masks && !io->inst_bits) return BT_ERR_BAD_ARG;   // the bytes are expanded from the bits
     if ((io->inst_bits && !aligned16(io->inst_bits)) || (io->inst_masks && !aligned16(io->inst_masks))) return BT_ERR_MISALIGNED;
+    if (io->seg_sweep && (!io->seg_img3 || !io->seg_prob_sum)) return BT_ERR_BAD_ARG;   // the record's IoU and score inputs
+    if (io->seg_sweep && !aligned16(io->seg_sweep)) return BT_ERR_MISALIGNED;
     return BT_OK;
 }
 

@@ -33,6 +33,20 @@ namespace bt {
 // for x > 1.5 * 2^-24 (pinned against torch in tests/golden/make_golden.py).
 __device__ __forceinline__ bool sigmoid_gt_half(float x) { return x > 8.940696716308594e-08f; }
 
+// Order-preserving image of an fp32 score: ascending key = descending score (sort keys of the NMS, sweep records).
+__device__ __forceinline__ uint32_t desc_key(float s) {
+    uint32_t u = __float_as_uint(s);
+    if (s != s) return 0u;                                   // NaN sorts first
+    if (u == 0x80000000u) u = 0u;                            // -0.0 == +0.0
+    uint32_t asc = (u & 0x80000000u) ? ~u : (u | 0x80000000u);
+    return ~asc;                                             // smaller key = higher score
+}
+
+// COCOeval area ranges (all, small, medium, large), bounds inclusive: an area lies outside range a when it is below
+// COCO_AREA_LO[a] or above COCO_AREA_HI[a].  Brace initialisers of a kernel's local const arrays.
+#define COCO_AREA_LO {0.0, 0.0, 32.0 * 32.0, 96.0 * 96.0}
+#define COCO_AREA_HI {1e10, 32.0 * 32.0, 96.0 * 96.0, 1e10}
+
 // Crop region of a detection at prototype resolution: pixels with r>=y1 & r<y2 & c>=x1 & c<x2
 // on the box scaled by proto/img (Ultralytics crop_mask).  Returns false for an empty region.
 __device__ __forceinline__ bool crop_region(const float *o, int crop, float rx, float ry, int PW, int PH, int &r_lo,

@@ -28,7 +28,8 @@
 //                     an image's instance masks is a 64-bit atomic OR per block whose returned old word gives the
 //                     newly set bits (union counters without a pass over the union); the projector mask owns its
 //                     cells.  Instruction-issue bound.
-//   finalize_kernel   one warp per image: counters -> Dice / IoU / tp-fp-fn-tn.
+//   finalize_kernel   one warp per image: counters -> Dice / IoU / tp-fp-fn-tn, and the image's v3 segmentation-mAP
+//                     record when BtIO.seg_sweep is set.
 // tcgen05 is deliberately not used: K = 32 at <= 0.5 FLOP/B, and TF32/BF16 accumulation would break the bit
 // parity of the thresholded masks with the fp32 reference.
 #include <cuda.h>
@@ -73,6 +74,11 @@ struct K3Params {
     long long *sweep;       // optional sweep state: per-image Dice / IoU are added to its header (2^-40 fixed point)
     u64 valid_tab[9];       // valid-pixel mask of a block by (row class, column class): first / interior / last
     float inv_NBX;
+    // v3 segmentation mAP (BtIO.seg_sweep); appended last so that the fields above keep their parameter offsets
+    long long *seg_sweep;   // optional sweep state: one record per image, written by finalize_kernel
+    const int32_t *image_base;
+    int image_offset, T;
+    double thrs[BT_MAX_IOU_THRS];
 };
 
 __device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
@@ -851,6 +857,47 @@ __device__ __forceinline__ void det_end(const K3Params &P, const DetWork &w, uns
     }
 }
 
+// v3 segmentation-mAP record of image b (running_main_v3.py:478-498): the projector mask, scored by its mean foreground
+// probability, against the GT mask, class 0 -- what btpost/segmap.py builds from the same outputs, for COCOeval with one
+// detection and one GT per image.  seg_prob_sum is exact in double: each addend is an fp32 per-cell sum of
+// probabilities >= 0.5, hence a multiple of 2^-24, and the total stays below 2^20 even at 1024^2, so every partial sum
+// fits in 44 bits.  The score therefore depends neither on the order of m1_item's atomics nor on the sharding.
+__device__ __forceinline__ void seg_map_record(const K3Params &P, int b, long long inter, long long pp, long long gsum) {
+    long long *hdr = P.seg_sweep;
+    const int T = P.T;
+    const float score = __fdiv_rn(__double2float_rn(__ldcg(P.seg_prob_sum + b)), __fadd_rn((float)pp, 1e-6f));
+    const long long uni = pp + gsum - inter;
+    const double iou = uni > 0 ? (double)inter / (double)uni : 0.0;
+    const unsigned long long tmask = (T >= 16) ? 0xffffull : ((1ull << T) - 1ull);
+    unsigned long long hit = 0ull;
+    for (int t = 0; t < T; ++t) hit |= (iou >= fmin(P.thrs[t], 1 - 1e-10) ? 1ull : 0ull) << t;
+    const double area_lo[BT_NUM_AREA] = COCO_AREA_LO;
+    const double area_hi[BT_NUM_AREA] = COCO_AREA_HI;
+    unsigned long long matched = 0ull, ignored = 0ull;
+#pragma unroll
+    for (int a = 0; a < BT_NUM_AREA; ++a) {
+        const bool gt_ig = (double)gsum < area_lo[a] || (double)gsum > area_hi[a];
+        const bool dt_out = (double)pp < area_lo[a] || (double)pp > area_hi[a];
+        matched |= hit << (a * T);
+        ignored |= ((gt_ig ? hit : 0ull) | (dt_out ? (~hit & tmask) : 0ull)) << (a * T);   // a hit takes the GT's flag
+        if (!gt_ig) atomicAdd(reinterpret_cast<unsigned long long *>(hdr + BT_SWEEP_NPIG + a * BT_MAX_CLASSES), 1ull);
+    }
+    atomicAdd(reinterpret_cast<unsigned long long *>(hdr + BT_SWEEP_N_IMAGES), 1ull);
+    const long long pos = (long long)atomicAdd(reinterpret_cast<unsigned long long *>(hdr + BT_SWEEP_N_RECORDS), 1ull);
+    if (pos >= __ldcg(hdr + BT_SWEEP_CAPACITY)) return;   // ring full: reported through the header (N_RECORDS > CAPACITY)
+    BtSweepRecord r;
+    r.matched = matched;
+    r.ignored = ignored;
+    r.score_key = desc_key(score);
+    r.image = (uint32_t)(P.image_offset + (P.image_base ? __ldg(P.image_base) : 0) + b);
+    r.rank = 0; r.class_rank = 0; r.label = 0;
+    r.pad[0] = r.pad[1] = r.pad[2] = 0;
+    uint4 *dst = reinterpret_cast<uint4 *>(reinterpret_cast<BtSweepRecord *>(hdr + BT_SWEEP_HEADER_I64) + pos);
+    const uint4 *src = reinterpret_cast<const uint4 *>(&r);
+    dst[0] = src[0];
+    dst[1] = src[1];
+}
+
 // per-image epilogue: |G|, Dice / IoU (test_model.py:15-23)
 __device__ __forceinline__ void finalize_image(const K3Params &P, int b, int lane) {
     int gg = 0;
@@ -880,6 +927,7 @@ __device__ __forceinline__ void finalize_image(const K3Params &P, int b, int lan
             atomicAdd(fs, (unsigned long long)__double2ll_rn((double)v_dice * 1099511627776.0));
             atomicAdd(fs + 1, (unsigned long long)__double2ll_rn((double)v_iou * 1099511627776.0));
         }
+        if (lane == 0 && P.seg_sweep) seg_map_record(P, b, inter, pp, gsum);
     }
 }
 
@@ -1051,6 +1099,9 @@ int launch_masks(const BtParams &p, const BtIO &io, const Workspace &w, cudaStre
     P.seg_mask = io.seg_mask; P.uni_mask = io.uni_mask; P.seg_logits = io.seg_logits;
     P.seg_prob_sum = io.seg_prob_sum; P.sweep = static_cast<long long *>(io.sweep);
     P.inst_bits = reinterpret_cast<uint32_t *>(io.inst_bits); P.inst_masks = io.inst_masks;
+    P.seg_sweep = static_cast<long long *>(io.seg_sweep); P.image_base = io.image_base; P.image_offset = p.image_offset;
+    P.T = p.num_iou_thrs;
+    for (int i = 0; i < p.num_iou_thrs; ++i) P.thrs[i] = p.iou_thrs[i];
     if (p.proto_w % (P.proto_bf16 ? 8 : 4) != 0) return BT_ERR_UNSUPPORTED;   // 16-byte global strides for the tensor map
     P.NBY = mask_blocks(p.proto_h); P.NBX = mask_blocks(p.proto_w);
     P.ntx = (p.proto_w + TA_W - 1) / TA_W; P.nty = (p.proto_h + TA_H - 1) / TA_H;

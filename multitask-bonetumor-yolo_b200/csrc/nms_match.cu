@@ -68,14 +68,6 @@ constexpr int SORT_SMALL_MAX = 4096; // same for the 512-thread variant (8 per t
 constexpr int GM_THREADS = 256;      // match_kernel block
 constexpr int MAX_CELLS = 256;
 
-__device__ __forceinline__ uint32_t desc_key(float s) {
-    uint32_t u = __float_as_uint(s);
-    if (s != s) return 0u;                                   // NaN sorts first
-    if (u == 0x80000000u) u = 0u;                            // -0.0 == +0.0
-    uint32_t asc = (u & 0x80000000u) ? ~u : (u | 0x80000000u);
-    return ~asc;                                             // smaller key = higher score
-}
-
 // i = earlier (kept) box, j = later candidate; operand order of std::max/std::min as in
 // torchvision's nms_kernel_impl so NaN coordinates behave identically.
 //
@@ -959,8 +951,8 @@ __global__ void __launch_bounds__(GM_THREADS) match_kernel(const __grid_constant
         s_gl[tid] = P.gt_labels[(size_t)b * P.max_gt + tid];
     }
     __syncthreads();
-    const double area_lo[BT_NUM_AREA] = {0.0, 0.0, 32.0 * 32.0, 96.0 * 96.0};
-    const double area_hi[BT_NUM_AREA] = {1e10, 32.0 * 32.0, 96.0 * 96.0, 1e10};
+    const double area_lo[BT_NUM_AREA] = COCO_AREA_LO;
+    const double area_hi[BT_NUM_AREA] = COCO_AREA_HI;
     if (tid < BT_NUM_AREA) {
         unsigned m = 0;
         for (int g = 0; g < G; ++g) {
