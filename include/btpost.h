@@ -94,7 +94,8 @@ typedef struct BtParams {
                                  persistent kernels of the mask stage size their grids for a GPU of their own (4 / 8 CTAs per
                                  SM); >= 2: for a shared one (3 / 6: other batches' CTAs find room beside them, measured
                                  -1.5 % per pipelined step).  Results do not depend on it.                              */
-    int32_t reserved[2];
+    int32_t io_soft_dice;     /* 0: `io` points to a BtIO; 1: to a BtIOSoftDice (a BtIO followed by the soft-Dice outputs) */
+    int32_t reserved[1];
 } BtParams;
 
 /* Device buffers.  Inputs are read-only.  Any OUTPUT pointer may be NULL to skip that output
@@ -172,6 +173,21 @@ typedef struct BtIO {
                                    Header: N_RECORDS, N_IMAGES, NPIG[a][0] (|G| inside area range a); the FSUM slots stay
                                    unused.  btpost_sweep_accumulate with nc = 1, max_det_per_image = 1 gives the tables. */
 } BtIO;
+
+/* v3 soft Dice of the projector probabilities (SURVEY.md A.4, src/running_main_v3.py:466-474): a BtIO followed by three
+ * optional outputs.  Pass a pointer to it as the `io` of every entry point, with BtParams.io_soft_dice = 1; BtIO itself
+ * keeps its layout.  p = 1 / (1 + exp(-x)) of every upsampled projector logit x (the oracle's fma-only exp, IEEE
+ * division; p = 0 for x < -87), t = the GT mask.  Each p is rounded to 2^-40 fixed point, so the sums do not depend on
+ * the order of the atomics. */
+typedef struct BtIOSoftDice {
+    BtIO io;
+    int64_t *seg_soft2;         /* [B, 2] sum of p * t and sum of p over the S^2 pixels, units of 2^-40; zeroed per call by
+                                   the NMS stage (like seg_prob_sum)                                                    */
+    float *seg_soft_dice;       /* [B] 2 A / (P + G) in double rounded to fp32 (A, P from seg_soft2, G = |G|); NaN when
+                                   P + G == 0.  Needs seg_soft2                                                         */
+    int64_t *seg_soft_acc;      /* [2] ACCUMULATED like cm / seg_cnt4: sum over images of round(soft Dice * 2^40), and the
+                                   number of images with a defined soft Dice.  Needs seg_soft2                          */
+} BtIOSoftDice;
 
 /* Library / build identification. */
 BTPOST_API int btpost_version(void);

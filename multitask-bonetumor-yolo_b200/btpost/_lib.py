@@ -34,7 +34,7 @@ class BtParams(C.Structure):
         ("proj_bias", C.c_float), ("num_iou_thrs", C.c_int32),
         ("iou_thrs", C.c_double * BT_MAX_IOU_THRS),
         ("image_offset", C.c_int32), ("nms_threads", C.c_int32), ("proto_dtype", C.c_int32), ("head_dtype", C.c_int32),
-        ("drop_gt_no_cand", C.c_int32), ("in_flight", C.c_int32), ("reserved", C.c_int32 * 2),
+        ("drop_gt_no_cand", C.c_int32), ("in_flight", C.c_int32), ("io_soft_dice", C.c_int32), ("reserved", C.c_int32 * 1),
     ]
 
 
@@ -52,6 +52,14 @@ _IO_FIELDS = [
 
 class BtIO(C.Structure):
     _fields_ = [(n, C.c_void_p) for n in _IO_FIELDS]
+
+
+SOFT_DICE_FIELDS = ["seg_soft2", "seg_soft_dice", "seg_soft_acc"]
+
+
+class BtIOSoftDice(BtIO):
+    """A BtIO followed by the soft-Dice outputs (pass it with BtParams.io_soft_dice = 1)."""
+    _fields_ = [(n, C.c_void_p) for n in SOFT_DICE_FIELDS]
 
 
 _lib = None

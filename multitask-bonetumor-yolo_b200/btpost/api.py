@@ -22,7 +22,7 @@ from dataclasses import dataclass, field
 import torch
 
 from . import _lib
-from ._lib import BtIO, BtParams
+from ._lib import BtIO, BtIOSoftDice, BtParams
 
 # Module constants with the reference's names and defaults (running_main_v2.py:51-53); overridable.
 CONF_TH = 0.05
@@ -130,6 +130,7 @@ class PostConfig:
     with_inst_masks: str | None = None   # None, "bits" ([B,K,S,S/8] bit-packed) or "dense" (+ [B,K,S,S] bytes)
     with_coco: bool = True
     with_seg_map: bool = False           # v3 segmentation-mAP prep (score numerator per image)
+    with_soft_dice: bool = False         # v3 soft Dice on the projector probabilities: seg_soft2 / seg_soft_dice (+ seg_soft_acc)
     num_anchors: int | None = None
     nms_threads: int = 0                 # 0 = auto; 512 / 1024 force a variant of the NMS kernel
     in_flight: int = 0                   # batches kept in flight on the device (Pipeline sets its depth): grid sizes of the mask stage
@@ -168,6 +169,7 @@ class PostProcessor:
         p.proto_dtype = _lib.PROTO_BF16 if cfg.proto_bf16 else _lib.PROTO_F32
         p.head_dtype = _lib.HEAD_BF16 if cfg.head_bf16 else _lib.HEAD_F32
         p.drop_gt_no_cand = int(cfg.drop_gt_no_cand)
+        p.io_soft_dice = int(cfg.with_soft_dice)   # the outputs below then travel in a BtIOSoftDice
         for i, v in enumerate(cfg.iou_thrs):
             p.iou_thrs[i] = v
         self.params = p
@@ -195,8 +197,12 @@ class PostProcessor:
         }
         if sweep is not None and not shared_counters:
             shared_counters = sweep.counters()   # the accumulators live in the sweep header: one all-reduce merges everything
+        if cfg.with_soft_dice:
+            o["seg_soft2"] = z(B, 2, dtype=torch.int64)
+            o["seg_soft_dice"] = z(B, dtype=torch.float32)
+            o["seg_soft_acc"] = z(2, dtype=torch.int64)
         if shared_counters:   # Pipeline: every slot adds into the same accumulators (device atomics)
-            for k in ("cm", "seg_cnt4", "uni_cnt4"):
+            for k in ("cm", "seg_cnt4", "uni_cnt4") + (("seg_soft_acc",) if cfg.with_soft_dice else ()):
                 o[k] = shared_counters[k]
         if cfg.with_seg_mask:
             o["seg_mask"] = z(B, S, S, dtype=torch.uint8)
@@ -221,14 +227,18 @@ class PostProcessor:
         if sweep is not None and sweep.seg_ptr is not None and not cfg.with_seg_map:
             raise ValueError("a sweep with a segmentation-mAP ring (seg_map_capacity > 0) needs with_seg_map=True "
                              "(the records are scored with the mask kernel's seg_prob_sum)")
+        if sweep is not None and sweep.soft_dice and not cfg.with_soft_dice:
+            raise ValueError("a sweep with soft_dice=True needs with_soft_dice=True (the mask kernel adds the per-image "
+                             "soft Dice into the sweep's seg_soft_acc)")
         self._empty_gt = torch.zeros(1, 6, dtype=torch.float32, device=dev)
         self.image_base = torch.zeros(1, dtype=torch.int32, device=dev)   # global index of image 0, read by the kernels
 
     # -- metric state ---------------------------------------------------------------------------
     def reset_metrics(self):
-        """Zero the accumulated counters (confusion matrix, global pixel tp/fp/fn/tn)."""
-        for k in ("cm", "seg_cnt4", "uni_cnt4"):
-            self.out[k].zero_()
+        """Zero the accumulated counters (confusion matrix, global pixel tp/fp/fn/tn, soft-Dice sum and count)."""
+        for k in ("cm", "seg_cnt4", "uni_cnt4", "seg_soft_acc"):
+            if k in self.out:
+                self.out[k].zero_()
 
     def check_gt_overflow(self):
         """Raises when an image of the last batch had more GT rows than ``max_gt`` (the reference has no limit; the
@@ -246,7 +256,7 @@ class PostProcessor:
                              f"got {t.dtype} {tuple(t.shape)} on {t.device}")
 
     def _io(self, head, protos, det_boxes_gt, masks_gt, proj_weight, maps=None, coeffs=None):
-        io = BtIO()
+        io = BtIOSoftDice() if self.cfg.with_soft_dice else BtIO()
         cfg, B, S, N = self.cfg, self.B, self.S, self.N
         hdt = torch.bfloat16 if cfg.head_bf16 else torch.float32
         if cfg.layout == _lib.LAYOUT_L2:
@@ -361,7 +371,8 @@ class Pipeline:
     slot's input buffers on that slot's stream and replays its step; a producer can instead write straight into
     ``inputs[slot]`` and call ``replay(slot)`` (zero-copy).  ``wait(slot)`` blocks the host until the slot's step is
     done and returns its outputs, which stay valid until the slot is used again (``depth`` steps later).  The
-    accumulated counters (cm, seg_cnt4, uni_cnt4) are shared by all slots (device atomics): ``counters(key)``.
+    accumulated counters (cm, seg_cnt4, uni_cnt4, seg_soft_acc) are shared by all slots (device atomics):
+    ``counters(key)``.
 
     ``det_boxes_gt`` lives in a fixed ``[gt_rows_cap, 6]`` buffer per slot; unused rows carry batch index -1, which
     matches no image."""
@@ -384,7 +395,7 @@ class Pipeline:
         self.sweep = sweep
         self.shared = sweep.counters() if sweep is not None else {
             "cm": torch.zeros(nc, nc, dtype=torch.int64, device=dev), "seg_cnt4": torch.zeros(4, dtype=torch.int64, device=dev),
-            "uni_cnt4": torch.zeros(4, dtype=torch.int64, device=dev)}
+            "uni_cnt4": torch.zeros(4, dtype=torch.int64, device=dev), "seg_soft_acc": torch.zeros(2, dtype=torch.int64, device=dev)}
         self.procs = [PostProcessor(cfg, dev, shared_counters=self.shared, sweep=sweep) for _ in range(depth)]
         N = self.procs[0].N
         self.gt_rows_cap = gt_rows_cap if gt_rows_cap is not None else 4 * B

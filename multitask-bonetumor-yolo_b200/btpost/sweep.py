@@ -346,14 +346,17 @@ class DeviceSweep:
     `Pipeline(..., sweep=...)`).  `capacity` = records the ring can hold (one per kept detection of this rank's
     shard; 32 bytes each).  `seg_map_capacity` > 0 adds a second sweep state for the v3 segmentation mAP
     (`BtIO.seg_sweep`: one record per image, so the number of images of this rank's shard; needs
-    `PostConfig.with_seg_map`); `finish()` then also returns the `seg_`-prefixed mAP keys."""
+    `PostConfig.with_seg_map`); `finish()` then also returns the `seg_`-prefixed mAP keys.  `soft_dice=True` (needs
+    `PostConfig.with_soft_dice`): `finish()` also returns v3's soft Dice, `seg_soft_dice` (the mean over the images with
+    a defined value, NaN when there is none) and `n_soft_dice_images`, from the `seg_soft_acc` header slots."""
 
     def __init__(self, nc: int, iou_thrs, max_dets=(1, 10, 100), capacity: int = 1 << 20, max_det_per_image: int = 300,
-                 device="cuda:0", seg_map_capacity: int = 0):
+                 device="cuda:0", seg_map_capacity: int = 0, soft_dice: bool = False):
         self.lib = _lib.load()
         self.nc, self.iou_thrs, self.max_dets = nc, [float(t) for t in iou_thrs], tuple(int(m) for m in max_dets)
         self.T, self.capacity, self.K = len(self.iou_thrs), int(capacity), int(max_det_per_image)
         self.seg_map_capacity = int(seg_map_capacity)
+        self.soft_dice = bool(soft_dice)
         self.device = torch.device(device)
         if self.device.type != "cuda":
             raise RuntimeError("DeviceSweep lives on a CUDA device (the records are written by the CUDA library)")
@@ -371,6 +374,7 @@ class DeviceSweep:
         self.cm = self.hdr[u: u + nc * nc].view(nc, nc)
         self.seg_cnt4 = self.hdr[u + 256: u + 260]
         self.uni_cnt4 = self.hdr[u + 260: u + 264]
+        self.seg_soft_acc = self.hdr[u + 264: u + 266]   # sum of soft Dice (2^-40 units), images with a defined value
         self.rec_thrs = torch.from_numpy(np.linspace(0.0, 1.0, 101)).to(self.device)
         self._md = (C.c_int32 * len(self.max_dets))(*self.max_dets)
         self.reset()
@@ -404,9 +408,9 @@ class DeviceSweep:
         del keep   # back to the allocator's cache
 
     def counters(self):
-        """cm / seg_cnt4 / uni_cnt4 views INSIDE the header: hand them to PostProcessor / Pipeline as accumulators and
-        they are merged by the same all-reduce."""
-        return {"cm": self.cm, "seg_cnt4": self.seg_cnt4, "uni_cnt4": self.uni_cnt4}
+        """cm / seg_cnt4 / uni_cnt4 / seg_soft_acc views INSIDE the header: hand them to PostProcessor / Pipeline as
+        accumulators and they are merged by the same all-reduce."""
+        return {"cm": self.cm, "seg_cnt4": self.seg_cnt4, "uni_cnt4": self.uni_cnt4, "seg_soft_acc": self.seg_soft_acc}
 
     def reset(self, stream=None):
         st = stream if stream is not None else torch.cuda.current_stream(self.device)
@@ -495,4 +499,7 @@ class DeviceSweep:
             "seg_dice": float(fs[0]) / ni, "seg_iou": float(fs[1]) / ni, "uni_dice": float(fs[2]) / ni, "uni_iou": float(fs[3]) / ni,
             "npig": h[_lib.SWEEP_NPIG: _lib.SWEEP_NPIG + 64].reshape(4, 16)[:, :nc].copy(), "precision": pr, "recall": rcl,
         })
+        if self.soft_dice:
+            s, k = int(h[u + 264]), int(h[u + 265])
+            res.update(seg_soft_dice=s / FSUM_SCALE / k if k else float("nan"), n_soft_dice_images=k)
         return res

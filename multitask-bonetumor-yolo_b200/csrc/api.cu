@@ -24,6 +24,7 @@ int check_params(const BtParams *p, const BtIO *io) {
     if (!(p->iou_thres == p->iou_thres)) return BT_ERR_BAD_ARG;
     if (p->nms_threads != 0 && p->nms_threads != 256 && p->nms_threads != 512 && p->nms_threads != 1024) return BT_ERR_BAD_ARG;
     if (p->in_flight < 0) return BT_ERR_BAD_ARG;
+    if (p->io_soft_dice != 0 && p->io_soft_dice != 1) return BT_ERR_BAD_ARG;
     if (p->proto_dtype != BT_PROTO_F32 && p->proto_dtype != BT_PROTO_BF16) return BT_ERR_BAD_ARG;
     if (p->head_dtype != BT_HEAD_F32 && p->head_dtype != BT_HEAD_BF16) return BT_ERR_BAD_ARG;
     if (p->layout == BT_LAYOUT_L1) {
@@ -68,7 +69,6 @@ static int check_stage2(const BtParams *p, const BtIO *io) {
 }
 
 static int check_stage3(const BtParams *p, const BtIO *io) {
-    (void)p;
     if (!io->protos || !io->masks_gt || !io->proj_weight || !io->dets || !io->det_count || !io->det_coeff)
         return BT_ERR_BAD_ARG;
     if (!aligned16(io->protos) || !aligned16(io->masks_gt)) return BT_ERR_MISALIGNED;
@@ -77,6 +77,8 @@ static int check_stage3(const BtParams *p, const BtIO *io) {
     if ((io->inst_bits && !aligned16(io->inst_bits)) || (io->inst_masks && !aligned16(io->inst_masks))) return BT_ERR_MISALIGNED;
     if (io->seg_sweep && (!io->seg_img3 || !io->seg_prob_sum)) return BT_ERR_BAD_ARG;   // the record's IoU and score inputs
     if (io->seg_sweep && !aligned16(io->seg_sweep)) return BT_ERR_MISALIGNED;
+    if (const BtIOSoftDice *sd = soft_io(*p, *io))
+        if ((sd->seg_soft_dice || sd->seg_soft_acc) && !sd->seg_soft2) return BT_ERR_BAD_ARG;   // computed from its sums
     return BT_OK;
 }
 

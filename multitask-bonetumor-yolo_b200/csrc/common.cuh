@@ -33,6 +33,34 @@ namespace bt {
 // for x > 1.5 * 2^-24 (pinned against torch in tests/golden/make_golden.py).
 __device__ __forceinline__ bool sigmoid_gt_half(float x) { return x > 8.940696716308594e-08f; }
 
+// exp shared bit-for-bit with oracle/btpost_oracle.c::bto_expf (Cody-Waite + degree-6 polynomial,
+// fma/mul/add only).  No overflow guard: the exponent add wraps above x ~ 88.
+__device__ __forceinline__ float bt_expf(float x) {
+    if (x < -87.0f) return 0.0f;
+    float t = __fmul_rn(x, 1.4426950408889634f);
+    float n = rintf(t);
+    float r = __fmaf_rn(n, -0.693145751953125f, x);
+    r = __fmaf_rn(n, -1.428606765330187e-06f, r);
+    float p = 1.3888889225e-03f;
+    p = __fmaf_rn(p, r, 8.3333337680e-03f);
+    p = __fmaf_rn(p, r, 4.1666667908e-02f);
+    p = __fmaf_rn(p, r, 1.6666667163e-01f);
+    p = __fmaf_rn(p, r, 0.5f);
+    p = __fmaf_rn(p, r, 1.0f);
+    p = __fmaf_rn(p, r, 1.0f);
+    int e = (int)n;
+    return __int_as_float(__float_as_int(p) + (e << 23));
+}
+
+// sigmoid(x) in units of 2^-40, the term of the soft-Dice sums (BtIOSoftDice.seg_soft2): 1 / (1 + bt_expf(-x)) rounded once
+// per operation, then scaled (exactly) and rounded to the nearest integer.  x < -87 gives 0: bt_expf(-x) would
+// wrap there, and the true value is below 2^-125, which rounds to 0 in this fixed point anyway.
+__device__ __forceinline__ long long soft_prob_fx40(float x) {
+    if (x < -87.0f) return 0ll;
+    const float p = __fdiv_rn(1.0f, __fadd_rn(1.0f, bt_expf(-x)));
+    return __float2ll_rn(__fmul_rn(p, 1099511627776.0f));
+}
+
 // Order-preserving image of an fp32 score: ascending key = descending score (sort keys of the NMS, sweep records).
 __device__ __forceinline__ uint32_t desc_key(float s) {
     uint32_t u = __float_as_uint(s);
@@ -88,6 +116,12 @@ struct Workspace {
 };
 
 static inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
+
+// The soft-Dice outputs when the caller passed a BtIOSoftDice (BtParams.io_soft_dice), else null.  `io` is then its
+// first member, so the cast recovers the enclosing struct.
+static inline const BtIOSoftDice *soft_io(const BtParams &p, const BtIO &io) {
+    return p.io_soft_dice ? reinterpret_cast<const BtIOSoftDice *>(&io) : nullptr;
+}
 
 // The candidate list holds every anchor that passes the filter (anchor order); BtParams.max_cand (Ultralytics max_nms)
 // limits how many of them, best score first, enter the NMS sweep.

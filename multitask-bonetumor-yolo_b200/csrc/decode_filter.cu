@@ -149,25 +149,6 @@ struct L2Decoder {
     }
 };
 
-// exp shared bit-for-bit with oracle/btpost_oracle.c::bto_expf (Cody-Waite + degree-6 polynomial,
-// fma/mul/add only).
-__device__ __forceinline__ float bt_expf(float x) {
-    if (x < -87.0f) return 0.0f;
-    float t = __fmul_rn(x, 1.4426950408889634f);
-    float n = rintf(t);
-    float r = __fmaf_rn(n, -0.693145751953125f, x);
-    r = __fmaf_rn(n, -1.428606765330187e-06f, r);
-    float p = 1.3888889225e-03f;
-    p = __fmaf_rn(p, r, 8.3333337680e-03f);
-    p = __fmaf_rn(p, r, 4.1666667908e-02f);
-    p = __fmaf_rn(p, r, 1.6666667163e-01f);
-    p = __fmaf_rn(p, r, 0.5f);
-    p = __fmaf_rn(p, r, 1.0f);
-    p = __fmaf_rn(p, r, 1.0f);
-    int e = (int)n;
-    return __int_as_float(__float_as_int(p) + (e << 23));
-}
-
 // ---- L1 decoder: three raw maps [4*R+nc, H, W]; DFL softmax expectation, anchors (x+.5,y+.5),
 // stride = img/W, class score = sigmoid(logit)  (running_main_v2.py:743-775, dist2bbox :97-107).
 template <bool BF16>

@@ -28,8 +28,8 @@
 //                     an image's instance masks is a 64-bit atomic OR per block whose returned old word gives the
 //                     newly set bits (union counters without a pass over the union); the projector mask owns its
 //                     cells.  Instruction-issue bound.
-//   finalize_kernel   one warp per image: counters -> Dice / IoU / tp-fp-fn-tn, and the image's v3 segmentation-mAP
-//                     record when BtIO.seg_sweep is set.
+//   finalize_kernel   one warp per image: counters -> Dice / IoU / tp-fp-fn-tn, the image's v3 segmentation-mAP
+//                     record when BtIO.seg_sweep is set, and its v3 soft Dice when BtIOSoftDice.seg_soft2 is set.
 // tcgen05 is deliberately not used: K = 32 at <= 0.5 FLOP/B, and TF32/BF16 accumulation would break the bit
 // parity of the thresholded masks with the fp32 reference.
 #include <cuda.h>
@@ -79,6 +79,10 @@ struct K3Params {
     const int32_t *image_base;
     int image_offset, T;
     double thrs[BT_MAX_IOU_THRS];
+    // v3 soft Dice (BtIOSoftDice.seg_soft2 / seg_soft_dice / seg_soft_acc); appended last for the same reason
+    long long *seg_soft2;   // [B, 2] optional: sum of p * t and of p, 2^-40 fixed point (zeroed by the NMS kernel)
+    float *seg_soft_dice;
+    long long *seg_soft_acc;
 };
 
 __device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
@@ -633,6 +637,7 @@ __device__ __forceinline__ void m1_item(const K3Params &P, int b, int q, int lan
     const int PH = P.PH, PW = P.PW, S_h = P.S_h, S_w = P.S_w, NBX = P.NBX, NBY = P.NBY;
     int inter = 0, area = 0;
     double psum = 0.0;
+    long long spt = 0, sp = 0;   // soft Dice: sum of p * t and of p over the valid pixels, units of 2^-40
     if (q < NBY * NBX) {
         int by = __float2int_rz(((float)q + 0.5f) * P.inv_NBX), bx = q - by * NBX;   // q / NBX without the integer division
         if (bx < 0) { --by; bx += NBX; } else if (bx >= NBX) { ++by; bx -= NBX; }
@@ -645,11 +650,11 @@ __device__ __forceinline__ void m1_item(const K3Params &P, int b, int q, int lan
 #pragma unroll
             for (int j = 0; j < 3; ++j) v[i][j] = __ldg(lm + rr[i] + cc[j]);
         const u64 gtw = __ldg(P.gtc + ((size_t)b * NBY + by) * NBX + bx);
-        if (!(P.seg_logits || P.seg_mask || P.seg_prob_sum)) {
+        if (!(P.seg_logits || P.seg_mask || P.seg_prob_sum || P.seg_soft2)) {
             const u64 bits = block_bits(v, by == 0, bx == 0) & block_valid(P, by, bx);
             area = __popcll(bits); inter = __popcll(bits & gtw);
         } else {
-            // dense outputs / v3 score: scalar path that keeps the logits
+            // dense outputs / v3 score / soft Dice: scalar path that keeps the logits
 #pragma unroll
             for (int a = 0; a < 2; ++a)
 #pragma unroll
@@ -660,9 +665,20 @@ __device__ __forceinline__ void m1_item(const K3Params &P, int b, int q, int lan
                     const int jl = (c == 0 || bx == 0) ? 0 : 1, jr = (c == 0) ? 1 : 2;
                     float lg[16];
                     unsigned bits = cell_bits_log(v[it][jl], v[it][jr], v[ib][jl], v[ib][jr], ci < 0, cj < 0, lg);
-                    bits &= cell_valid(ci, cj, PH, PW, S_h, S_w);
+                    const unsigned valid = cell_valid(ci, cj, PH, PW, S_h, S_w);
+                    const unsigned gt = (unsigned)((gtw >> (16 * (2 * a + c))) & 0xffffull);
+                    bits &= valid;
                     area += __popc(bits);
-                    inter += __popc(bits & (unsigned)((gtw >> (16 * (2 * a + c))) & 0xffffull));
+                    inter += __popc(bits & gt);
+                    if (P.seg_soft2) {
+#pragma unroll
+                        for (int k = 0; k < 16; ++k)
+                            if ((valid >> k) & 1u) {
+                                const long long pf = soft_prob_fx40(lg[k]);
+                                sp += pf;
+                                if ((gt >> k) & 1u) spt += pf;
+                            }
+                    }
                     if (P.seg_prob_sum && bits) {
                         float ps = 0.0f;   // v3 seg-mAP score numerator: sigmoid over the foreground pixels of the cell
 #pragma unroll
@@ -698,6 +714,18 @@ __device__ __forceinline__ void m1_item(const K3Params &P, int b, int q, int lan
 #pragma unroll
         for (int d = 16; d > 0; d >>= 1) psum += __shfl_down_sync(0xffffffffu, psum, d);
         if (lane == 0 && psum != 0.0) atomicAdd(&P.seg_prob_sum[b], psum);
+    }
+    if (P.seg_soft2) {   // integer sums: exact, so the order of the lanes and of the items does not matter
+#pragma unroll
+        for (int d = 16; d > 0; d >>= 1) {
+            spt += __shfl_down_sync(0xffffffffu, spt, d);
+            sp += __shfl_down_sync(0xffffffffu, sp, d);
+        }
+        if (lane == 0) {
+            unsigned long long *s2 = reinterpret_cast<unsigned long long *>(P.seg_soft2 + 2 * b);
+            if (spt) atomicAdd(s2, (unsigned long long)spt);
+            if (sp) atomicAdd(s2 + 1, (unsigned long long)sp);
+        }
     }
 }
 
@@ -898,6 +926,22 @@ __device__ __forceinline__ void seg_map_record(const K3Params &P, int b, long lo
     dst[1] = src[1];
 }
 
+// v3 soft Dice of image b (SURVEY.md A.4; DiceScore on the projector probabilities, running_main_v3.py:466-474):
+// 2 A / (P + G) with A = sum p * t and P = sum p from m1_item's 2^-40 sums and G = |G|, in double, rounded to fp32;
+// NaN (and left out of the accumulator's count) when P + G == 0, as the reference's mean skips NaN.
+__device__ __forceinline__ void soft_dice_image(const K3Params &P, int b, long long gsum) {
+    const long long a = __ldcg(P.seg_soft2 + 2 * b), p = __ldcg(P.seg_soft2 + 2 * b + 1);
+    const bool defined = p != 0 || gsum != 0;
+    const float d = defined ? __double2float_rn(2.0 * (double)a / ((double)p + (double)gsum * 1099511627776.0))
+                            : __int_as_float(0x7fc00000);
+    if (P.seg_soft_dice) P.seg_soft_dice[b] = d;
+    if (P.seg_soft_acc && defined) {
+        unsigned long long *acc = reinterpret_cast<unsigned long long *>(P.seg_soft_acc);
+        atomicAdd(acc, (unsigned long long)__double2ll_rn((double)d * 1099511627776.0));
+        atomicAdd(acc + 1, 1ull);
+    }
+}
+
 // per-image epilogue: |G|, Dice / IoU (test_model.py:15-23)
 __device__ __forceinline__ void finalize_image(const K3Params &P, int b, int lane) {
     int gg = 0;
@@ -928,6 +972,7 @@ __device__ __forceinline__ void finalize_image(const K3Params &P, int b, int lan
             atomicAdd(fs + 1, (unsigned long long)__double2ll_rn((double)v_iou * 1099511627776.0));
         }
         if (lane == 0 && P.seg_sweep) seg_map_record(P, b, inter, pp, gsum);
+        if (lane == 0 && P.seg_soft2) soft_dice_image(P, b, gsum);
     }
 }
 
@@ -1102,6 +1147,10 @@ int launch_masks(const BtParams &p, const BtIO &io, const Workspace &w, cudaStre
     P.seg_sweep = static_cast<long long *>(io.seg_sweep); P.image_base = io.image_base; P.image_offset = p.image_offset;
     P.T = p.num_iou_thrs;
     for (int i = 0; i < p.num_iou_thrs; ++i) P.thrs[i] = p.iou_thrs[i];
+    if (const BtIOSoftDice *sd = soft_io(p, io)) {
+        P.seg_soft2 = reinterpret_cast<long long *>(sd->seg_soft2); P.seg_soft_dice = sd->seg_soft_dice;
+        P.seg_soft_acc = reinterpret_cast<long long *>(sd->seg_soft_acc);
+    }
     if (p.proto_w % (P.proto_bf16 ? 8 : 4) != 0) return BT_ERR_UNSUPPORTED;   // 16-byte global strides for the tensor map
     P.NBY = mask_blocks(p.proto_h); P.NBX = mask_blocks(p.proto_w);
     P.ntx = (p.proto_w + TA_W - 1) / TA_W; P.nty = (p.proto_h + TA_H - 1) / TA_H;

@@ -156,6 +156,7 @@ struct K2Params {
     long long *sweep;     // optional sweep state (header + record ring, include/btpost.h)
     int image_offset, drop_gt_no_cand;
     const int32_t *image_base;
+    long long *seg_soft2;   // soft-Dice sums of the mask kernel (optional), zeroed here; last: earlier offsets stay
 };
 
 // =================================================================================================
@@ -463,6 +464,7 @@ __global__ void __launch_bounds__(K2_THREADS, K2_THREADS == 512 ? NMS_MINB_512 :
     if (tid == 10 && b == 0) *P.pool_used = 0ull;
     if (tid == 11 && b == 0) { P.n_items[0] = 0; P.n_items[1] = 0; }
     if (tid == 9 && P.seg_prob_sum) P.seg_prob_sum[b] = 0.0;
+    if (tid == 12 && P.seg_soft2) { P.seg_soft2[2 * b] = 0; P.seg_soft2[2 * b + 1] = 0; }
     for (int i = tid; i < K; i += K2_THREADS) {
         if (P.inst_area) P.inst_area[(size_t)b * K + i] = 0;
         if (P.inst_inter) P.inst_inter[(size_t)b * K + i] = 0;
@@ -1123,7 +1125,7 @@ int launch_nms_match(const BtParams &p, const BtIO &io, const Workspace &w, cuda
     for (int i = 0; i < p.num_iou_thrs; ++i) P.thrs[i] = p.iou_thrs[i];
     P.dt_match = io.dt_match; P.dt_ignore = io.dt_ignore; P.gt_ignore = io.gt_ignore;
     P.acc = w.acc; P.inst_area = io.inst_area; P.inst_inter = io.inst_inter;
-    P.seg_prob_sum = io.seg_prob_sum;
+    P.seg_prob_sum = io.seg_prob_sum; if (const BtIOSoftDice *sd = soft_io(p, io)) P.seg_soft2 = reinterpret_cast<long long *>(sd->seg_soft2);
     P.sweep = static_cast<long long *>(io.sweep); P.image_offset = p.image_offset; P.drop_gt_no_cand = p.drop_gt_no_cand; P.image_base = io.image_base;
     P.centre_cull = (p.iou_thres >= 0.55) ? 1 : 0;
     P.crop = p.crop; P.PW = p.proto_w; P.PH = p.proto_h;

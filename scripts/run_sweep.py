@@ -10,7 +10,8 @@ COCOeval.accumulate as CUDA kernels (btpost.DeviceSweep.finish).
     python -m torch.distributed.run --nproc-per-node 8 --master-addr 127.0.0.1 scripts/run_sweep.py --images 16384
 Prints one JSON line with mAP / mAP50 / Dice / F1 and the device time of the sweep.  --seg-map adds the v3 segmentation
 mAP (one record per image, appended by the mask stage to a second sweep state; seg_map / seg_map_50 in the line); the
-default run leaves it out, so that its numbers stay comparable with earlier profiles."""
+default run leaves it out, so that its numbers stay comparable with earlier profiles.  --soft-dice adds v3's soft Dice
+on the projector probabilities (seg_soft_dice in the line; one exp and one division per output pixel in the mask stage)."""
 import argparse, json, os, sys, time
 from pathlib import Path
 ROOT = Path(__file__).resolve().parents[1]
@@ -27,6 +28,7 @@ ap.add_argument("--max-det", dest="max_det", type=int, default=100)
 ap.add_argument("--depth", type=int, default=4)
 ap.add_argument("--seed", type=int, default=20265)
 ap.add_argument("--seg-map", dest="seg_map", action="store_true", help="also the v3 segmentation mAP (seg_map, seg_map_50)")
+ap.add_argument("--soft-dice", dest="soft_dice", action="store_true", help="also v3's soft Dice on the projector probabilities")
 args = ap.parse_args()
 rank, world, lrank = (int(os.environ.get(k, d)) for k, d in (("RANK", 0), ("WORLD_SIZE", 1), ("LOCAL_RANK", 0)))
 torch.cuda.set_device(lrank)
@@ -41,9 +43,9 @@ if world > 1:
 B, K = args.batch, args.max_det
 nbatches = args.images // B
 mine = [i for i in range(nbatches) if i % world == rank]          # whole batches b = r (mod G)
-cfg = PostConfig(batch=B, img_size=args.img, gt_mode=1, max_det=K, with_seg_map=args.seg_map)
+cfg = PostConfig(batch=B, img_size=args.img, gt_mode=1, max_det=K, with_seg_map=args.seg_map, with_soft_dice=args.soft_dice)
 sweep = DeviceSweep(cfg.nc, map_iou_thresholds(), (1, 10, 100), capacity=max(len(mine), 1) * B * K, max_det_per_image=K, device=dev,
-                    seg_map_capacity=max(len(mine), 1) * B if args.seg_map else 0)
+                    seg_map_capacity=max(len(mine), 1) * B if args.seg_map else 0, soft_dice=args.soft_dice)
 probe = synth.make_batch_device(synth.SynthConfig(batch=B, img_size=args.img, seed=args.seed), dev)
 pipe = Pipeline(cfg, dev, depth=args.depth, proj_weight=probe["proj_weight"], proj_bias=probe["proj_bias"], sweep=sweep)
 del probe
@@ -83,6 +85,8 @@ if rank == 0:
     keys = ("n_images", "n_records", "map", "map_50", "map_75", "mar_100", "seg_f1", "seg_dice", "seg_iou", "uni_dice", "uni_iou")
     if args.seg_map:
         keys += ("seg_map", "seg_map_50")
+    if args.soft_dice:
+        keys += ("seg_soft_dice",)
     line = {k: res[k] for k in keys}
     line.update(world=world, images=nbatches * B, batches_in_flight=args.depth, device_ms_batches_incl_generation=tms[0],
                 device_ms_reduce_gather_accumulate=tms[1], device_ms_total=tms[2], host_s=time.perf_counter() - t_host)
