@@ -103,7 +103,8 @@ typedef struct BtParams {
  * A=BT_NUM_AREA, T=num_iou_thrs. */
 typedef struct BtIO {
     /* ---- inputs ---- */
-    const void *head;           /* L2: [B, 4+nc+nm, N] fp32 or bf16 (head_dtype) (segment_preds_cat, main_modelv2.py:367) */
+    const void *head;           /* L2: [B, 4+nc+nm, N] fp32 or bf16 (head_dtype) (segment_preds_cat, main_modelv2.py:367),
+                                   16-byte aligned; N <= 32768, or N <= 8192 when N % 4 != 0 (L1: N <= 32768)      */
     const void *maps[3];        /* L1: [B, 4*reg_max+nc, H_l, W_l], strides 8/16/32; fp32 or bf16 (head_dtype) */
     const void *coeffs;         /* L1: mask coefficients [B, nm, N] (Segment `mc`), same dtype as the maps   */
     const void *protos;         /* [B, nm, proto_h, proto_w] fp32 (or bf16: proto_dtype), 16-byte aligned */

@@ -10,6 +10,14 @@ namespace bt {
 
 static inline bool aligned16(const void *p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
 
+// Anchor limit of the decode/filter kernel: one cluster of 8 CTAs of at most 1024 threads covers an image in one pass.
+// The L2 decoder reads 4 anchors per thread when N % 4 == 0 (N <= 8 * 1024 * 4) and 1 otherwise (N <= 8 * 1024); the
+// L1 decoder always takes up to 4 anchors per thread, interleaved, whatever N % 4 is.
+static int check_anchor_limit(const BtParams *p) {
+    const int per_thread = (p->layout == BT_LAYOUT_L1 || p->num_anchors % 4 == 0) ? 4 : 1;
+    return p->num_anchors > 8 * 1024 * per_thread ? BT_ERR_UNSUPPORTED : BT_OK;
+}
+
 int check_params(const BtParams *p, const BtIO *io) {
     if (!p || !io) return BT_ERR_BAD_ARG;
     if (p->batch <= 0 || p->num_anchors <= 0 || p->nc <= 0 || p->max_det <= 0) return BT_ERR_BAD_ARG;
@@ -36,7 +44,7 @@ int check_params(const BtParams *p, const BtIO *io) {
     } else if (p->layout != BT_LAYOUT_L2) {
         return BT_ERR_BAD_ARG;
     }
-    return BT_OK;
+    return check_anchor_limit(p);
 }
 
 static int check_ws(const BtParams *p, void *ws, size_t ws_bytes) {
@@ -49,6 +57,7 @@ static int check_ws(const BtParams *p, void *ws, size_t ws_bytes) {
 static int check_stage1(const BtParams *p, const BtIO *io) {
     if (p->layout == BT_LAYOUT_L2) {
         if (!io->head) return BT_ERR_BAD_ARG;
+        if (!aligned16(io->head)) return BT_ERR_MISALIGNED;   // the decoder reads 4 anchors of a row with one vector load
     } else {
         if (!io->maps[0] || !io->maps[1] || !io->maps[2]) return BT_ERR_BAD_ARG;
     }
@@ -147,9 +156,10 @@ const char *btpost_error_string(int code) {
     switch (code) {
         case BT_OK: return "ok";
         case BT_ERR_BAD_ARG: return "bad argument (null pointer, non-positive size or inconsistent parameters)";
-        case BT_ERR_UNSUPPORTED: return "unsupported shape (need nm=32, proto=img/4, img_w%32==0, nc<=16, max_gt<=32)";
+        case BT_ERR_UNSUPPORTED: return "unsupported shape (need nm=32, proto=img/4, img_w%32==0, nc<=16, max_gt<=32, max_det<=4096, and at most 32768 "
+                                         "anchors; an L2 head with N % 4 != 0 at most 8192)";
         case BT_ERR_WORKSPACE: return "workspace too small (see btpost_workspace_bytes)";
-        case BT_ERR_MISALIGNED: return "misaligned pointer (workspace 256 B; protos/masks 16 B)";
+        case BT_ERR_MISALIGNED: return "misaligned pointer (workspace 256 B; head/protos/masks 16 B)";
         case BT_ERR_CUDA: return "CUDA launch failed";
         case BT_ERR_NCCL: return "NCCL call failed";
         default: return "unknown error";
@@ -159,6 +169,7 @@ const char *btpost_error_string(int code) {
 int btpost_workspace_bytes(const BtParams *p, size_t *bytes) {
     if (!p || !bytes) return BT_ERR_BAD_ARG;
     if (p->batch <= 0 || p->num_anchors <= 0) return BT_ERR_BAD_ARG;
+    if (int rc = check_anchor_limit(p)) return rc;   // a configuration btpost_run would reject fails here already
     *bytes = carve(p, nullptr).bytes;
     return BT_OK;
 }

@@ -491,8 +491,7 @@ int launch_decode_filter(const BtParams &p, const BtIO &io, const Workspace &w, 
     if (p.layout == BT_LAYOUT_L2) {
         P.head = io.head; P.C = 4 + p.nc + p.nm;
         const bool bf16 = p.head_dtype == BT_HEAD_BF16;
-        bool vec = (p.num_anchors % 4 == 0) && ((reinterpret_cast<uintptr_t>(io.head) & 15) == 0);
-        if (block_for(vec ? 4 : 1) > K1_MAX_THREADS) return BT_ERR_UNSUPPORTED;  // > 32768 (262144 vectorised) anchors
+        const bool vec = p.num_anchors % 4 == 0;   // the head is 16-byte aligned (check_stage1); anchor limits in check_params
         dim3 block(block_for(vec ? 4 : 1));
         const bool small = block.x <= 320;
         if (bf16) {
@@ -520,12 +519,10 @@ int launch_decode_filter(const BtParams &p, const BtIO &io, const Workspace &w, 
         const bool bf16 = p.head_dtype == BT_HEAD_BF16;   // raw maps of a bf16-mixed forward (running_main_v2.py:1324)
         if (bf16) {
             if (block_for(4) <= 320) decode_filter_l1_kernel<4, 320, true><<<grid, dim3(block_for(4)), 0, s>>>(P);
-            else if (block_for(1) <= K1_MAX_THREADS) decode_filter_l1_kernel<1, K1_MAX_THREADS, true><<<grid, dim3(block_for(1)), 0, s>>>(P);
             else if (block_for(2) <= K1_MAX_THREADS) decode_filter_l1_kernel<2, K1_MAX_THREADS, true><<<grid, dim3(block_for(2)), 0, s>>>(P);
             else if (block_for(4) <= K1_MAX_THREADS) decode_filter_l1_kernel<4, K1_MAX_THREADS, true><<<grid, dim3(block_for(4)), 0, s>>>(P);
             else return BT_ERR_UNSUPPORTED;
         } else if (block_for(4) <= 320) decode_filter_l1_kernel<4, 320><<<grid, dim3(block_for(4)), 0, s>>>(P);
-        else if (block_for(1) <= K1_MAX_THREADS) decode_filter_l1_kernel<1, K1_MAX_THREADS><<<grid, dim3(block_for(1)), 0, s>>>(P);
         else if (block_for(2) <= K1_MAX_THREADS) decode_filter_l1_kernel<2, K1_MAX_THREADS><<<grid, dim3(block_for(2)), 0, s>>>(P);
         else if (block_for(4) <= K1_MAX_THREADS) decode_filter_l1_kernel<4, K1_MAX_THREADS><<<grid, dim3(block_for(4)), 0, s>>>(P);
         else return BT_ERR_UNSUPPORTED;

@@ -27,7 +27,8 @@ def run_cuda(batch, dev="cuda:0", gt_f32=False, l1=False, **kw):
                      gt_mask_dtype=_lib.MASK_F32 if gt_f32 else _lib.MASK_U8, nms_threads=kw.get("nms_threads", 0),
                      proto_bf16=bool(kw.get("proto_bf16", False)), head_bf16=bool(kw.get("head_bf16", False)),
                      drop_gt_no_cand=bool(kw.get("drop_gt_no_cand", 0)), with_inst_masks=kw.get("with_inst_masks"),
-                     num_anchors=kw.get("num_anchors"), with_seg_mask=True, with_seg_logits=True, with_uni_mask=True, with_coco=True, with_seg_map=True)
+                     num_anchors=kw.get("num_anchors"), with_seg_mask=True, with_seg_logits=True, with_uni_mask=True, with_coco=True, with_seg_map=True,
+                     with_soft_dice=bool(kw.get("with_soft_dice", False)))
     pp = PostProcessor(cfg, dev)
     d = to_dev(batch, dev, gt_f32, bool(kw.get("proto_bf16", False)), bool(kw.get("head_bf16", False)))
     extra = {}
@@ -40,8 +41,8 @@ def run_cuda(batch, dev="cuda:0", gt_f32=False, l1=False, **kw):
     return {k: v.cpu().numpy() for k, v in out.items()}, pp
 
 
-def make(batch=2, img_size=640, seed=20261, l1=False, image_offset=0):
-    cfg = synth.SynthConfig(batch=batch, img_size=img_size, seed=seed, image_offset=image_offset)
+def make(batch=2, img_size=640, seed=20261, l1=False, image_offset=0, nc=3):
+    cfg = synth.SynthConfig(batch=batch, img_size=img_size, seed=seed, image_offset=image_offset, nc=nc)
     b = synth.make_batch(cfg, l1=l1)
     b["cfg"] = cfg
     return b
@@ -101,8 +102,11 @@ def oracle_parallel(batch, workers=None, chunk=1, **kw):
     def one(b0):
         b1 = min(B, b0 + chunk)
         sub = dict(batch)
-        for k in ("head", "protos", "masks_gt"):
-            sub[k] = batch[k][b0:b1]
+        for k in ("head", "protos", "masks_gt", "coeffs"):
+            if k in batch:
+                sub[k] = batch[k][b0:b1]
+        if "maps" in batch:                        # the raw-map (L1) layout: three per-level maps
+            sub["maps"] = [m[b0:b1] for m in batch["maps"]]
         rows = gt[(gt[:, 0] >= b0) & (gt[:, 0] < b1)].copy() if len(gt) else gt
         if len(rows):
             rows[:, 0] -= b0

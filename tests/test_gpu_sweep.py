@@ -33,10 +33,10 @@ def test_device_sweep_matches_cpu_sweep_of_oracle_outputs():
     np.testing.assert_allclose(a["precision"].cpu().numpy(), b["precision"].numpy(), rtol=1e-12)
 
 
-def _oracle_ap(outs, offsets, max_dets=(1, 10, 100), drop=False):
+def _oracle_ap(outs, offsets, max_dets=(1, 10, 100), drop=False, nc=3):
     """oracle.accumulate_ap over a list of oracle batch outputs (images in global order)."""
     thrs = oracle.iou_thresholds()
-    recs, npig = [], np.zeros((4, 3), np.int64)
+    recs, npig = [], np.zeros((4, nc), np.int64)
     order = np.argsort(offsets)
     for i in order:
         out = outs[i]
@@ -50,7 +50,7 @@ def _oracle_ap(outs, offsets, max_dets=(1, 10, 100), drop=False):
                 for gi in range(g):
                     if not out["gt_ignore"][b, a, gi]:
                         npig[a, out["gt_labels"][b, gi]] += 1
-    return oracle.accumulate_ap(recs, npig, thrs, max_dets, 3), npig
+    return oracle.accumulate_ap(recs, npig, thrs, max_dets, nc), npig
 
 
 @pytest.mark.parametrize("quantise", [False, True])
