@@ -95,7 +95,11 @@ typedef struct BtParams {
                                  SM); >= 2: for a shared one (3 / 6: other batches' CTAs find room beside them, measured
                                  -1.5 % per pipelined step).  Results do not depend on it.                              */
     int32_t io_soft_dice;     /* 0: `io` points to a BtIO; 1: to a BtIOSoftDice (a BtIO followed by the soft-Dice outputs) */
-    int32_t reserved[1];
+    union {                   /* io_micro took the former reserved word: the size and every offset are unchanged      */
+        int32_t io_micro;     /* 1: `io` points to a BtIOMicro (a BtIOSoftDice followed by micro_sweep); its soft-Dice pointers
+                                 are then read whatever io_soft_dice says (NULL skips them).  0: see io_soft_dice        */
+        int32_t reserved[1];
+    };
 } BtParams;
 
 /* Device buffers.  Inputs are read-only.  Any OUTPUT pointer may be NULL to skip that output
@@ -190,6 +194,27 @@ typedef struct BtIOSoftDice {
                                    number of images with a defined soft Dice.  Needs seg_soft2                          */
 } BtIOSoftDice;
 
+/* Class-agnostic box mAP (torchmetrics MeanAveragePrecision(average="micro"), which sets every prediction and target label
+ * to 0 before the COCO evaluation): a BtIOSoftDice followed by a third sweep state.  Pass a pointer to it as the `io` of
+ * every entry point, with BtParams.io_micro = 1; BtIO and BtIOSoftDice keep their layouts. */
+typedef struct BtIOMicro {
+    BtIOSoftDice sd;
+    void *micro_sweep;          /* optional sweep state (same format as BtIO.sweep, 16-byte aligned; needs dt_match): match_kernel
+                                   runs COCOeval.evaluateImg a second time per image with the labels ignored -- one category,
+                                   every kept detection in its descending-score order, every GT of the image, the same area
+                                   ranges, IoU thresholds and ignore rules -- on the IoUs of the class-aware pass, and appends
+                                   ONE record per kept detection.  The class-aware outputs do not depend on it.  Record fields:
+                                     matched / ignored  bit a * T + t, from the class-agnostic matching
+                                     score_key, image, rank   as in BtIO.sweep
+                                     class_rank = rank  (the maxDets cut is per image: greedy matching in score order means
+                                                        that the cut only drops records, so matching all K and cutting in
+                                                        the accumulate is exact)
+                                     label = 0
+                                   Header: N_RECORDS, N_IMAGES, NPIG[a][0] (non-ignored GTs of every class in area range a;
+                                   drop_gt_no_cand removes them as it does for BtIO.sweep); the FSUM slots stay unused.
+                                   btpost_sweep_accumulate with nc = 1, max_det_per_image = max_det gives the tables. */
+} BtIOMicro;
+
 /* Library / build identification. */
 BTPOST_API int btpost_version(void);
 BTPOST_API const char *btpost_error_string(int code);
@@ -238,7 +263,8 @@ BTPOST_API int btpost_run(const BtParams *p, const BtIO *io, void *ws, size_t ws
  * With BtIO.sweep set, btpost_run / btpost_nms_match / btpost_masks append to it on the device (no host work per
  * batch): match_kernel writes one record per kept detection and adds the batch's non-ignored GT counts and image
  * count, finalize_kernel adds the per-image Dice / IoU (2^-40 fixed point, so the sums do not depend on the order of
- * the atomics).  A second state at BtIO.seg_sweep collects the v3 segmentation mAP (one record per image, nc = 1).
+ * the atomics).  A second state at BtIO.seg_sweep collects the v3 segmentation mAP (one record per image, nc = 1), a third at
+ * BtIOMicro.micro_sweep the class-agnostic box mAP (one record per kept detection, nc = 1).
  * Every header slot is a plain sum, so shards are merged by ONE all-reduce(SUM) over the header (the
  * metric-counter all-reduce of the north star) plus one all-gather of the records (AP needs the global score order).
  * The caller may point BtIO.cm / seg_cnt4 / uni_cnt4 into the header's user slots so that they travel with it. */
@@ -282,6 +308,17 @@ BTPOST_API int btpost_sweep_accumulate(void *records, int64_t n_records, const i
                                        int32_t num_max_dets, int32_t max_det_per_image, int64_t num_images,
                                        double *precision, double *recall, void *scratch, size_t scratch_bytes,
                                        void *stream);
+/* btpost_sweep_accumulate plus COCOeval.accumulate's third table (NULL skips it): `scores` [T, num_rec, nc, BT_NUM_AREA,
+ * num_max_dets] (device, doubles, the layout of `precision`) = the fp32 score, widened, of the first record of the
+ * (class, area range, maxDet) sequence -- the class's records with class_rank < maxDet, ignored ones included, in sort
+ * order -- whose recall reaches recall threshold r (for r = 0: the sequence's first record, whatever its match / ignore
+ * state); 0 when no record reaches it (an empty sequence included); -1 where the class has no non-ignored GT.  This is
+ * the score at which pycocotools reaches each recall: how an operating point is chosen. */
+BTPOST_API int btpost_sweep_accumulate_ext(void *records, int64_t n_records, const int64_t *npig, const double *rec_thrs,
+                                           int32_t num_rec, int32_t nc, int32_t num_iou_thrs, const int32_t *max_dets,
+                                           int32_t num_max_dets, int32_t max_det_per_image, int64_t num_images,
+                                           double *precision, double *recall, double *scores, void *scratch,
+                                           size_t scratch_bytes, void *stream);
 
 #ifdef __cplusplus
 }

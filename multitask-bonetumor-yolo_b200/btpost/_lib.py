@@ -22,7 +22,12 @@ GT_LITERAL, GT_INTENDED = 0, 1
 MASK_U8, MASK_F32 = 0, 1
 
 
+class _IoMicro(C.Union):
+    _fields_ = [("io_micro", C.c_int32), ("reserved", C.c_int32 * 1)]
+
+
 class BtParams(C.Structure):
+    _anonymous_ = ("_io_micro",)
     _fields_ = [
         ("batch", C.c_int32), ("num_anchors", C.c_int32), ("nc", C.c_int32), ("nm", C.c_int32),
         ("reg_max", C.c_int32), ("img_h", C.c_int32), ("img_w", C.c_int32),
@@ -34,7 +39,7 @@ class BtParams(C.Structure):
         ("proj_bias", C.c_float), ("num_iou_thrs", C.c_int32),
         ("iou_thrs", C.c_double * BT_MAX_IOU_THRS),
         ("image_offset", C.c_int32), ("nms_threads", C.c_int32), ("proto_dtype", C.c_int32), ("head_dtype", C.c_int32),
-        ("drop_gt_no_cand", C.c_int32), ("in_flight", C.c_int32), ("io_soft_dice", C.c_int32), ("reserved", C.c_int32 * 1),
+        ("drop_gt_no_cand", C.c_int32), ("in_flight", C.c_int32), ("io_soft_dice", C.c_int32), ("_io_micro", _IoMicro),
     ]
 
 
@@ -60,6 +65,11 @@ SOFT_DICE_FIELDS = ["seg_soft2", "seg_soft_dice", "seg_soft_acc"]
 class BtIOSoftDice(BtIO):
     """A BtIO followed by the soft-Dice outputs (pass it with BtParams.io_soft_dice = 1)."""
     _fields_ = [(n, C.c_void_p) for n in SOFT_DICE_FIELDS]
+
+
+class BtIOMicro(BtIOSoftDice):
+    """A BtIOSoftDice followed by the class-agnostic sweep state (pass it with BtParams.io_micro = 1)."""
+    _fields_ = [("micro_sweep", C.c_void_p)]
 
 
 _lib = None
@@ -93,7 +103,10 @@ def load():
     L.btpost_sweep_accumulate.argtypes = [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32,
                                           C.POINTER(C.c_int32), C.c_int32, C.c_int32, C.c_int64, C.c_void_p, C.c_void_p,
                                           C.c_void_p, C.c_size_t, C.c_void_p]
-    for name in ("btpost_sweep_bytes", "btpost_sweep_reset", "btpost_sweep_accumulate_bytes", "btpost_sweep_accumulate"):
+    L.btpost_sweep_accumulate_ext.argtypes = (L.btpost_sweep_accumulate.argtypes[:13] + [C.c_void_p]
+                                              + L.btpost_sweep_accumulate.argtypes[13:])   # + scores after recall
+    for name in ("btpost_sweep_bytes", "btpost_sweep_reset", "btpost_sweep_accumulate_bytes", "btpost_sweep_accumulate",
+                 "btpost_sweep_accumulate_ext"):
         getattr(L, name).restype = C.c_int
     _lib = L
     return L

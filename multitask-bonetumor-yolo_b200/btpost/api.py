@@ -22,7 +22,7 @@ from dataclasses import dataclass, field
 import torch
 
 from . import _lib
-from ._lib import BtIO, BtIOSoftDice, BtParams
+from ._lib import BtIO, BtIOMicro, BtIOSoftDice, BtParams
 
 # Module constants with the reference's names and defaults (running_main_v2.py:51-53); overridable.
 CONF_TH = 0.05
@@ -170,6 +170,7 @@ class PostProcessor:
         p.head_dtype = _lib.HEAD_BF16 if cfg.head_bf16 else _lib.HEAD_F32
         p.drop_gt_no_cand = int(cfg.drop_gt_no_cand)
         p.io_soft_dice = int(cfg.with_soft_dice)   # the outputs below then travel in a BtIOSoftDice
+        p.io_micro = int(sweep is not None and sweep.micro_ptr is not None)   # ... or in a BtIOMicro with the micro state
         for i, v in enumerate(cfg.iou_thrs):
             p.iou_thrs[i] = v
         self.params = p
@@ -256,7 +257,7 @@ class PostProcessor:
                              f"got {t.dtype} {tuple(t.shape)} on {t.device}")
 
     def _io(self, head, protos, det_boxes_gt, masks_gt, proj_weight, maps=None, coeffs=None):
-        io = BtIOSoftDice() if self.cfg.with_soft_dice else BtIO()
+        io = BtIOMicro() if self.params.io_micro else BtIOSoftDice() if self.cfg.with_soft_dice else BtIO()
         cfg, B, S, N = self.cfg, self.B, self.S, self.N
         hdt = torch.bfloat16 if cfg.head_bf16 else torch.float32
         if cfg.layout == _lib.LAYOUT_L2:
@@ -292,6 +293,8 @@ class PostProcessor:
         if self.sweep is not None:
             io.sweep = self.sweep.ptr
             io.seg_sweep = self.sweep.seg_ptr
+            if self.params.io_micro:
+                io.micro_sweep = self.sweep.micro_ptr
             io.image_base = self.image_base.data_ptr()
         self._keepalive = (head, protos, det_boxes_gt, masks_gt, proj_weight, maps, coeffs)
         return io

@@ -22,7 +22,9 @@ per-detection records, GT counts, image count and Dice / IoU sums to a caller-ow
 batch (`BtIO.sweep`, zero host work per batch), shards are merged by ONE all-reduce of the 4 KB header and one
 `all_gather_into_tensor` of the records, and COCOeval.accumulate runs as CUDA kernels (`btpost_sweep_accumulate`:
 radix sort + scans + 101-point lookup).  With `seg_map_capacity` it also owns the v3 segmentation-mAP state, to which the
-mask stage appends one record per image (`BtIO.seg_sweep`); it rides in the same collectives (`merge_sweeps`).
+mask stage appends one record per image (`BtIO.seg_sweep`); with `micro=True` it owns the class-agnostic state
+(`BtIOMicro.micro_sweep`, torchmetrics `average="micro"`), to which the COCO matching appends one record per kept
+detection.  Every state rides in the same collectives (`merge_sweeps`).
 """
 from __future__ import annotations
 
@@ -348,10 +350,15 @@ class DeviceSweep:
     (`BtIO.seg_sweep`: one record per image, so the number of images of this rank's shard; needs
     `PostConfig.with_seg_map`); `finish()` then also returns the `seg_`-prefixed mAP keys.  `soft_dice=True` (needs
     `PostConfig.with_soft_dice`): `finish()` also returns v3's soft Dice, `seg_soft_dice` (the mean over the images with
-    a defined value, NaN when there is none) and `n_soft_dice_images`, from the `seg_soft_acc` header slots."""
+    a defined value, NaN when there is none) and `n_soft_dice_images`, from the `seg_soft_acc` header slots.
+    `micro=True` adds the class-agnostic state (`BtIOMicro.micro_sweep`, torchmetrics `MeanAveragePrecision(
+    average="micro")`: every label counts as one class, so a well-placed box with the wrong class is a hit): one record
+    per kept detection, so the same capacity as the detection ring; `finish()` then also returns the `micro_`-prefixed
+    mAP / mAR keys and the `micro_precision` / `micro_recall` tables (the per-class keys stay the class-aware ones, as in
+    torchmetrics)."""
 
     def __init__(self, nc: int, iou_thrs, max_dets=(1, 10, 100), capacity: int = 1 << 20, max_det_per_image: int = 300,
-                 device="cuda:0", seg_map_capacity: int = 0, soft_dice: bool = False):
+                 device="cuda:0", seg_map_capacity: int = 0, soft_dice: bool = False, micro: bool = False):
         self.lib = _lib.load()
         self.nc, self.iou_thrs, self.max_dets = nc, [float(t) for t in iou_thrs], tuple(int(m) for m in max_dets)
         self.T, self.capacity, self.K = len(self.iou_thrs), int(capacity), int(max_det_per_image)
@@ -370,6 +377,10 @@ class DeviceSweep:
         if self.seg_map_capacity:
             self.seg_buf, self.seg_hdr, self.seg_records = self._state(self.seg_map_capacity)
             self.seg_ptr = self.seg_buf.data_ptr()
+        self.micro_buf = self.micro_hdr = self.micro_records = self.micro_ptr = None
+        if micro:
+            self.micro_buf, self.micro_hdr, self.micro_records = self._state(self.capacity)
+            self.micro_ptr = self.micro_buf.data_ptr()
         u = _lib.SWEEP_USER
         self.cm = self.hdr[u: u + nc * nc].view(nc, nc)
         self.seg_cnt4 = self.hdr[u + 256: u + 260]
@@ -402,9 +413,12 @@ class DeviceSweep:
         world = max(world, 1)
         per, seg = -(-int(total_records) // world), self.seg_map_capacity
         rows = lambda n: torch.empty(max(n, 1), REC_BYTES, dtype=torch.uint8, device=self.device)
-        keep = [scratch(total_records), rows(world * (per + seg)), rows(int(total_records))] + tables(self.nc)
+        micro = per if self.micro_ptr is not None else 0
+        keep = [scratch(total_records), rows(world * (per + seg + micro)), rows(int(total_records))] + tables(self.nc)
         if seg:
             keep += [scratch(world * seg), rows(per + seg), rows(world * seg)] + tables(1)
+        if micro:
+            keep += [scratch(total_records), rows(int(total_records))] + tables(1)
         del keep   # back to the allocator's cache
 
     def counters(self):
@@ -415,16 +429,18 @@ class DeviceSweep:
     def reset(self, stream=None):
         st = stream if stream is not None else torch.cuda.current_stream(self.device)
         with torch.cuda.device(self.device):
-            for ptr, cap in ((self.ptr, self.capacity), (self.seg_ptr, self.seg_map_capacity)):
+            for ptr, cap in ((self.ptr, self.capacity), (self.seg_ptr, self.seg_map_capacity), (self.micro_ptr, self.capacity)):
                 if ptr is not None:
                     _lib.check(self.lib.btpost_sweep_reset(C.c_void_p(ptr), C.c_int64(cap), C.c_void_p(st.cuda_stream)),
                                "btpost_sweep_reset")
 
-    def _accumulate(self, rec, n, hdr, nc, max_det_per_image, num_images_bound):
-        """btpost_sweep_accumulate on `n` merged records (reordered in place) -> (precision, recall) numpy tables."""
+    def _accumulate(self, rec, n, hdr, nc, max_det_per_image, num_images_bound, scores=False):
+        """btpost_sweep_accumulate_ext on `n` merged records (reordered in place) -> (precision, recall) device tables, and
+        the score table when `scores`."""
         T, A, M = self.T, 4, len(self.max_dets)
         precision = torch.empty(T, 101, nc, A, M, dtype=torch.float64, device=self.device)
         recall = torch.empty(T, nc, A, M, dtype=torch.float64, device=self.device)
+        sc = torch.empty_like(precision) if scores else None
         sb = C.c_size_t()
         _lib.check(self.lib.btpost_sweep_accumulate_bytes(C.c_int64(n), C.byref(sb)), "btpost_sweep_accumulate_bytes")
         scratch = torch.empty(sb.value, dtype=torch.uint8, device=self.device)
@@ -432,19 +448,23 @@ class DeviceSweep:
         bound = num_images_bound if num_images_bound is not None else (int(rec[:, 20:24].contiguous().view(torch.int32).max()) + 1 if n else 1)
         st = torch.cuda.current_stream(self.device)
         with torch.cuda.device(self.device):
-            rc = self.lib.btpost_sweep_accumulate(
+            rc = self.lib.btpost_sweep_accumulate_ext(
                 C.c_void_p(rec.data_ptr() if n else 0), C.c_int64(n), C.c_void_p(npig.data_ptr()), C.c_void_p(self.rec_thrs.data_ptr()),
                 C.c_int32(101), C.c_int32(nc), C.c_int32(T), self._md, C.c_int32(M), C.c_int32(max_det_per_image), C.c_int64(bound),
-                C.c_void_p(precision.data_ptr()), C.c_void_p(recall.data_ptr()), C.c_void_p(scratch.data_ptr()), C.c_size_t(sb.value),
-                C.c_void_p(st.cuda_stream))
-        _lib.check(rc, "btpost_sweep_accumulate")
-        return precision, recall
+                C.c_void_p(precision.data_ptr()), C.c_void_p(recall.data_ptr()), C.c_void_p(sc.data_ptr() if scores else 0),
+                C.c_void_p(scratch.data_ptr()), C.c_size_t(sb.value), C.c_void_p(st.cuda_stream))
+        _lib.check(rc, "btpost_sweep_accumulate_ext")
+        return (precision, recall, sc) if scores else (precision, recall)
 
     @torch.no_grad()
-    def finish(self, group=None, num_images_bound: int | None = None, timings: dict | None = None) -> dict:
+    def finish(self, group=None, num_images_bound: int | None = None, timings: dict | None = None,
+               extended_summary: bool = False) -> dict:
         """End of the sweep: merge the shards (header all-reduce + record all-gather), run COCOeval.accumulate on the
-        device and summarize.  Every rank returns the same result.  `timings` (developer aid): filled with the host time
-        of each stage in ms, with a device synchronisation after each."""
+        device and summarize.  Every rank returns the same result.  `extended_summary=True` (torchmetrics'
+        flag of that name) also returns COCOeval.accumulate's score table: `scores` next to `precision` / `recall`, and
+        `seg_map_scores` / `micro_scores` for the other states (same layout as the precision tables: the confidence at
+        which each recall threshold is reached).  `timings` (developer aid): filled with the host time of each stage in
+        ms, with a device synchronisation after each."""
         import time as _time
         _t = [_time.perf_counter()]
 
@@ -459,6 +479,9 @@ class DeviceSweep:
         states = [("", self.hdr, self.records, self.capacity)]
         if seg:
             states.append(("segmentation ", self.seg_hdr, self.seg_records, self.seg_map_capacity))
+        micro = self.micro_ptr is not None
+        if micro:
+            states.append(("class-agnostic ", self.micro_hdr, self.micro_records, self.capacity))
         n_here = [int(h[_lib.SWEEP_N_RECORDS]) for _, h, _, _ in states]
         _mark("read_count")
         for (what, _, _, cap), n in zip(states, n_here):
@@ -474,18 +497,35 @@ class DeviceSweep:
         hdr, n = hdrs[0], int(sum(ns[0]))
         n_images = int(hdr[_lib.SWEEP_N_IMAGES])
         nc = self.nc
-        precision, recall = self._accumulate(recs[0], n, hdr, nc, self.K, num_images_bound)
+        ext = bool(extended_summary)
+        tables = self._accumulate(recs[0], n, hdr, nc, self.K, num_images_bound, ext)
         if seg:
-            seg_tables = self._accumulate(recs[1], int(sum(ns[1])), hdrs[1], 1, 1, num_images_bound)
+            seg_tables = self._accumulate(recs[1], int(sum(ns[1])), hdrs[1], 1, 1, num_images_bound, ext)
+        if micro:
+            mi = len(states) - 1
+            micro_tables = self._accumulate(recs[mi], int(sum(ns[mi])), hdrs[mi], 1, self.K, num_images_bound, ext)
         _mark("accumulate")
-        pr, rcl = precision.cpu().numpy(), recall.cpu().numpy()
+        tables = [t.cpu().numpy() for t in tables]
+        pr, rcl = tables[0], tables[1]
         h = hdr.cpu().numpy()
         res = summarize(pr, rcl, self.iou_thrs, self.max_dets)
+        if ext:
+            res["scores"] = tables[2]
         if seg:
-            spr, srcl = (t.cpu().numpy() for t in seg_tables)
-            res.update({f"seg_{k}": v for k, v in summarize(spr, srcl, self.iou_thrs, self.max_dets).items()})
+            st = [t.cpu().numpy() for t in seg_tables]
+            res.update({f"seg_{k}": v for k, v in summarize(st[0], st[1], self.iou_thrs, self.max_dets).items()})
             # seg_precision is the pixel precision of the projector mask: the seg-mAP tables carry the seg_map_ prefix
-            res.update(n_seg_records=int(sum(ns[1])), seg_map_precision=spr, seg_map_recall=srcl)
+            res.update(n_seg_records=int(sum(ns[1])), seg_map_precision=st[0], seg_map_recall=st[1])
+            if ext:
+                res["seg_map_scores"] = st[2]
+        if micro:
+            mt = [t.cpu().numpy() for t in micro_tables]
+            # the per-class keys stay the class-aware ones (torchmetrics recomputes them in macro mode under "micro")
+            res.update({f"micro_{k}": v for k, v in summarize(mt[0], mt[1], self.iou_thrs, self.max_dets).items()
+                        if not k.endswith("per_class")})
+            res.update(n_micro_records=int(sum(ns[mi])), micro_precision=mt[0], micro_recall=mt[1])
+            if ext:
+                res["micro_scores"] = mt[2]
         _mark("summarize")
         ni = max(n_images, 1)
         u = _lib.SWEEP_USER

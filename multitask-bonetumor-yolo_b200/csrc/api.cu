@@ -33,6 +33,7 @@ int check_params(const BtParams *p, const BtIO *io) {
     if (p->nms_threads != 0 && p->nms_threads != 256 && p->nms_threads != 512 && p->nms_threads != 1024) return BT_ERR_BAD_ARG;
     if (p->in_flight < 0) return BT_ERR_BAD_ARG;
     if (p->io_soft_dice != 0 && p->io_soft_dice != 1) return BT_ERR_BAD_ARG;
+    if (p->io_micro != 0 && p->io_micro != 1) return BT_ERR_BAD_ARG;
     if (p->proto_dtype != BT_PROTO_F32 && p->proto_dtype != BT_PROTO_BF16) return BT_ERR_BAD_ARG;
     if (p->head_dtype != BT_HEAD_F32 && p->head_dtype != BT_HEAD_BF16) return BT_ERR_BAD_ARG;
     if (p->layout == BT_LAYOUT_L1) {
@@ -74,6 +75,10 @@ static int check_stage2(const BtParams *p, const BtIO *io) {
     if (io->dt_match && (!io->gt_count || !io->gt_boxes || !io->gt_labels || p->num_iou_thrs <= 0)) return BT_ERR_BAD_ARG;
     if (io->sweep && !io->dt_match) return BT_ERR_BAD_ARG;   // the records are written by the COCO matching
     if (io->sweep && (reinterpret_cast<uintptr_t>(io->sweep) & 15)) return BT_ERR_MISALIGNED;
+    if (void *ms = micro_sweep_of(*p, *io)) {
+        if (!io->dt_match) return BT_ERR_BAD_ARG;   // the class-agnostic pass runs inside the COCO matching
+        if (!aligned16(ms)) return BT_ERR_MISALIGNED;
+    }
     return BT_OK;
 }
 

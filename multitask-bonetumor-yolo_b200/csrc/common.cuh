@@ -117,10 +117,14 @@ struct Workspace {
 
 static inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
-// The soft-Dice outputs when the caller passed a BtIOSoftDice (BtParams.io_soft_dice), else null.  `io` is then its
-// first member, so the cast recovers the enclosing struct.
+// The soft-Dice outputs when the caller passed a BtIOSoftDice (BtParams.io_soft_dice) or a BtIOMicro (io_micro), else
+// null.  `io` is then the first member of the enclosing struct, so the cast recovers it.
 static inline const BtIOSoftDice *soft_io(const BtParams &p, const BtIO &io) {
-    return p.io_soft_dice ? reinterpret_cast<const BtIOSoftDice *>(&io) : nullptr;
+    return (p.io_soft_dice || p.io_micro) ? reinterpret_cast<const BtIOSoftDice *>(&io) : nullptr;
+}
+// The class-agnostic sweep state of a BtIOMicro (BtParams.io_micro), else null.
+static inline void *micro_sweep_of(const BtParams &p, const BtIO &io) {
+    return p.io_micro ? reinterpret_cast<const BtIOMicro *>(&io)->micro_sweep : nullptr;
 }
 
 // The candidate list holds every anchor that passes the filter (anchor order); BtParams.max_cand (Ultralytics max_nms)

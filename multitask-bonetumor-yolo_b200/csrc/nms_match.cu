@@ -157,6 +157,7 @@ struct K2Params {
     int image_offset, drop_gt_no_cand;
     const int32_t *image_base;
     long long *seg_soft2;   // soft-Dice sums of the mask kernel (optional), zeroed here; last: earlier offsets stay
+    long long *micro_sweep; // optional class-agnostic sweep state (BtIOMicro)
 };
 
 // =================================================================================================
@@ -909,9 +910,132 @@ __global__ void __launch_bounds__(GM_THREADS) plan_kernel(const __grid_constant_
 // =================================================================================================
 // COCOeval.evaluateImg (one CTA per image)
 // =================================================================================================
+// Ordered compaction of the detections with s_can[k] != 0 into s_list (block-wide); every thread gets their number.
+__device__ __forceinline__ int compact_list(const int *s_can, int *s_list, int D, int *s_warpcnt) {
+    const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
+    int base = 0;
+    for (int k0 = 0; k0 < D; k0 += GM_THREADS) {
+        int k = k0 + tid;
+        bool f = (k < D) && s_can[k] != 0;
+        unsigned m = __ballot_sync(0xffffffffu, f);
+        if (lane == 0) s_warpcnt[wid] = __popc(m);
+        __syncthreads();
+        int off = base, tot = 0;
+        for (int w = 0; w < GM_THREADS / 32; ++w) { int v = s_warpcnt[w]; if (w < wid) off += v; tot += v; }
+        __syncthreads();
+        if (f) s_list[off + __popc(m & ((1u << lane) - 1u))] = k;
+        base += tot;
+    }
+    __syncthreads();
+    return base;
+}
+
+// COCOeval.evaluateImg's greedy matching for one (area range, IoU threshold) -- record bit `bit` = a * T + t -- over the
+// compacted list in score order.  `gign`: bit g = GT g is ignored in this area range.  AGN: labels play no part (the
+// class-agnostic state) and only the record bits are written; otherwise dt_match / dt_ignore too, and the record bits
+// when `bits`.
+template <bool AGN>
+__device__ __forceinline__ void greedy_match(const K2Params &P, int b, int bit, int G, unsigned gign, const int *s_list, int nl,
+                                             const int *s_dl, const int *s_gl, const double *s_db, const double *s_gb,
+                                             const double *s_iou, bool iou_in_smem, bool bits, unsigned long long *s_mbits,
+                                             unsigned long long *s_gibits) {
+    const int T = P.T, K = P.max_det, a = bit / T, t = bit - a * T;
+    unsigned gm = 0;
+    const double thr = fmin(P.thrs[t], 1 - 1e-10);
+    for (int li = 0; li < nl; ++li) {
+        const int d = s_list[li];
+        const int dl = s_dl[d];
+        double best = thr;
+        int m = -1;
+        for (int pass = 0; pass < 2; ++pass) {
+            if (pass == 1 && m >= 0) break;          // matched a regular GT: stop at the first ignored one
+            for (int g = 0; g < G; ++g) {
+                if ((((gign >> g) & 1u) != 0) != (pass == 1)) continue;
+                if ((gm >> g) & 1u) continue;
+                if (!AGN && s_gl[g] != dl) continue;
+                double v = iou_in_smem ? s_iou[d * G + g] : bb_iou(s_db + d * 4, s_gb + g * 4);
+                if (v < best) continue;
+                best = v;
+                m = g;
+            }
+        }
+        if (m >= 0) {
+            gm |= 1u << m;
+            if (!AGN) {
+                size_t o = (((size_t)b * BT_NUM_AREA + a) * T + t) * K + d;
+                P.dt_match[o] = m + 1;
+                if (P.dt_ignore) P.dt_ignore[o] = (gign >> m) & 1u;
+            }
+            if (bits) {
+                atomicOr(&s_mbits[d], 1ull << bit);
+                if ((gign >> m) & 1u) atomicOr(&s_gibits[d], 1ull << bit);
+            }
+        }
+    }
+}
+
+// One image's records and header sums in the sweep state `hdr` (include/btpost.h "Sweep state").  AGN: the
+// class-agnostic state -- label 0, class_rank = rank, NPIG[a][0] counts the GTs of every class.
+template <bool AGN>
+__device__ __forceinline__ void append_records(const K2Params &P, long long *hdr, int b, int D, int G, const unsigned *gign,
+                                               const int *s_dl, const int *s_gl, const double *s_db,
+                                               const unsigned long long *s_mbits, const unsigned long long *s_gibits) {
+    const int tid = threadIdx.x, T = P.T, K = P.max_det;
+    const double area_lo[BT_NUM_AREA] = COCO_AREA_LO;
+    const double area_hi[BT_NUM_AREA] = COCO_AREA_HI;
+    BtSweepRecord *ring = reinterpret_cast<BtSweepRecord *>(hdr + BT_SWEEP_HEADER_I64);
+    __shared__ long long s_rbase, s_rcap;
+    if (tid == 0) {
+        atomicAdd(reinterpret_cast<unsigned long long *>(hdr + BT_SWEEP_N_IMAGES), 1ull);
+        s_rbase = D ? (long long)atomicAdd(reinterpret_cast<unsigned long long *>(hdr + BT_SWEEP_N_RECORDS), (unsigned long long)D) : 0;
+        s_rcap = hdr[BT_SWEEP_CAPACITY];
+    }
+    // non-ignored GT per (area range, class); v2 drops the target of an image without candidates (running_main_v2.py:797-814)
+    if (!(P.drop_gt_no_cand && P.n_cand[b] == 0)) {
+        const int ncls = AGN ? 1 : P.nc;
+        for (int q = tid; q < BT_NUM_AREA * ncls; q += GM_THREADS) {
+            const int a = q / ncls, c = q - a * ncls;
+            int cnt = 0;
+            for (int g = 0; g < G; ++g) cnt += ((AGN || s_gl[g] == c) && !((gign[a] >> g) & 1u)) ? 1 : 0;
+            if (cnt) atomicAdd(reinterpret_cast<unsigned long long *>(hdr + BT_SWEEP_NPIG + a * BT_MAX_CLASSES + c), (unsigned long long)cnt);
+        }
+    }
+    __syncthreads();
+    const unsigned long long tmask = (T >= 16) ? 0xffffull : ((1ull << T) - 1ull);
+    for (int d = tid; d < D; d += GM_THREADS) {
+        const long long pos = s_rbase + d;
+        if (pos >= s_rcap) continue;   // ring full: reported through the header (N_RECORDS > CAPACITY)
+        const int lab = AGN ? 0 : s_dl[d];
+        int cr = d;
+        if (!AGN) {
+            cr = 0;
+            for (int j = 0; j < d; ++j) cr += (s_dl[j] == lab) ? 1 : 0;
+        }
+        const double ar = s_db[d * 4 + 2] * s_db[d * 4 + 3];
+        unsigned long long amask = 0ull;   // unmatched detections outside the area range are ignored
+#pragma unroll
+        for (int a = 0; a < BT_NUM_AREA; ++a)
+            if (ar < area_lo[a] || ar > area_hi[a]) amask |= tmask << (a * T);
+        const unsigned long long mb = s_mbits[d];
+        BtSweepRecord r;
+        r.matched = mb;
+        r.ignored = s_gibits[d] | (~mb & amask);
+        r.score_key = desc_key(P.dets[((size_t)b * K + d) * 6 + 4]);
+        r.image = (uint32_t)(P.image_offset + (P.image_base ? __ldg(P.image_base) : 0) + b);
+        r.rank = (uint16_t)d;
+        r.class_rank = (uint16_t)cr;
+        r.label = (uint8_t)lab;
+        r.pad[0] = r.pad[1] = r.pad[2] = 0;
+        uint4 *dst = reinterpret_cast<uint4 *>(ring + pos);
+        const uint4 *src = reinterpret_cast<const uint4 *>(&r);
+        dst[0] = src[0];
+        dst[1] = src[1];
+    }
+}
+
 __global__ void __launch_bounds__(GM_THREADS) match_kernel(const __grid_constant__ K2Params P) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
-    const int b = blockIdx.x, tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
+    const int b = blockIdx.x, tid = threadIdx.x;
     const int K = P.max_det;
     if (P.dt_match == nullptr) return;
     BT_PHASE_INIT();
@@ -933,7 +1057,6 @@ __global__ void __launch_bounds__(GM_THREADS) match_kernel(const __grid_constant
     __shared__ int s_gl[32];
     __shared__ unsigned s_gign[BT_NUM_AREA];
     __shared__ int s_warpcnt[GM_THREADS / 32];
-    __shared__ int s_nlist;
 
     for (int k = tid; k < D; k += GM_THREADS) {
         s_mbits[k] = 0ull; s_gibits[k] = 0ull;
@@ -996,109 +1119,48 @@ __global__ void __launch_bounds__(GM_THREADS) match_kernel(const __grid_constant
         }
     }
     __syncthreads();
-    // ordered compaction of the detections that can match at the loosest threshold
-    {
-        int base = 0;
-        for (int k0 = 0; k0 < D; k0 += GM_THREADS) {
-            int k = k0 + tid;
-            bool f = (k < D) && s_can[k] != 0;
-            unsigned m = __ballot_sync(0xffffffffu, f);
-            if (lane == 0) s_warpcnt[wid] = __popc(m);
-            __syncthreads();
-            int off = base, tot = 0;
-            for (int w = 0; w < GM_THREADS / 32; ++w) { int v = s_warpcnt[w]; if (w < wid) off += v; tot += v; }
-            __syncthreads();
-            if (f) s_list[off + __popc(m & ((1u << lane) - 1u))] = k;
-            base += tot;
-        }
-        if (tid == 0) s_nlist = base;
-        __syncthreads();
-    }
-    // greedy matching, one thread per (area range, threshold), over the compacted list only
-    if (tid < BT_NUM_AREA * T) {
-        const int a = tid / T, t = tid - a * T;
-        const unsigned gign = s_gign[a];
-        unsigned gm = 0;
-        const double thr = fmin(P.thrs[t], 1 - 1e-10);
-        const int nl = s_nlist;
-        for (int li = 0; li < nl; ++li) {
-            const int d = s_list[li];
-            const int dl = s_dl[d];
-            double best = thr;
-            int m = -1;
-            for (int pass = 0; pass < 2; ++pass) {
-                if (pass == 1 && m >= 0) break;          // matched a regular GT: stop at the first ignored one
-                for (int g = 0; g < G; ++g) {
-                    if ((((gign >> g) & 1u) != 0) != (pass == 1)) continue;
-                    if ((gm >> g) & 1u) continue;
-                    if (s_gl[g] != dl) continue;
-                    double v = iou_in_smem ? s_iou[d * G + g] : bb_iou(s_db + d * 4, s_gb + g * 4);
-                    if (v < best) continue;
-                    best = v;
-                    m = g;
-                }
-            }
-            if (m >= 0) {
-                gm |= 1u << m;
-                size_t o = (((size_t)b * BT_NUM_AREA + a) * T + t) * K + d;
-                P.dt_match[o] = m + 1;
-                if (P.dt_ignore) P.dt_ignore[o] = (gign >> m) & 1u;
-                if (P.sweep) {
-                    atomicOr(&s_mbits[d], 1ull << tid);
-                    if ((gign >> m) & 1u) atomicOr(&s_gibits[d], 1ull << tid);
-                }
-            }
-        }
-    }
+    // ordered compaction of the detections that can match at the loosest threshold, then greedy matching, one thread per
+    // (area range, threshold), over the compacted list only
+    const int nl = compact_list(s_can, s_list, D, s_warpcnt);
+    if (tid < BT_NUM_AREA * T)
+        greedy_match<false>(P, b, tid, G, s_gign[tid / T], s_list, nl, s_dl, s_gl, s_db, s_gb, s_iou, iou_in_smem,
+                            P.sweep != nullptr, s_mbits, s_gibits);
     BT_PHASE_MARK(1, 7);   // COCO matching
     // ---- sweep records (a9): what torchmetrics keeps per image for COCOeval.accumulate, appended on the device
     if (P.sweep) {
         __syncthreads();
-        long long *hdr = P.sweep;
-        BtSweepRecord *ring = reinterpret_cast<BtSweepRecord *>(hdr + BT_SWEEP_HEADER_I64);
-        __shared__ long long s_rbase, s_rcap;
-        if (tid == 0) {
-            atomicAdd(reinterpret_cast<unsigned long long *>(hdr + BT_SWEEP_N_IMAGES), 1ull);
-            s_rbase = D ? (long long)atomicAdd(reinterpret_cast<unsigned long long *>(hdr + BT_SWEEP_N_RECORDS), (unsigned long long)D) : 0;
-            s_rcap = hdr[BT_SWEEP_CAPACITY];
-        }
-        // non-ignored GT per (area range, class); v2 drops the target of an image without candidates (running_main_v2.py:797-814)
-        if (!(P.drop_gt_no_cand && P.n_cand[b] == 0)) {
-            for (int q = tid; q < BT_NUM_AREA * P.nc; q += GM_THREADS) {
-                const int a = q / P.nc, c = q - a * P.nc;
-                int cnt = 0;
-                for (int g = 0; g < G; ++g) cnt += (s_gl[g] == c && !((s_gign[a] >> g) & 1u)) ? 1 : 0;
-                if (cnt) atomicAdd(reinterpret_cast<unsigned long long *>(hdr + BT_SWEEP_NPIG + a * BT_MAX_CLASSES + c), (unsigned long long)cnt);
+        append_records<false>(P, P.sweep, b, D, G, s_gign, s_dl, s_gl, s_db, s_mbits, s_gibits);
+    }
+    // ---- class-agnostic state (BtIOMicro.micro_sweep): evaluateImg once more with every label set to 0 (torchmetrics
+    // average="micro"), on the IoUs of the pass above.  Only the class predicate differs; dt_match / dt_ignore /
+    // gt_ignore and the class-aware records are written before this and do not depend on it.
+    if (P.micro_sweep) {
+        __syncthreads();   // the pass above is done with s_can / s_list / the bit tables
+        __shared__ unsigned s_gign_agn[BT_NUM_AREA];
+        if (tid < BT_NUM_AREA) {
+            unsigned m = 0;
+            for (int g = 0; g < G; ++g) {
+                const double ar = s_gb[g * 4 + 2] * s_gb[g * 4 + 3];
+                if (ar < area_lo[tid] || ar > area_hi[tid]) m |= 1u << g;
             }
+            s_gign_agn[tid] = m;
+        }
+        for (int k = tid; k < D; k += GM_THREADS) {
+            s_mbits[k] = 0ull; s_gibits[k] = 0ull;
+            double best = -1.0;
+            for (int g = 0; g < G; ++g) {
+                const double v = iou_in_smem ? s_iou[k * G + g] : bb_iou(s_db + k * 4, s_gb + g * 4);
+                if (v > best) best = v;
+            }
+            s_can[k] = (best >= thr_min) ? 1 : 0;
         }
         __syncthreads();
-        const unsigned long long tmask = (T >= 16) ? 0xffffull : ((1ull << T) - 1ull);
-        for (int d = tid; d < D; d += GM_THREADS) {
-            const long long pos = s_rbase + d;
-            if (pos >= s_rcap) continue;   // ring full: reported through the header (N_RECORDS > CAPACITY)
-            const int lab = s_dl[d];
-            int cr = 0;
-            for (int j = 0; j < d; ++j) cr += (s_dl[j] == lab) ? 1 : 0;
-            const double ar = s_db[d * 4 + 2] * s_db[d * 4 + 3];
-            unsigned long long amask = 0ull;   // unmatched detections outside the area range are ignored
-#pragma unroll
-            for (int a = 0; a < BT_NUM_AREA; ++a)
-                if (ar < area_lo[a] || ar > area_hi[a]) amask |= tmask << (a * T);
-            const unsigned long long mb = s_mbits[d];
-            BtSweepRecord r;
-            r.matched = mb;
-            r.ignored = s_gibits[d] | (~mb & amask);
-            r.score_key = desc_key(P.dets[((size_t)b * K + d) * 6 + 4]);
-            r.image = (uint32_t)(P.image_offset + (P.image_base ? __ldg(P.image_base) : 0) + b);
-            r.rank = (uint16_t)d;
-            r.class_rank = (uint16_t)cr;
-            r.label = (uint8_t)lab;
-            r.pad[0] = r.pad[1] = r.pad[2] = 0;
-            uint4 *dst = reinterpret_cast<uint4 *>(ring + pos);
-            const uint4 *src = reinterpret_cast<const uint4 *>(&r);
-            dst[0] = src[0];
-            dst[1] = src[1];
-        }
+        const int nla = compact_list(s_can, s_list, D, s_warpcnt);
+        if (tid < BT_NUM_AREA * T)
+            greedy_match<true>(P, b, tid, G, s_gign_agn[tid / T], s_list, nla, s_dl, s_gl, s_db, s_gb, s_iou, iou_in_smem, true,
+                               s_mbits, s_gibits);
+        __syncthreads();
+        append_records<true>(P, P.micro_sweep, b, D, G, s_gign_agn, s_dl, s_gl, s_db, s_mbits, s_gibits);
     }
 }
 
@@ -1127,6 +1189,7 @@ int launch_nms_match(const BtParams &p, const BtIO &io, const Workspace &w, cuda
     P.acc = w.acc; P.inst_area = io.inst_area; P.inst_inter = io.inst_inter;
     P.seg_prob_sum = io.seg_prob_sum; if (const BtIOSoftDice *sd = soft_io(p, io)) P.seg_soft2 = reinterpret_cast<long long *>(sd->seg_soft2);
     P.sweep = static_cast<long long *>(io.sweep); P.image_offset = p.image_offset; P.drop_gt_no_cand = p.drop_gt_no_cand; P.image_base = io.image_base;
+    P.micro_sweep = static_cast<long long *>(micro_sweep_of(p, io));
     P.centre_cull = (p.iou_thres >= 0.55) ? 1 : 0;
     P.crop = p.crop; P.PW = p.proto_w; P.PH = p.proto_h;
     P.rx = (float)((double)p.proto_w / (double)p.img_w);

@@ -17,6 +17,8 @@
 //      beats the true positive before it, and the right-to-left running max of pycocotools is exactly that maximum),
 //      so every true positive does one atomic max into the bin of the LAST recall threshold it reaches and a suffix
 //      max over the 101 bins finishes the job.  Doubles throughout, same expressions as numpy.
+//   3. optional (btpost_sweep_accumulate_ext): pycocotools' `scores` table, written by the walk at the one position that
+//      first reaches each recall threshold.
 #include "common.cuh"
 
 namespace bt {
@@ -169,7 +171,15 @@ struct AccParams {
     uint2 *totals;                 // [nc][ncombo]
     u64 *table;                    // [nc][ncombo][R] bit patterns of non-negative doubles
     double *precision, *recall;
+    double *scores;                // optional [T][R][nc][A][M] (btpost_sweep_accumulate_ext)
+    u64 *first_inc;                // [nc][4] first record of each (class, maxDet) sequence (only with `scores`)
 };
+
+// fp32 score of a record (inverse of desc_key; -0.0 comes back as +0.0)
+__device__ __forceinline__ double key_score(unsigned key) {
+    const unsigned asc = ~key;
+    return (double)__uint_as_float((asc & 0x80000000u) ? (asc & 0x7fffffffu) : ~asc);
+}
 
 __global__ void class_bounds_kernel(const AccParams P) {
     const int c = threadIdx.x;
@@ -203,15 +213,23 @@ template <bool WALK>
 __global__ void __launch_bounds__(ACC_THREADS) acc_chunk_kernel(const AccParams P) {
     __shared__ u64 s_m[ACC_CHUNK], s_i[ACC_CHUNK];
     __shared__ unsigned short s_cr[ACC_CHUNK];
+    __shared__ unsigned s_sk[ACC_CHUNK];
     int c, cnt, first;
     long long r0;
     if (!chunk_of(P, blockIdx.x, c, r0, cnt, first)) return;
     for (int i = threadIdx.x; i < cnt; i += ACC_THREADS) {
         const BtSweepRecord &r = P.rec[r0 + i];
-        s_m[i] = r.matched; s_i[i] = r.ignored; s_cr[i] = r.class_rank;
+        s_m[i] = r.matched; s_i[i] = r.ignored; s_cr[i] = r.class_rank; s_sk[i] = r.score_key;
     }
     __syncthreads();
     const int A = BT_NUM_AREA;
+    // score table: where each (class, maxDet) sequence starts -- its first record may be ignored at every (area,
+    // threshold), so the tp / fp prefixes cannot tell the walk whether a chunk holds it
+    if (!WALK && P.scores && threadIdx.x < P.M) {
+        const int md = P.max_dets[threadIdx.x];
+        for (int i = 0; i < cnt; ++i)
+            if (s_cr[i] < md) { atomicMin(P.first_inc + c * 4 + threadIdx.x, (u64)(r0 + i)); break; }
+    }
     for (int combo = threadIdx.x; combo < P.ncombo; combo += ACC_THREADS) {
         const int m = combo / (A * P.T), bit = combo - m * A * P.T, a = bit / P.T;
         const int md = P.max_dets[m];
@@ -234,12 +252,36 @@ __global__ void __launch_bounds__(ACC_THREADS) acc_chunk_kernel(const AccParams 
             u64 *tab = P.table + ((size_t)c * P.ncombo + combo) * P.R;
             int bin = -1, cur_bin = -1;
             double cur_max = 0.0;
+            // score table: recall threshold r is first reached at the sequence's first record (r with rec_thrs[r] <= 0)
+            // or at a true positive, and exactly one position reaches it first, so plain stores suffice.  sbin = last
+            // threshold reached before the current position.
+            double *sc = nullptr;
+            size_t sc_stride = 0;
+            u64 seq0 = ~0ull;
+            int sbin = -1;
+            if (P.scores) {
+                const int t = bit - a * P.T;
+                sc = P.scores + (((size_t)t * P.R * P.nc + c) * A + a) * P.M + m;
+                sc_stride = (size_t)P.nc * A * P.M;
+                seq0 = P.first_inc[c * 4 + m];
+                if ((u64)r0 > seq0) {
+                    const double rc0 = (double)tp / npd;
+                    while (sbin + 1 < P.R && P.rec_thrs[sbin + 1] <= rc0) ++sbin;
+                }
+            }
+            auto settle = [&](int i, double rc) {
+                while (sbin + 1 < P.R && P.rec_thrs[sbin + 1] <= rc) sc[(size_t)(++sbin) * sc_stride] = key_score(s_sk[i]);
+            };
             for (int i = 0; i < cnt; ++i) {
                 const unsigned ok = (s_cr[i] < md) & (unsigned)(~(s_i[i] >> bit) & 1ull);
-                if (!ok) continue;
-                if (!((s_m[i] >> bit) & 1ull)) { ++fp; continue; }
+                if (!ok || !((s_m[i] >> bit) & 1ull)) {
+                    fp += ok;
+                    if (sc && (u64)(r0 + i) == seq0) settle(i, (double)tp / npd);
+                    continue;
+                }
                 ++tp;
                 const double rc = (double)tp / npd;
+                if (sc) settle(i, rc);
                 while (bin + 1 < P.R && P.rec_thrs[bin + 1] <= rc) ++bin;   // last recall threshold this position reaches
                 if (bin < 0) continue;
                 const double pr = (double)tp / ((double)(fp + tp) + eps);
@@ -277,6 +319,11 @@ __global__ void __launch_bounds__(32) acc_scan_kernel(const AccParams P) {
         cfp += __shfl_sync(0xffffffffu, ifp, 31);
     }
     if (lane == 0) P.totals[(size_t)c * P.ncombo + combo] = make_uint2(ctp, cfp);
+    if (P.scores) {   // the walk overwrites the thresholds that some record reaches
+        const int A = BT_NUM_AREA, m = combo / (A * P.T), bit = combo - m * A * P.T, a = bit / P.T, t = bit - a * P.T;
+        const double v = P.npig[a * BT_MAX_CLASSES + c] == 0 ? -1.0 : 0.0;
+        for (int r = lane; r < P.R; r += 32) P.scores[((((size_t)t * P.R + r) * P.nc + c) * A + a) * P.M + m] = v;
+    }
 }
 
 __global__ void __launch_bounds__(ACC_THREADS) acc_final_kernel(const AccParams P) {
@@ -307,6 +354,7 @@ struct AccScratch {
     long long *cls_start;
     uint2 *sums, *totals;
     u64 *table;
+    u64 *first_inc;       // [BT_MAX_CLASSES][4]
     size_t bytes;
 };
 static AccScratch acc_carve(long long n, void *base) {
@@ -327,6 +375,7 @@ static AccScratch acc_carve(long long n, void *base) {
     s.sums = reinterpret_cast<uint2 *>(take((size_t)chunks * ACC_MAX_COMBOS * sizeof(uint2)));
     s.totals = reinterpret_cast<uint2 *>(take((size_t)BT_MAX_CLASSES * ACC_MAX_COMBOS * sizeof(uint2)));
     s.table = reinterpret_cast<u64 *>(take((size_t)BT_MAX_CLASSES * ACC_MAX_COMBOS * ACC_MAX_REC * sizeof(u64)));
+    s.first_inc = reinterpret_cast<u64 *>(take((size_t)BT_MAX_CLASSES * 4 * sizeof(u64)));
     s.bytes = off;
     return s;
 }
@@ -361,6 +410,14 @@ int btpost_sweep_accumulate(void *records, int64_t n_records, const int64_t *npi
                             int32_t nc, int32_t num_iou_thrs, const int32_t *max_dets, int32_t num_max_dets,
                             int32_t max_det_per_image, int64_t num_images, double *precision, double *recall, void *scratch,
                             size_t scratch_bytes, void *stream) {
+    return btpost_sweep_accumulate_ext(records, n_records, npig, rec_thrs, num_rec, nc, num_iou_thrs, max_dets, num_max_dets,
+                                       max_det_per_image, num_images, precision, recall, nullptr, scratch, scratch_bytes, stream);
+}
+
+int btpost_sweep_accumulate_ext(void *records, int64_t n_records, const int64_t *npig, const double *rec_thrs, int32_t num_rec,
+                                int32_t nc, int32_t num_iou_thrs, const int32_t *max_dets, int32_t num_max_dets,
+                                int32_t max_det_per_image, int64_t num_images, double *precision, double *recall,
+                                double *scores, void *scratch, size_t scratch_bytes, void *stream) {
     if (!npig || !rec_thrs || !max_dets || !precision || !recall || !scratch || n_records < 0 || (n_records > 0 && !records))
         return BT_ERR_BAD_ARG;
     if (nc <= 0 || nc > BT_MAX_CLASSES || num_iou_thrs <= 0 || num_iou_thrs > BT_MAX_IOU_THRS || num_max_dets <= 0 ||
@@ -402,7 +459,9 @@ int btpost_sweep_accumulate(void *records, int64_t n_records, const int64_t *npi
     P.rec_thrs = rec_thrs; P.npig = reinterpret_cast<const long long *>(npig);
     P.cls_start = sc.cls_start; P.sums = sc.sums; P.totals = sc.totals; P.table = sc.table;
     P.precision = precision; P.recall = recall;
+    P.scores = scores; P.first_inc = sc.first_inc;
     if (cudaMemsetAsync(sc.table, 0, (size_t)nc * P.ncombo * num_rec * sizeof(u64), s) != cudaSuccess) return BT_ERR_CUDA;
+    if (scores && cudaMemsetAsync(sc.first_inc, 0xff, (size_t)BT_MAX_CLASSES * 4 * sizeof(u64), s) != cudaSuccess) return BT_ERR_CUDA;
     class_bounds_kernel<<<1, 32, 0, s>>>(P);
     const int chunks = (int)((n + ACC_CHUNK - 1) / ACC_CHUNK) + nc;
     acc_chunk_kernel<false><<<chunks, ACC_THREADS, 0, s>>>(P);
