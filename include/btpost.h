@@ -320,6 +320,28 @@ BTPOST_API int btpost_sweep_accumulate_ext(void *records, int64_t n_records, con
                                            double *precision, double *recall, double *scores, void *scratch,
                                            size_t scratch_bytes, void *stream);
 
+/* ------------------------------------------------------------------------------------------------------------------
+ * Surface distances of a predicted mask against the GT mask: Hausdorff distance, HD95 and ASSD per image, in pixels of
+ * the network input (MONAI's compute_hausdorff_distance / compute_average_surface_distance with symmetric ASSD, made
+ * exact; DESIGN.md §4).  P = pred != 0, G = gt != 0; edge(M) = M AND NOT erode(M) with the 4-neighbour cross and
+ * background outside the image; d = Euclidean distance from each edge pixel of one mask to the nearest edge pixel of the
+ * other, computed exactly (integer squared distances, sqrt in double).
+ *   hd   = the largest d of both directions
+ *   hd95 = max over the two directions of torch.quantile(d.double(), 0.95) (linear interpolation)
+ *   assd = mean of the d of both directions together
+ * Each is rounded once to fp32.  An image whose P or G is empty gets NaN in all three and is not counted in `acc`.
+ * A pure function of the masks: the same bytes whatever else is in the batch.
+ *
+ * `pred` [B, S, S] bytes (PostProcessor's seg_mask), `gt` [B, 1, S, S] u8 or f32 (gt_mask_dtype), both 16-byte aligned;
+ * S % 32 == 0 and S <= 1280.  Outputs hd, hd95, assd [B] (device).  `acc` [4] (device, may be NULL) is ACCUMULATED:
+ * sum of round(hd * 2^32), of round(hd95 * 2^32), of round(assd * 2^32) (the fp32 values, widened) over the images with
+ * defined values, and their count; integer sums, so the words do not depend on the order of the images.  `scratch` from
+ * btpost_surface_bytes (256-byte aligned; 8 * B * S^2 bytes plus 64 * B rounded up to 256).  Arguments are checked before any CUDA call. */
+BTPOST_API int btpost_surface_bytes(int32_t batch, int32_t img, size_t *bytes);
+BTPOST_API int btpost_surface_distance(int32_t batch, int32_t img, const uint8_t *pred, const void *gt, int32_t gt_mask_dtype,
+                                       float *hd, float *hd95, float *assd, int64_t *acc, void *scratch, size_t scratch_bytes,
+                                       void *stream);
+
 #ifdef __cplusplus
 }
 #endif

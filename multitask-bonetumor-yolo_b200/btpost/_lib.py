@@ -105,8 +105,11 @@ def load():
                                           C.c_void_p, C.c_size_t, C.c_void_p]
     L.btpost_sweep_accumulate_ext.argtypes = (L.btpost_sweep_accumulate.argtypes[:13] + [C.c_void_p]
                                               + L.btpost_sweep_accumulate.argtypes[13:])   # + scores after recall
+    L.btpost_surface_bytes.argtypes = [C.c_int32, C.c_int32, C.POINTER(C.c_size_t)]
+    L.btpost_surface_distance.argtypes = [C.c_int32, C.c_int32] + [C.c_void_p] * 2 + [C.c_int32] + [C.c_void_p] * 5 + [C.c_size_t,
+                                                                                                                      C.c_void_p]
     for name in ("btpost_sweep_bytes", "btpost_sweep_reset", "btpost_sweep_accumulate_bytes", "btpost_sweep_accumulate",
-                 "btpost_sweep_accumulate_ext"):
+                 "btpost_sweep_accumulate_ext", "btpost_surface_bytes", "btpost_surface_distance"):
         getattr(L, name).restype = C.c_int
     _lib = L
     return L

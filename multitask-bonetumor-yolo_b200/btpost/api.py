@@ -131,6 +131,8 @@ class PostConfig:
     with_coco: bool = True
     with_seg_map: bool = False           # v3 segmentation-mAP prep (score numerator per image)
     with_soft_dice: bool = False         # v3 soft Dice on the projector probabilities: seg_soft2 / seg_soft_dice (+ seg_soft_acc)
+    with_surface_dist: bool = False      # Hausdorff distance, HD95 and ASSD of the projector mask against the GT mask, per image:
+                                         # seg_hd / seg_hd95 / seg_assd (+ seg_surf_acc); implies the seg_mask output
     num_anchors: int | None = None
     nms_threads: int = 0                 # 0 = auto; 512 / 1024 force a variant of the NMS kernel
     in_flight: int = 0                   # batches kept in flight on the device (Pipeline sets its depth): grid sizes of the mask stage
@@ -202,10 +204,15 @@ class PostProcessor:
             o["seg_soft2"] = z(B, 2, dtype=torch.int64)
             o["seg_soft_dice"] = z(B, dtype=torch.float32)
             o["seg_soft_acc"] = z(2, dtype=torch.int64)
+        if cfg.with_surface_dist:
+            for k in ("seg_hd", "seg_hd95", "seg_assd"):
+                o[k] = z(B, dtype=torch.float32)
+            o["seg_surf_acc"] = z(4, dtype=torch.int64)
         if shared_counters:   # Pipeline: every slot adds into the same accumulators (device atomics)
-            for k in ("cm", "seg_cnt4", "uni_cnt4") + (("seg_soft_acc",) if cfg.with_soft_dice else ()):
+            for k in (("cm", "seg_cnt4", "uni_cnt4") + (("seg_soft_acc",) if cfg.with_soft_dice else ())
+                      + (("seg_surf_acc",) if cfg.with_surface_dist else ())):
                 o[k] = shared_counters[k]
-        if cfg.with_seg_mask:
+        if cfg.with_seg_mask or cfg.with_surface_dist:   # the surface distances are computed from the projector mask bytes
             o["seg_mask"] = z(B, S, S, dtype=torch.uint8)
         if cfg.with_seg_logits:
             o["seg_logits"] = z(B, S, S, dtype=torch.float32)
@@ -222,6 +229,11 @@ class PostProcessor:
         if cfg.with_seg_map:
             o["seg_prob_sum"] = z(B, dtype=torch.float64)
         self.out = o
+        self._surf_scratch = None
+        if cfg.with_surface_dist:
+            nb = C.c_size_t()
+            _lib.check(self.lib.btpost_surface_bytes(B, S, C.byref(nb)), "btpost_surface_bytes")
+            self._surf_scratch = torch.empty(nb.value, dtype=torch.uint8, device=dev)   # torch allocations are 512-byte aligned
         self.sweep = sweep                # a btpost.sweep.DeviceSweep: records are appended by the library itself
         if sweep is not None and not cfg.with_coco:
             raise ValueError("a sweep needs with_coco=True (the records are written by the COCO matching)")
@@ -231,13 +243,17 @@ class PostProcessor:
         if sweep is not None and sweep.soft_dice and not cfg.with_soft_dice:
             raise ValueError("a sweep with soft_dice=True needs with_soft_dice=True (the mask kernel adds the per-image "
                              "soft Dice into the sweep's seg_soft_acc)")
+        if sweep is not None and sweep.surface and not cfg.with_surface_dist:
+            raise ValueError("a sweep with surface=True needs with_surface_dist=True (the surface-distance kernel adds the "
+                             "per-image HD / HD95 / ASSD into the sweep's seg_surf_acc)")
         self._empty_gt = torch.zeros(1, 6, dtype=torch.float32, device=dev)
         self.image_base = torch.zeros(1, dtype=torch.int32, device=dev)   # global index of image 0, read by the kernels
 
     # -- metric state ---------------------------------------------------------------------------
     def reset_metrics(self):
-        """Zero the accumulated counters (confusion matrix, global pixel tp/fp/fn/tn, soft-Dice sum and count)."""
-        for k in ("cm", "seg_cnt4", "uni_cnt4", "seg_soft_acc"):
+        """Zero the accumulated counters (confusion matrix, global pixel tp/fp/fn/tn, soft-Dice and surface-distance sums
+        and counts)."""
+        for k in ("cm", "seg_cnt4", "uni_cnt4", "seg_soft_acc", "seg_surf_acc"):
             if k in self.out:
                 self.out[k].zero_()
 
@@ -302,7 +318,9 @@ class PostProcessor:
     def run(self, head, protos, det_boxes_gt, masks_gt, proj_weight, proj_bias=0.0, *, maps=None, coeffs=None,
             stage="run", stream=None, image_offset=0):
         """Enqueue the hot path for one batch on the current (or given) CUDA stream; returns the
-        dict of output tensors (device, padded to ``max_det`` / ``max_gt``; see include/btpost.h)."""
+        dict of output tensors (device, padded to ``max_det`` / ``max_gt``; see include/btpost.h).  With
+        ``with_surface_dist``, stages "run" and "masks" are followed on the same stream by btpost_surface_distance on the
+        projector mask they wrote."""
         # module constants are read at call time, as the reference reads its globals inside the loop
         if self.cfg.conf_thres is None:
             self.params.conf_thres = CONF_TH
@@ -322,6 +340,14 @@ class PostProcessor:
                 rc = fn(C.byref(self.params), C.byref(io), C.c_void_p(self._ws_ptr), C.c_size_t(self._ws_bytes),
                         C.c_void_p(st.cuda_stream))
         _lib.check(rc, f"btpost_{stage}")
+        if self.cfg.with_surface_dist and stage in ("run", "masks"):
+            o, sc = self.out, self._surf_scratch
+            with torch.cuda.device(self.device):
+                rc = self.lib.btpost_surface_distance(
+                    self.B, self.S, C.c_void_p(o["seg_mask"].data_ptr()), C.c_void_p(io.masks_gt), self.cfg.gt_mask_dtype,
+                    *(C.c_void_p(o[k].data_ptr()) for k in ("seg_hd", "seg_hd95", "seg_assd", "seg_surf_acc")),
+                    C.c_void_p(sc.data_ptr()), C.c_size_t(sc.numel()), C.c_void_p(st.cuda_stream))
+            _lib.check(rc, "btpost_surface_distance")
         return self.out
 
     def capture(self, head, protos, det_boxes_gt, masks_gt, proj_weight, proj_bias=0.0, image_stride=0, **kw):
@@ -374,7 +400,7 @@ class Pipeline:
     slot's input buffers on that slot's stream and replays its step; a producer can instead write straight into
     ``inputs[slot]`` and call ``replay(slot)`` (zero-copy).  ``wait(slot)`` blocks the host until the slot's step is
     done and returns its outputs, which stay valid until the slot is used again (``depth`` steps later).  The
-    accumulated counters (cm, seg_cnt4, uni_cnt4, seg_soft_acc) are shared by all slots (device atomics):
+    accumulated counters (cm, seg_cnt4, uni_cnt4, seg_soft_acc, seg_surf_acc) are shared by all slots (device atomics):
     ``counters(key)``.
 
     ``det_boxes_gt`` lives in a fixed ``[gt_rows_cap, 6]`` buffer per slot; unused rows carry batch index -1, which
@@ -398,7 +424,8 @@ class Pipeline:
         self.sweep = sweep
         self.shared = sweep.counters() if sweep is not None else {
             "cm": torch.zeros(nc, nc, dtype=torch.int64, device=dev), "seg_cnt4": torch.zeros(4, dtype=torch.int64, device=dev),
-            "uni_cnt4": torch.zeros(4, dtype=torch.int64, device=dev), "seg_soft_acc": torch.zeros(2, dtype=torch.int64, device=dev)}
+            "uni_cnt4": torch.zeros(4, dtype=torch.int64, device=dev), "seg_soft_acc": torch.zeros(2, dtype=torch.int64, device=dev),
+            "seg_surf_acc": torch.zeros(4, dtype=torch.int64, device=dev)}
         self.procs = [PostProcessor(cfg, dev, shared_counters=self.shared, sweep=sweep) for _ in range(depth)]
         N = self.procs[0].N
         self.gt_rows_cap = gt_rows_cap if gt_rows_cap is not None else 4 * B

@@ -241,6 +241,7 @@ REC_BYTES = 32
 REC_DTYPE = np.dtype([("matched", "<u8"), ("ignored", "<u8"), ("score_key", "<u4"), ("image", "<u4"), ("rank", "<u2"),
                       ("class_rank", "<u2"), ("label", "u1"), ("pad", "u1", (3,))])
 FSUM_SCALE = float(2 ** 40)
+SURF_SCALE = float(2 ** 32)   # seg_surf_acc (btpost_surface_distance's acc)
 
 
 def summarize(precision, recall, iou_thrs, max_dets):
@@ -355,15 +356,19 @@ class DeviceSweep:
     average="micro")`: every label counts as one class, so a well-placed box with the wrong class is a hit): one record
     per kept detection, so the same capacity as the detection ring; `finish()` then also returns the `micro_`-prefixed
     mAP / mAR keys and the `micro_precision` / `micro_recall` tables (the per-class keys stay the class-aware ones, as in
-    torchmetrics)."""
+    torchmetrics).  `surface=True` (needs `PostConfig.with_surface_dist`): `finish()` also returns the means over the images
+    with defined values (NaN when there is none) of the projector mask's Hausdorff distance, HD95 and ASSD, `seg_hd`,
+    `seg_hd95` and `seg_assd`, and `n_surface_images`, from the `seg_surf_acc` header slots."""
 
     def __init__(self, nc: int, iou_thrs, max_dets=(1, 10, 100), capacity: int = 1 << 20, max_det_per_image: int = 300,
-                 device="cuda:0", seg_map_capacity: int = 0, soft_dice: bool = False, micro: bool = False):
+                 device="cuda:0", seg_map_capacity: int = 0, soft_dice: bool = False, micro: bool = False,
+                 surface: bool = False):
         self.lib = _lib.load()
         self.nc, self.iou_thrs, self.max_dets = nc, [float(t) for t in iou_thrs], tuple(int(m) for m in max_dets)
         self.T, self.capacity, self.K = len(self.iou_thrs), int(capacity), int(max_det_per_image)
         self.seg_map_capacity = int(seg_map_capacity)
         self.soft_dice = bool(soft_dice)
+        self.surface = bool(surface)
         self.device = torch.device(device)
         if self.device.type != "cuda":
             raise RuntimeError("DeviceSweep lives on a CUDA device (the records are written by the CUDA library)")
@@ -386,6 +391,7 @@ class DeviceSweep:
         self.seg_cnt4 = self.hdr[u + 256: u + 260]
         self.uni_cnt4 = self.hdr[u + 260: u + 264]
         self.seg_soft_acc = self.hdr[u + 264: u + 266]   # sum of soft Dice (2^-40 units), images with a defined value
+        self.seg_surf_acc = self.hdr[u + 266: u + 270]   # sums of HD, HD95, ASSD (2^-32 units), images with defined values
         self.rec_thrs = torch.from_numpy(np.linspace(0.0, 1.0, 101)).to(self.device)
         self._md = (C.c_int32 * len(self.max_dets))(*self.max_dets)
         self.reset()
@@ -422,9 +428,10 @@ class DeviceSweep:
         del keep   # back to the allocator's cache
 
     def counters(self):
-        """cm / seg_cnt4 / uni_cnt4 / seg_soft_acc views INSIDE the header: hand them to PostProcessor / Pipeline as
-        accumulators and they are merged by the same all-reduce."""
-        return {"cm": self.cm, "seg_cnt4": self.seg_cnt4, "uni_cnt4": self.uni_cnt4, "seg_soft_acc": self.seg_soft_acc}
+        """cm / seg_cnt4 / uni_cnt4 / seg_soft_acc / seg_surf_acc views INSIDE the header: hand them to PostProcessor /
+        Pipeline as accumulators and they are merged by the same all-reduce."""
+        return {"cm": self.cm, "seg_cnt4": self.seg_cnt4, "uni_cnt4": self.uni_cnt4, "seg_soft_acc": self.seg_soft_acc,
+                "seg_surf_acc": self.seg_surf_acc}
 
     def reset(self, stream=None):
         st = stream if stream is not None else torch.cuda.current_stream(self.device)
@@ -542,4 +549,8 @@ class DeviceSweep:
         if self.soft_dice:
             s, k = int(h[u + 264]), int(h[u + 265])
             res.update(seg_soft_dice=s / FSUM_SCALE / k if k else float("nan"), n_soft_dice_images=k)
+        if self.surface:
+            k = int(h[u + 269])
+            res.update({key: int(h[u + 266 + i]) / SURF_SCALE / k if k else float("nan")
+                        for i, key in enumerate(("seg_hd", "seg_hd95", "seg_assd"))}, n_surface_images=k)
         return res

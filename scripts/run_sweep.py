@@ -13,7 +13,9 @@ mAP (one record per image, appended by the mask stage to a second sweep state; s
 default run leaves it out, so that its numbers stay comparable with earlier profiles.  --soft-dice adds v3's soft Dice
 on the projector probabilities (seg_soft_dice in the line; one exp and one division per output pixel in the mask stage).
 --micro adds the class-agnostic box mAP (torchmetrics average="micro": a third sweep state, one record per kept detection,
-filled by a second matching pass of the COCO kernel; micro_map / micro_map_50 in the line)."""
+filled by a second matching pass of the COCO kernel; micro_map / micro_map_50 in the line).  --surface adds the projector
+mask's Hausdorff distance, HD95 and ASSD against the GT mask (btpost_surface_distance after the mask stage of every batch;
+the means seg_hd / seg_hd95 / seg_assd in the line)."""
 import argparse, json, os, sys, time
 from pathlib import Path
 ROOT = Path(__file__).resolve().parents[1]
@@ -32,6 +34,7 @@ ap.add_argument("--seed", type=int, default=20265)
 ap.add_argument("--seg-map", dest="seg_map", action="store_true", help="also the v3 segmentation mAP (seg_map, seg_map_50)")
 ap.add_argument("--soft-dice", dest="soft_dice", action="store_true", help="also v3's soft Dice on the projector probabilities")
 ap.add_argument("--micro", action="store_true", help="also the class-agnostic box mAP (micro_map, micro_map_50)")
+ap.add_argument("--surface", action="store_true", help="also the projector mask's HD / HD95 / ASSD (seg_hd, seg_hd95, seg_assd)")
 args = ap.parse_args()
 rank, world, lrank = (int(os.environ.get(k, d)) for k, d in (("RANK", 0), ("WORLD_SIZE", 1), ("LOCAL_RANK", 0)))
 torch.cuda.set_device(lrank)
@@ -46,9 +49,11 @@ if world > 1:
 B, K = args.batch, args.max_det
 nbatches = args.images // B
 mine = [i for i in range(nbatches) if i % world == rank]          # whole batches b = r (mod G)
-cfg = PostConfig(batch=B, img_size=args.img, gt_mode=1, max_det=K, with_seg_map=args.seg_map, with_soft_dice=args.soft_dice)
+cfg = PostConfig(batch=B, img_size=args.img, gt_mode=1, max_det=K, with_seg_map=args.seg_map, with_soft_dice=args.soft_dice,
+                 with_surface_dist=args.surface)
 sweep = DeviceSweep(cfg.nc, map_iou_thresholds(), (1, 10, 100), capacity=max(len(mine), 1) * B * K, max_det_per_image=K, device=dev,
-                    seg_map_capacity=max(len(mine), 1) * B if args.seg_map else 0, soft_dice=args.soft_dice, micro=args.micro)
+                    seg_map_capacity=max(len(mine), 1) * B if args.seg_map else 0, soft_dice=args.soft_dice, micro=args.micro,
+                    surface=args.surface)
 probe = synth.make_batch_device(synth.SynthConfig(batch=B, img_size=args.img, seed=args.seed), dev)
 pipe = Pipeline(cfg, dev, depth=args.depth, proj_weight=probe["proj_weight"], proj_bias=probe["proj_bias"], sweep=sweep)
 del probe
@@ -92,6 +97,8 @@ if rank == 0:
         keys += ("seg_soft_dice",)
     if args.micro:
         keys += ("micro_map", "micro_map_50")
+    if args.surface:
+        keys += ("seg_hd", "seg_hd95", "seg_assd", "n_surface_images")
     line = {k: res[k] for k in keys}
     line.update(world=world, images=nbatches * B, batches_in_flight=args.depth, device_ms_batches_incl_generation=tms[0],
                 device_ms_reduce_gather_accumulate=tms[1], device_ms_total=tms[2], host_s=time.perf_counter() - t_host)
