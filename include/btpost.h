@@ -255,6 +255,26 @@ BTPOST_API int btpost_masks_parts(const BtParams *p, const BtIO *io, void *ws, s
  * they use different workspaces / output buffers (two calls that share a workspace must be ordered by the caller). */
 BTPOST_API int btpost_run(const BtParams *p, const BtIO *io, void *ws, size_t ws_bytes, void *stream);
 
+/* Binned precision-recall / ROC state of the projector probabilities (torchmetrics BinaryPrecisionRecallCurve / BinaryROC /
+ * BinaryAUROC / BinaryAveragePrecision with thresholds=T; DESIGN.md §4).  Every one of the S^2 pixels of every image counts:
+ * p = 1 / (1 + exp(-x)) of its upsampled projector logit x exactly as soft Dice computes it (BtIOSoftDice; p = 0 for
+ * x < -87), t = its GT bit (the one seg_cnt4 counts).  A pixel is predicted positive at threshold k iff p >= thr[k]; a NaN
+ * p is below every threshold.
+ *
+ * PRECONDITION: enqueued after btpost_masks or btpost_run on the same workspace, stream and BtParams.  It reads the
+ * projector logits [B, proto_h, proto_w] and the GT block words those calls leave in the workspace, so no other call may
+ * use the workspace in between.
+ *
+ * `thresholds` [num_thresholds] is a HOST array: fp32 values in [0, 1], non-decreasing, 2 <= num_thresholds <=
+ * BT_MAX_CURVE_THRS (torchmetrics' thresholds=T is the fp32 linspace(0, 1, T)); it is copied into the launch.
+ * `hist` [2, num_thresholds + 1] int64 (device, 8-byte aligned) is ACCUMULATED like seg_cnt4: hist[t][j] += pixels with GT
+ * bit t and exactly j thresholds <= p.  Confusion counts at threshold k: tp = sum_{j>k} hist[1][j], fp = sum_{j>k}
+ * hist[0][j], fn = sum_{j<=k} hist[1][j], tn = sum_{j<=k} hist[0][j].  Integer sums: the words do not depend on the launch
+ * shape, the order or the batch composition.  Arguments are checked before any CUDA call. */
+#define BT_MAX_CURVE_THRS 1024
+BTPOST_API int btpost_seg_curve(const BtParams *p, void *ws, size_t ws_bytes, const float *thresholds, int32_t num_thresholds,
+                                int64_t *hist, void *stream);
+
 /* ------------------------------------------------------------------------------------------------------------------
  * Sweep state (a9 accumulate/summarize; replaces torchmetrics MeanAveragePrecision's state lists + COCOeval.accumulate,
  * src/running_main_v2.py:884-892, :1017-1098, src/evaluate_model.py:180-182, :291-319).

@@ -16,6 +16,7 @@ LIB_PATH = Path(os.environ.get("BTPOST_LIB", _HERE / "libbtpost.so"))
 
 BT_NUM_AREA = 4
 BT_MAX_IOU_THRS = 16
+BT_MAX_CURVE_THRS = 1024
 LAYOUT_L2, LAYOUT_L1 = 0, 1
 CLASS_AGNOSTIC, CLASS_AWARE, CLASS_OFFSET = 0, 1, 2
 GT_LITERAL, GT_INTENDED = 0, 1
@@ -108,8 +109,9 @@ def load():
     L.btpost_surface_bytes.argtypes = [C.c_int32, C.c_int32, C.POINTER(C.c_size_t)]
     L.btpost_surface_distance.argtypes = [C.c_int32, C.c_int32] + [C.c_void_p] * 2 + [C.c_int32] + [C.c_void_p] * 5 + [C.c_size_t,
                                                                                                                       C.c_void_p]
+    L.btpost_seg_curve.argtypes = [C.POINTER(BtParams), C.c_void_p, C.c_size_t, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p]
     for name in ("btpost_sweep_bytes", "btpost_sweep_reset", "btpost_sweep_accumulate_bytes", "btpost_sweep_accumulate",
-                 "btpost_sweep_accumulate_ext", "btpost_surface_bytes", "btpost_surface_distance"):
+                 "btpost_sweep_accumulate_ext", "btpost_surface_bytes", "btpost_surface_distance", "btpost_seg_curve"):
         getattr(L, name).restype = C.c_int
     _lib = L
     return L

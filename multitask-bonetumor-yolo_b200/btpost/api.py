@@ -19,9 +19,10 @@ import ctypes as C
 import dataclasses
 from dataclasses import dataclass, field
 
+import numpy as np
 import torch
 
-from . import _lib
+from . import _lib, segcurve
 from ._lib import BtIO, BtIOMicro, BtIOSoftDice, BtParams
 
 # Module constants with the reference's names and defaults (running_main_v2.py:51-53); overridable.
@@ -133,6 +134,8 @@ class PostConfig:
     with_soft_dice: bool = False         # v3 soft Dice on the projector probabilities: seg_soft2 / seg_soft_dice (+ seg_soft_acc)
     with_surface_dist: bool = False      # Hausdorff distance, HD95 and ASSD of the projector mask against the GT mask, per image:
                                          # seg_hd / seg_hd95 / seg_assd (+ seg_surf_acc); implies the seg_mask output
+    seg_curve: int | list | None = None  # binned PR / ROC state of the projector probabilities: T thresholds (an int: fp32
+                                         # linspace(0, 1, T)) or a list of them; accumulates seg_curve [2, T+1] (btpost.segcurve)
     num_anchors: int | None = None
     nms_threads: int = 0                 # 0 = auto; 512 / 1024 force a variant of the NMS kernel
     in_flight: int = 0                   # batches kept in flight on the device (Pipeline sets its depth): grid sizes of the mask stage
@@ -208,9 +211,20 @@ class PostProcessor:
             for k in ("seg_hd", "seg_hd95", "seg_assd"):
                 o[k] = z(B, dtype=torch.float32)
             o["seg_surf_acc"] = z(4, dtype=torch.int64)
+        self.curve_thresholds = None if cfg.seg_curve is None else segcurve.thresholds(cfg.seg_curve)
+        if self.curve_thresholds is not None:
+            o["seg_curve"] = z(2, len(self.curve_thresholds) + 1, dtype=torch.int64)
+            self._curve_thr = (C.c_float * len(self.curve_thresholds))(*self.curve_thresholds.tolist())
+        sweep_thr = None if sweep is None else sweep.seg_curve_thresholds
+        if sweep is not None and (sweep_thr is None) != (self.curve_thresholds is None):
+            raise ValueError("a sweep with seg_curve needs PostConfig.seg_curve with the same thresholds, and a PostConfig "
+                             "with seg_curve a sweep with the same thresholds (or no sweep)")
+        if sweep_thr is not None and not np.array_equal(sweep_thr, self.curve_thresholds):
+            raise ValueError("the sweep's seg_curve thresholds differ from PostConfig.seg_curve's")
         if shared_counters:   # Pipeline: every slot adds into the same accumulators (device atomics)
             for k in (("cm", "seg_cnt4", "uni_cnt4") + (("seg_soft_acc",) if cfg.with_soft_dice else ())
-                      + (("seg_surf_acc",) if cfg.with_surface_dist else ())):
+                      + (("seg_surf_acc",) if cfg.with_surface_dist else ())
+                      + (("seg_curve",) if self.curve_thresholds is not None else ())):
                 o[k] = shared_counters[k]
         if cfg.with_seg_mask or cfg.with_surface_dist:   # the surface distances are computed from the projector mask bytes
             o["seg_mask"] = z(B, S, S, dtype=torch.uint8)
@@ -252,8 +266,8 @@ class PostProcessor:
     # -- metric state ---------------------------------------------------------------------------
     def reset_metrics(self):
         """Zero the accumulated counters (confusion matrix, global pixel tp/fp/fn/tn, soft-Dice and surface-distance sums
-        and counts)."""
-        for k in ("cm", "seg_cnt4", "uni_cnt4", "seg_soft_acc", "seg_surf_acc"):
+        and counts, the binned curve state)."""
+        for k in ("cm", "seg_cnt4", "uni_cnt4", "seg_soft_acc", "seg_surf_acc", "seg_curve"):
             if k in self.out:
                 self.out[k].zero_()
 
@@ -305,7 +319,8 @@ class PostProcessor:
         self._check_in(proj_weight, (cfg.nm,), torch.float32, "proj_weight")
         io.proj_weight = proj_weight.data_ptr()
         for k, v in self.out.items():
-            setattr(io, k, v.data_ptr())
+            if k != "seg_curve":   # not a BtIO field: btpost_seg_curve's accumulator
+                setattr(io, k, v.data_ptr())
         if self.sweep is not None:
             io.sweep = self.sweep.ptr
             io.seg_sweep = self.sweep.seg_ptr
@@ -319,8 +334,9 @@ class PostProcessor:
             stage="run", stream=None, image_offset=0):
         """Enqueue the hot path for one batch on the current (or given) CUDA stream; returns the
         dict of output tensors (device, padded to ``max_det`` / ``max_gt``; see include/btpost.h).  With
-        ``with_surface_dist``, stages "run" and "masks" are followed on the same stream by btpost_surface_distance on the
-        projector mask they wrote."""
+        ``seg_curve``, stages "run" and "masks" are followed on the same stream by btpost_seg_curve on the projector logits
+        and GT words they left in the workspace; with ``with_surface_dist``, by btpost_surface_distance on the projector
+        mask they wrote."""
         # module constants are read at call time, as the reference reads its globals inside the loop
         if self.cfg.conf_thres is None:
             self.params.conf_thres = CONF_TH
@@ -340,6 +356,12 @@ class PostProcessor:
                 rc = fn(C.byref(self.params), C.byref(io), C.c_void_p(self._ws_ptr), C.c_size_t(self._ws_bytes),
                         C.c_void_p(st.cuda_stream))
         _lib.check(rc, f"btpost_{stage}")
+        if self.curve_thresholds is not None and stage in ("run", "masks"):
+            with torch.cuda.device(self.device):
+                rc = self.lib.btpost_seg_curve(C.byref(self.params), C.c_void_p(self._ws_ptr), C.c_size_t(self._ws_bytes),
+                                               self._curve_thr, len(self.curve_thresholds),
+                                               C.c_void_p(self.out["seg_curve"].data_ptr()), C.c_void_p(st.cuda_stream))
+            _lib.check(rc, "btpost_seg_curve")
         if self.cfg.with_surface_dist and stage in ("run", "masks"):
             o, sc = self.out, self._surf_scratch
             with torch.cuda.device(self.device):
@@ -400,7 +422,7 @@ class Pipeline:
     slot's input buffers on that slot's stream and replays its step; a producer can instead write straight into
     ``inputs[slot]`` and call ``replay(slot)`` (zero-copy).  ``wait(slot)`` blocks the host until the slot's step is
     done and returns its outputs, which stay valid until the slot is used again (``depth`` steps later).  The
-    accumulated counters (cm, seg_cnt4, uni_cnt4, seg_soft_acc, seg_surf_acc) are shared by all slots (device atomics):
+    accumulated counters (cm, seg_cnt4, uni_cnt4, seg_soft_acc, seg_surf_acc, seg_curve) are shared by all slots (device atomics):
     ``counters(key)``.
 
     ``det_boxes_gt`` lives in a fixed ``[gt_rows_cap, 6]`` buffer per slot; unused rows carry batch index -1, which
@@ -426,6 +448,8 @@ class Pipeline:
             "cm": torch.zeros(nc, nc, dtype=torch.int64, device=dev), "seg_cnt4": torch.zeros(4, dtype=torch.int64, device=dev),
             "uni_cnt4": torch.zeros(4, dtype=torch.int64, device=dev), "seg_soft_acc": torch.zeros(2, dtype=torch.int64, device=dev),
             "seg_surf_acc": torch.zeros(4, dtype=torch.int64, device=dev)}
+        if sweep is None and cfg.seg_curve is not None:
+            self.shared["seg_curve"] = torch.zeros(2, len(segcurve.thresholds(cfg.seg_curve)) + 1, dtype=torch.int64, device=dev)
         self.procs = [PostProcessor(cfg, dev, shared_counters=self.shared, sweep=sweep) for _ in range(depth)]
         N = self.procs[0].N
         self.gt_rows_cap = gt_rows_cap if gt_rows_cap is not None else 4 * B

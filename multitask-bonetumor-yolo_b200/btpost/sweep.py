@@ -34,7 +34,7 @@ import numpy as np
 import torch
 import torch.distributed as dist
 
-from . import _lib
+from . import _lib, segcurve
 
 AREA_NAMES = ("all", "small", "medium", "large")
 
@@ -283,12 +283,13 @@ def merge_shards(hdr: torch.Tensor, records: torch.Tensor, group=None):
 
 
 @torch.no_grad()
-def merge_sweeps(hdrs, rings, group=None):
+def merge_sweeps(hdrs, rings, group=None, extra=()):
     """`merge_shards` for several sweep states at once (the detection sweep and the segmentation-mAP sweep) with the
     same three collectives: the record counts in one all-gather, the headers, concatenated, in ONE all-reduce (each
     `hdrs[s]` is summed in place), the valid records of every state in one `all_gather_into_tensor` (each state padded to
-    its largest shard).  Returns (ns, merged): per state, the n_per_rank list and the records of all ranks concatenated
-    in rank order."""
+    its largest shard).  `extra`: further int64 counter tensors (the binned curve state), contiguous and on the headers'
+    device, concatenated into the same all-reduce and summed in place.  Returns (ns, merged): per state, the n_per_rank
+    list and the records of all ranks concatenated in rank order."""
     S = len(hdrs)
     n_local = [int(min(int(h[_lib.SWEEP_N_RECORDS]), r.shape[0])) for h, r in zip(hdrs, rings)]
     if not (dist.is_available() and dist.is_initialized()) or dist.get_world_size(group) == 1:
@@ -296,12 +297,13 @@ def merge_sweeps(hdrs, rings, group=None):
     W, dev = dist.get_world_size(group), hdrs[0].device
     counts = torch.zeros(W * S, dtype=torch.int64, device=dev)
     dist.all_gather_into_tensor(counts, torch.tensor(n_local, dtype=torch.int64, device=dev), group=group)
-    if S == 1:
+    summed = list(hdrs) + [e.view(-1) for e in extra]
+    if len(summed) == 1:
         dist.all_reduce(hdrs[0], group=group)
     else:
-        cat = torch.cat(list(hdrs))
+        cat = torch.cat(summed)
         dist.all_reduce(cat, group=group)
-        for h, v in zip(hdrs, cat.split([h.numel() for h in hdrs])):
+        for h, v in zip(summed, cat.split([h.numel() for h in summed])):
             h.copy_(v)
     ns = [[int(v) for v in col] for col in zip(*counts.view(W, S).tolist())]   # ns[s][rank]
     caps = [max(max(n), 1) for n in ns]
@@ -358,11 +360,15 @@ class DeviceSweep:
     mAP / mAR keys and the `micro_precision` / `micro_recall` tables (the per-class keys stay the class-aware ones, as in
     torchmetrics).  `surface=True` (needs `PostConfig.with_surface_dist`): `finish()` also returns the means over the images
     with defined values (NaN when there is none) of the projector mask's Hausdorff distance, HD95 and ASSD, `seg_hd`,
-    `seg_hd95` and `seg_assd`, and `n_surface_images`, from the `seg_surf_acc` header slots."""
+    `seg_hd95` and `seg_assd`, and `n_surface_images`, from the `seg_surf_acc` header slots.  `seg_curve` = T or a list of
+    thresholds (needs `PostConfig.seg_curve` with the same thresholds): the sweep owns the binned curve state `seg_curve`
+    [2, T+1] (`counters()`), merged in the header all-reduce; `finish()` also returns `seg_curve_thresholds`,
+    `seg_curve_confmat` (torchmetrics' [T, 2, 2] state), `seg_pr_curve` (precision, recall, thresholds), `seg_roc` (fpr,
+    tpr, thresholds), `seg_ap` and `seg_auroc` of the projector probabilities over every pixel (`btpost.segcurve`)."""
 
     def __init__(self, nc: int, iou_thrs, max_dets=(1, 10, 100), capacity: int = 1 << 20, max_det_per_image: int = 300,
                  device="cuda:0", seg_map_capacity: int = 0, soft_dice: bool = False, micro: bool = False,
-                 surface: bool = False):
+                 surface: bool = False, seg_curve: int | list | None = None):
         self.lib = _lib.load()
         self.nc, self.iou_thrs, self.max_dets = nc, [float(t) for t in iou_thrs], tuple(int(m) for m in max_dets)
         self.T, self.capacity, self.K = len(self.iou_thrs), int(capacity), int(max_det_per_image)
@@ -392,6 +398,10 @@ class DeviceSweep:
         self.uni_cnt4 = self.hdr[u + 260: u + 264]
         self.seg_soft_acc = self.hdr[u + 264: u + 266]   # sum of soft Dice (2^-40 units), images with a defined value
         self.seg_surf_acc = self.hdr[u + 266: u + 270]   # sums of HD, HD95, ASSD (2^-32 units), images with defined values
+        self.seg_curve_thresholds = self.seg_curve = None
+        if seg_curve is not None:
+            self.seg_curve_thresholds = segcurve.thresholds(seg_curve)
+            self.seg_curve = torch.zeros(2, len(self.seg_curve_thresholds) + 1, dtype=torch.int64, device=self.device)
         self.rec_thrs = torch.from_numpy(np.linspace(0.0, 1.0, 101)).to(self.device)
         self._md = (C.c_int32 * len(self.max_dets))(*self.max_dets)
         self.reset()
@@ -428,10 +438,14 @@ class DeviceSweep:
         del keep   # back to the allocator's cache
 
     def counters(self):
-        """cm / seg_cnt4 / uni_cnt4 / seg_soft_acc / seg_surf_acc views INSIDE the header: hand them to PostProcessor /
-        Pipeline as accumulators and they are merged by the same all-reduce."""
-        return {"cm": self.cm, "seg_cnt4": self.seg_cnt4, "uni_cnt4": self.uni_cnt4, "seg_soft_acc": self.seg_soft_acc,
-                "seg_surf_acc": self.seg_surf_acc}
+        """cm / seg_cnt4 / uni_cnt4 / seg_soft_acc / seg_surf_acc views INSIDE the header, and the seg_curve state when
+        the sweep has one: hand them to PostProcessor / Pipeline as accumulators and they are merged by the same
+        all-reduce."""
+        c = {"cm": self.cm, "seg_cnt4": self.seg_cnt4, "uni_cnt4": self.uni_cnt4, "seg_soft_acc": self.seg_soft_acc,
+             "seg_surf_acc": self.seg_surf_acc}
+        if self.seg_curve is not None:
+            c["seg_curve"] = self.seg_curve
+        return c
 
     def reset(self, stream=None):
         st = stream if stream is not None else torch.cuda.current_stream(self.device)
@@ -440,6 +454,9 @@ class DeviceSweep:
                 if ptr is not None:
                     _lib.check(self.lib.btpost_sweep_reset(C.c_void_p(ptr), C.c_int64(cap), C.c_void_p(st.cuda_stream)),
                                "btpost_sweep_reset")
+        if self.seg_curve is not None:
+            with torch.cuda.stream(st):
+                self.seg_curve.zero_()
 
     def _accumulate(self, rec, n, hdr, nc, max_det_per_image, num_images_bound, scores=False):
         """btpost_sweep_accumulate_ext on `n` merged records (reordered in place) -> (precision, recall) device tables, and
@@ -495,7 +512,8 @@ class DeviceSweep:
             if n > cap:
                 raise RuntimeError(f"DeviceSweep {what}ring too small: {n} records offered, capacity {cap}")
         hdrs = [h.clone() for _, h, _, _ in states]
-        ns, recs = merge_sweeps(hdrs, [r for _, _, r, _ in states], group)
+        curve = self.seg_curve.clone() if self.seg_curve is not None else None
+        ns, recs = merge_sweeps(hdrs, [r for _, _, r, _ in states], group, extra=() if curve is None else (curve,))
         _mark("merge_shards")
         for i, ((_, _, ring, _), rec) in enumerate(zip(states, recs)):
             if sum(ns[i]) and rec.data_ptr() == ring.data_ptr():
@@ -553,4 +571,9 @@ class DeviceSweep:
             k = int(h[u + 269])
             res.update({key: int(h[u + 266 + i]) / SURF_SCALE / k if k else float("nan")
                         for i, key in enumerate(("seg_hd", "seg_hd95", "seg_assd"))}, n_surface_images=k)
+        if curve is not None:
+            cm = segcurve.confmat(curve)
+            m = segcurve.curve_metrics(cm, self.seg_curve_thresholds)
+            res.update(seg_curve_thresholds=self.seg_curve_thresholds.copy(), seg_curve_confmat=cm, seg_pr_curve=m["pr_curve"],
+                       seg_roc=m["roc"], seg_ap=m["ap"], seg_auroc=m["auroc"])
         return res

@@ -18,8 +18,9 @@ static int check_anchor_limit(const BtParams *p) {
     return p->num_anchors > 8 * 1024 * per_thread ? BT_ERR_UNSUPPORTED : BT_OK;
 }
 
-int check_params(const BtParams *p, const BtIO *io) {
-    if (!p || !io) return BT_ERR_BAD_ARG;
+// The problem description alone (btpost_seg_curve takes no BtIO).
+static int check_shape(const BtParams *p) {
+    if (!p) return BT_ERR_BAD_ARG;
     if (p->batch <= 0 || p->num_anchors <= 0 || p->nc <= 0 || p->max_det <= 0) return BT_ERR_BAD_ARG;
     if (p->nc > BT_MAX_CLASSES || p->nm != 32) return BT_ERR_UNSUPPORTED;
     if (p->max_gt <= 0 || p->max_gt > 32) return BT_ERR_UNSUPPORTED;
@@ -46,6 +47,11 @@ int check_params(const BtParams *p, const BtIO *io) {
         return BT_ERR_BAD_ARG;
     }
     return check_anchor_limit(p);
+}
+
+int check_params(const BtParams *p, const BtIO *io) {
+    if (!p || !io) return BT_ERR_BAD_ARG;
+    return check_shape(p);
 }
 
 static int check_ws(const BtParams *p, void *ws, size_t ws_bytes) {
@@ -257,6 +263,22 @@ int btpost_run(const BtParams *p, const BtIO *io, void *ws, size_t ws_bytes, voi
     if (join_rec && !ok(cudaStreamWaitEvent(s, side->join, 0)) && rc == BT_OK) rc = BT_ERR_CUDA;
     side_release(side, dev);
     return rc;
+}
+
+int btpost_seg_curve(const BtParams *p, void *ws, size_t ws_bytes, const float *thresholds, int32_t num_thresholds,
+                     int64_t *hist, void *stream) {
+    if (!thresholds || !hist) return BT_ERR_BAD_ARG;
+    if (num_thresholds < 2 || num_thresholds > BT_MAX_CURVE_THRS) return BT_ERR_BAD_ARG;
+    for (int i = 0; i < num_thresholds; ++i) {
+        const float v = thresholds[i];
+        if (!(v >= 0.0f && v <= 1.0f)) return BT_ERR_BAD_ARG;   // NaN fails too
+        if (i > 0 && v < thresholds[i - 1]) return BT_ERR_BAD_ARG;
+    }
+    if (reinterpret_cast<uintptr_t>(hist) & 7) return BT_ERR_MISALIGNED;
+    int rc = check_shape(p);
+    if (rc == BT_OK) rc = check_ws(p, ws, ws_bytes);
+    if (rc != BT_OK) return rc;
+    return launch_seg_curve(*p, carve(p, ws), thresholds, num_thresholds, hist, static_cast<cudaStream_t>(stream));
 }
 
 }  // extern "C"

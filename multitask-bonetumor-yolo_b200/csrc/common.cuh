@@ -52,13 +52,20 @@ __device__ __forceinline__ float bt_expf(float x) {
     return __int_as_float(__float_as_int(p) + (e << 23));
 }
 
-// sigmoid(x) in units of 2^-40, the term of the soft-Dice sums (BtIOSoftDice.seg_soft2): 1 / (1 + bt_expf(-x)) rounded once
-// per operation, then scaled (exactly) and rounded to the nearest integer.  x < -87 gives 0: bt_expf(-x) would
-// wrap there, and the true value is below 2^-125, which rounds to 0 in this fixed point anyway.
+// sigmoid(x) in fp32, the projector probability of soft Dice and of the binned curves (btpost_seg_curve): 1 / (1 +
+// bt_expf(-x)) rounded once per operation.  x < -87 gives 0: bt_expf(-x) would wrap there, and the true value is below
+// 2^-125.  A NaN x gives NaN.
+__device__ __forceinline__ float soft_prob(float x) {
+    if (x < -87.0f) return 0.0f;
+    return __fdiv_rn(1.0f, __fadd_rn(1.0f, bt_expf(-x)));
+}
+
+// sigmoid(x) in units of 2^-40, the term of the soft-Dice sums (BtIOSoftDice.seg_soft2): soft_prob(x) scaled (exactly)
+// and rounded to the nearest integer.  (The early return keeps the integer 0 off the float path, as before soft_prob was
+// factored out: cells_kernel compiles to the same instructions.)
 __device__ __forceinline__ long long soft_prob_fx40(float x) {
     if (x < -87.0f) return 0ll;
-    const float p = __fdiv_rn(1.0f, __fadd_rn(1.0f, bt_expf(-x)));
-    return __float2ll_rn(__fmul_rn(p, 1099511627776.0f));
+    return __float2ll_rn(__fmul_rn(soft_prob(x), 1099511627776.0f));
 }
 
 // Order-preserving image of an fp32 score: ascending key = descending score (sort keys of the NMS, sweep records).
@@ -222,5 +229,7 @@ int launch_nms_match(const BtParams &p, const BtIO &io, const Workspace &w, cuda
 // parts: BT_MASKS_PACK (GT bits; independent of the detections), BT_MASKS_CONTRACT (the pass over the prototypes),
 // BT_MASKS_CELLS (upsample + threshold + counters + per-image finalize)
 int launch_masks(const BtParams &p, const BtIO &io, const Workspace &w, cudaStream_t s, int parts = 7);
+// binned PR / ROC state of the projector probabilities from the logits and GT words a mask-stage call left in `w`
+int launch_seg_curve(const BtParams &p, const Workspace &w, const float *thr, int T, int64_t *hist, cudaStream_t s);
 
 }  // namespace bt

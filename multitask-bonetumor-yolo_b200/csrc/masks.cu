@@ -30,6 +30,8 @@
 //                     cells.  Instruction-issue bound.
 //   finalize_kernel   one warp per image: counters -> Dice / IoU / tp-fp-fn-tn, the image's v3 segmentation-mAP
 //                     record when BtIO.seg_sweep is set, and its v3 soft Dice when BtIOSoftDice.seg_soft2 is set.
+// A fifth kernel, seg_curve_kernel (btpost_seg_curve, its own entry point), runs after them when the caller asks for the
+// binned PR / ROC state of the projector probabilities.
 // tcgen05 is deliberately not used: K = 32 at <= 0.5 FLOP/B, and TF32/BF16 accumulation would break the bit
 // parity of the thresholded masks with the fp32 reference.
 #include <cuda.h>
@@ -729,6 +731,112 @@ __device__ __forceinline__ void m1_item(const K3Params &P, int b, int q, int lan
     }
 }
 
+// =================================================================================================
+// seg_curve_kernel (btpost_seg_curve): binned precision-recall / ROC state of the projector probabilities.  Reads the
+// projector logits at prototype resolution and the GT block words that btpost_masks left in the workspace, redoes
+// m1_item's bilinear x4 per 2x2 cell block (block_geo / cell_bits_log / cell_valid: the logits of cells_kernel, bit for
+// bit), and counts every valid pixel in hist[t][j], t = its GT bit, j = the number of thresholds <= p = soft_prob(x).
+// =================================================================================================
+// A persistent grid of 3 CTAs per SM (up to 85 registers; at 4, ptxas spills), few enough CTAs that the flush (at most
+// 2 (T + 1) atomics per CTA) stays small; each thread takes one block (<= 64 pixels) at a time, grid-strided
+constexpr int CV_THREADS = 256, CV_CTAS_PER_SM = 3;
+constexpr int CV_LUT = 2048;   // cells of the threshold table
+
+struct CurveParams {
+    int B, S_h, S_w, PH, PW, NBY, NBX;
+    int T;                  // thresholds
+    int span;               // power of two > T (building the threshold table)
+    const float *lm;        // [B, PH, PW] projector logits (workspace)
+    const u64 *gtc;         // [B, NBY, NBX] GT bits per 2x2 block of cells (workspace)
+    unsigned long long *hist;   // [2, T + 1], accumulated
+    float thr[BT_MAX_CURVE_THRS];   // non-decreasing, in [0, 1] (checked by the entry point)
+};
+
+// Finding j: a table over CV_LUT equal cells of [0, 1] gives, for the cell of p, the thresholds below the cell (all <= p)
+// and those in it; a search over the few in the cell finishes (one or two compares for linspace thresholds, at most
+// log2(T) whatever the list).
+// Counting: neighbouring pixels of a lane's block mostly fall in one bin, so a lane counts its run of equal bins in a
+// register and adds the run to the CTA's u32 bins in shared memory with one atomic when the bin changes (measured on a
+// B200 at 64 x 640^2, T = 101: 128 us, against 202 us with a warp match per pixel and one atomic per distinct bin).  The
+// CTA's bins go to `hist` once, with one 64-bit atomic per non-zero bin.  Integer sums: the words do not depend on the
+// launch shape.
+__global__ void __launch_bounds__(CV_THREADS, CV_CTAS_PER_SM) seg_curve_kernel(const __grid_constant__ CurveParams P) {
+    __shared__ float s_thr[BT_MAX_CURVE_THRS];
+    __shared__ unsigned short s_lut[CV_LUT + 2];   // s_lut[c] = thresholds < c / CV_LUT (c <= CV_LUT); s_lut[CV_LUT + 1] = T
+    __shared__ uint32_t s_hist[2 * (BT_MAX_CURVE_THRS + 1)];
+    const int T = P.T, nbins = 2 * (T + 1);
+    for (int i = threadIdx.x; i < T; i += CV_THREADS) s_thr[i] = P.thr[i];
+    for (int i = threadIdx.x; i < nbins; i += CV_THREADS) s_hist[i] = 0u;
+    __syncthreads();
+    for (int c = threadIdx.x; c < CV_LUT + 2; c += CV_THREADS) {
+        const float lo = (float)c * (1.0f / CV_LUT);   // exact
+        int n = 0;
+        for (int step = P.span >> 1; step > 0; step >>= 1)
+            if (n + step <= T && s_thr[n + step - 1] < lo) n += step;
+        s_lut[c] = (unsigned short)(c == CV_LUT + 1 ? T : n);
+    }
+    __syncthreads();
+    const int PH = P.PH, PW = P.PW, NBX = P.NBX;
+    const long long per_image = (long long)P.NBY * NBX, total = P.B * per_image;
+    const long long stride = (long long)gridDim.x * CV_THREADS;
+    uint32_t run_key = 0u, run_n = 0u;   // this lane's current run of pixels in one bin
+    for (long long q = (long long)blockIdx.x * CV_THREADS + threadIdx.x; q < total; q += stride) {
+        int by = 0, bx = 0;
+        float v[3][3];
+        u64 gtw;
+        {
+            const int b = (int)(q / per_image), r = (int)(q - b * per_image);
+            by = r / NBX; bx = r - by * NBX;
+            const BlockGeo g = block_geo(by, bx, PH, PW);
+            const float *lm = P.lm + (size_t)b * PH * PW;
+            const int rr[3] = {g.r0 * PW, g.r1 * PW, g.r2 * PW}, cc[3] = {g.c0, g.c1, g.c2};
+#pragma unroll
+            for (int i = 0; i < 3; ++i)
+#pragma unroll
+                for (int j = 0; j < 3; ++j) v[i][j] = __ldg(lm + rr[i] + cc[j]);
+            gtw = __ldg(P.gtc + q);
+        }
+#pragma unroll
+        for (int a = 0; a < 2; ++a)
+#pragma unroll
+            for (int c = 0; c < 2; ++c) {
+                const int ci = 2 * by - 1 + a, cj = 2 * bx - 1 + c;
+                // m1_item's corners v[it][jl] .. v[ib][jr] as selects (a runtime index would put v in local memory)
+                const bool up = a == 1 && by != 0, left = c == 1 && bx != 0;
+                const float v00 = up ? (left ? v[1][1] : v[1][0]) : (left ? v[0][1] : v[0][0]);
+                const float v01 = up ? v[1][c + 1] : v[0][c + 1];
+                const float v10 = left ? v[a + 1][1] : v[a + 1][0];
+                float lg[16];
+                cell_bits_log(v00, v01, v10, v[a + 1][c + 1], ci < 0, cj < 0, lg);
+                const unsigned valid = cell_valid(ci, cj, PH, PW, P.S_h, P.S_w);
+                const unsigned gt = (unsigned)(gtw >> (16 * (2 * a + c))) & 0xffffu;
+#pragma unroll
+                for (int k = 0; k < 16; ++k) {
+                    const float p = soft_prob(lg[k]);
+                    // thresholds <= p: those below p's cell, then a search among the cell's own (a NaN p: cell 0, j = 0)
+                    const int cell = p == p ? (int)__fmul_rn(p, (float)CV_LUT) : 0;   // p in [0, 1]
+                    int j = s_lut[cell], n = s_lut[cell + 1] - j;
+                    while (n > 0) {
+                        const int h = n >> 1;
+                        if (s_thr[j + h] <= p) { j += h + 1; n -= h + 1; } else { n = h; }
+                    }
+                    const uint32_t key = ((gt >> k) & 1u) * (uint32_t)(T + 1) + (uint32_t)j;
+                    if ((valid >> k) & 1u) {
+                        if (key != run_key) {
+                            if (run_n) atomicAdd(&s_hist[run_key], run_n);
+                            run_key = key; run_n = 0u;
+                        }
+                        ++run_n;
+                    }
+                }
+            }
+    }
+    if (run_n) atomicAdd(&s_hist[run_key], run_n);
+    __syncthreads();
+    for (int i = threadIdx.x; i < nbins; i += CV_THREADS)
+        if (const uint32_t n = s_hist[i]) atomicAdd(P.hist + i, (unsigned long long)n);
+}
+
 // Optional output: the block's 8 x 8 pixels into the detection's bit-packed plane (zeroed beforehand).  A block row is
 // 8 pixels starting at x = 8bx - 2 (6 pixels at x = 0 for bx = 0), so it shares its 32-bit word with the neighbouring
 // blocks: fire-and-forget atomic ORs (RED) into the L2.  Pixels outside the image are already masked out of `bits`.
@@ -1215,6 +1323,29 @@ int launch_masks(const BtParams &p, const BtIO &io, const Workspace &w, cudaStre
             if (io.uni_mask) union_dense_kernel<<<p.batch, C_THREADS, 0, s>>>(P);
         }
     }
+    return cudaGetLastError() == cudaSuccess ? BT_OK : BT_ERR_CUDA;
+}
+
+int launch_seg_curve(const BtParams &p, const Workspace &w, const float *thr, int T, int64_t *hist, cudaStream_t s) {
+    CurveParams P{};
+    P.B = p.batch; P.S_h = p.img_h; P.S_w = p.img_w; P.PH = p.proto_h; P.PW = p.proto_w;
+    P.NBY = mask_blocks(p.proto_h); P.NBX = mask_blocks(p.proto_w);
+    P.T = T; P.span = next_pow2(T + 1);
+    P.lm = w.lm; P.gtc = w.gtc; P.hist = reinterpret_cast<unsigned long long *>(hist);
+    for (int i = 0; i < T; ++i) P.thr[i] = thr[i];
+    static int sm_count_dev[64] = {};   // per device ordinal, as in launch_masks
+    int dev = 0;
+    if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) return BT_ERR_CUDA;
+    if (!sm_count_dev[dev] &&
+        (cudaDeviceGetAttribute(&sm_count_dev[dev], cudaDevAttrMultiProcessorCount, dev) != cudaSuccess || sm_count_dev[dev] <= 0))
+        return BT_ERR_CUDA;
+    // A CTA's u32 bins count at most about 64 * blocks / grid pixels: the grid grows before that could reach 2^31.
+    const long long blocks = (long long)p.batch * P.NBY * P.NBX;
+    long long grid = (blocks + CV_THREADS - 1) / CV_THREADS, cap = (long long)sm_count_dev[dev] * CV_CTAS_PER_SM;
+    if (grid > cap) grid = cap;
+    const long long min_grid = (blocks * 64 + 0x7fffffffll) / 0x80000000ll;
+    if (grid < min_grid) grid = min_grid;
+    seg_curve_kernel<<<(unsigned)grid, CV_THREADS, 0, s>>>(P);
     return cudaGetLastError() == cudaSuccess ? BT_OK : BT_ERR_CUDA;
 }
 

@@ -15,7 +15,8 @@ on the projector probabilities (seg_soft_dice in the line; one exp and one divis
 --micro adds the class-agnostic box mAP (torchmetrics average="micro": a third sweep state, one record per kept detection,
 filled by a second matching pass of the COCO kernel; micro_map / micro_map_50 in the line).  --surface adds the projector
 mask's Hausdorff distance, HD95 and ASSD against the GT mask (btpost_surface_distance after the mask stage of every batch;
-the means seg_hd / seg_hd95 / seg_assd in the line)."""
+the means seg_hd / seg_hd95 / seg_assd in the line).  --seg-curve T adds the binned PR / ROC state of the projector
+probabilities at T thresholds (btpost_seg_curve after the mask stage of every batch; seg_ap / seg_auroc in the line)."""
 import argparse, json, os, sys, time
 from pathlib import Path
 ROOT = Path(__file__).resolve().parents[1]
@@ -35,6 +36,8 @@ ap.add_argument("--seg-map", dest="seg_map", action="store_true", help="also the
 ap.add_argument("--soft-dice", dest="soft_dice", action="store_true", help="also v3's soft Dice on the projector probabilities")
 ap.add_argument("--micro", action="store_true", help="also the class-agnostic box mAP (micro_map, micro_map_50)")
 ap.add_argument("--surface", action="store_true", help="also the projector mask's HD / HD95 / ASSD (seg_hd, seg_hd95, seg_assd)")
+ap.add_argument("--seg-curve", dest="seg_curve", type=int, default=None,
+                help="also pixel AP / AUROC of the projector probabilities at this many thresholds (seg_ap, seg_auroc)")
 args = ap.parse_args()
 rank, world, lrank = (int(os.environ.get(k, d)) for k, d in (("RANK", 0), ("WORLD_SIZE", 1), ("LOCAL_RANK", 0)))
 torch.cuda.set_device(lrank)
@@ -50,10 +53,10 @@ B, K = args.batch, args.max_det
 nbatches = args.images // B
 mine = [i for i in range(nbatches) if i % world == rank]          # whole batches b = r (mod G)
 cfg = PostConfig(batch=B, img_size=args.img, gt_mode=1, max_det=K, with_seg_map=args.seg_map, with_soft_dice=args.soft_dice,
-                 with_surface_dist=args.surface)
+                 with_surface_dist=args.surface, seg_curve=args.seg_curve)
 sweep = DeviceSweep(cfg.nc, map_iou_thresholds(), (1, 10, 100), capacity=max(len(mine), 1) * B * K, max_det_per_image=K, device=dev,
                     seg_map_capacity=max(len(mine), 1) * B if args.seg_map else 0, soft_dice=args.soft_dice, micro=args.micro,
-                    surface=args.surface)
+                    surface=args.surface, seg_curve=args.seg_curve)
 probe = synth.make_batch_device(synth.SynthConfig(batch=B, img_size=args.img, seed=args.seed), dev)
 pipe = Pipeline(cfg, dev, depth=args.depth, proj_weight=probe["proj_weight"], proj_bias=probe["proj_bias"], sweep=sweep)
 del probe
@@ -99,6 +102,8 @@ if rank == 0:
         keys += ("micro_map", "micro_map_50")
     if args.surface:
         keys += ("seg_hd", "seg_hd95", "seg_assd", "n_surface_images")
+    if args.seg_curve is not None:
+        keys += ("seg_ap", "seg_auroc")
     line = {k: res[k] for k in keys}
     line.update(world=world, images=nbatches * B, batches_in_flight=args.depth, device_ms_batches_incl_generation=tms[0],
                 device_ms_reduce_gather_accumulate=tms[1], device_ms_total=tms[2], host_s=time.perf_counter() - t_host)
